@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- edges/sec, forward+backward, per GNN layer (`Block`) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], "C3"): a batch of 256 synthetic complete bipartite graphs of
 2394 fibres x 12 classes (28 728 edges each), Fdim 10, fp32, train mode; one step = one `Block`
@@ -91,7 +91,14 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-profile", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="c3 / c5a: after the timed steps, write the outputs and gradients of the last step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("c3", "c5a")):
+        ap.error("--dump-outputs writes what the GPU path of c3 / c5a computes")
+    return args
 
 
 def measured_peaks():
@@ -358,9 +365,11 @@ class BlockStepper:
     """One data-parallel step of the layer: Block forward + backward w.r.t. all four outputs on static inputs, then
     the flat-bucket all-reduce; optionally captured as a CUDA graph (the NCCL all-reduce is a node of the graph)."""
 
-    def __init__(self, blk, ei, xs, ups, bucket, dev, use_graph, warmup=3, pool=None):
+    def __init__(self, blk, ei, xs, ups, bucket, dev, use_graph, warmup=3, pool=None, keep_results=False):
         self.blk, self.ei, self.xs, self.ups, self.bucket, self.dev = blk, ei, xs, ups, bucket, dev
         self.out = None
+        self.keep_results = keep_results
+        self.results = None
         self.graph = None
         if use_graph:
             cur = torch.cuda.current_stream(dev)
@@ -386,6 +395,12 @@ class BlockStepper:
         torch.autograd.backward([o_s, o_t, o_e, o_u], self.ups)
         self.bucket.all_reduce()
         self.out = o_u.detach().sum()        # the step's result (what the end-to-end leg reads back); no autograd graph kept
+        if self.keep_results:
+            # what a caller of the step receives; a graph replay rewrites these tensors in place.  Off by default: the
+            # tensors it keeps alive would change how the timed step's memory is laid out
+            self.results = {n: o.detach() for n, o in zip(("x_s", "x_t", "x_e", "u"), (o_s, o_t, o_e, o_u))}
+            self.results.update({"grad_" + n: x.grad for n, x in zip(("x_s", "x_t", "x_e", "u"), xs)})
+            self.results.update({"grad_" + n: p.grad for n, p in self.blk.named_parameters() if p.grad is not None})
         return self.out
 
     def __call__(self):
@@ -394,6 +409,25 @@ class BlockStepper:
         else:
             self.eager()
         return self.out
+
+
+DUMP_ARRAY_BYTES = 7 << 20       # eight arrays scale with the graphs (four outputs, four input gradients): 56 MB of the 64
+
+
+def dump_outputs(path, arrays):
+    """Write every array as path/<name>.npy in float32.  An array larger than DUMP_ARRAY_BYTES is reduced to a fixed,
+    seeded sample of its rows (leading dimensions flattened, rows kept whole and in order): the same rows on every run
+    with the same arguments, so that the files of two builds can be compared element for element."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() * 4 > DUMP_ARRAY_BYTES:
+            rows = t.reshape(-1, t.shape[-1] if t.dim() > 1 else 1)
+            keep = max(1, DUMP_ARRAY_BYTES // (4 * rows.shape[1]))
+            idx = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = rows[idx.to(rows.device)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
 
 
 def make_inputs(G, S, T, E, F, dev, seed):
@@ -461,17 +495,21 @@ def run_ours(args):
         return ms
 
     # kernels of one step (counted on an eager step: a graph replay launches the same kernels without host calls)
-    eager = BlockStepper(blk, ei, ins, ups, bucket, dev, use_graph=False, warmup=max(args.warmup, 3))
+    keep = bool(args.dump_outputs)
+    eager = BlockStepper(blk, ei, ins, ups, bucket, dev, use_graph=False, warmup=max(args.warmup, 3),
+                         keep_results=keep and not use_graph)
     n0 = lib.pfs_launch_count()
     eager()
     launches_per_step = int(lib.pfs_launch_count() - n0)
-    stepper = BlockStepper(blk, ei, ins, ups, bucket, dev, use_graph=True, warmup=1) if use_graph else eager
+    stepper = BlockStepper(blk, ei, ins, ups, bucket, dev, use_graph=True, warmup=1, keep_results=keep) if use_graph else eager
     for _ in range(max(args.warmup, 3)):
         stepper()
     sampler = ClockSampler(local_rank)
     sampler.start()
     ms = timed(stepper, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, stepper.results)
     ms_per_step = ms / args.steps
     edges_total = float(E) * G * world
     value = edges_total / (ms_per_step * 1e-3)
@@ -527,7 +565,7 @@ def run_ours(args):
         sets = [ins, [torch.empty_like(x) for x in ins]]
         pool = stepper.graph.pool() if use_graph else None
         steppers = [stepper, BlockStepper(blk, ei, sets[1], ups, bucket, dev, use_graph=use_graph, warmup=1, pool=pool)]
-        ms_e = pipelined_e2e(dev, host, sets, steppers, timed, max(3, args.steps))
+        ms_e = pipelined_e2e(dev, host, sets, steppers, timed, args.steps)
         e2e = {"value": edges_total / (ms_e * 1e-3), "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4,
                "ms_per_step": ms_e, "pipelined": E2E_NOTE, "h2d_gbs_per_gpu": h2d / (ms_e * 1e-3) / 1e9,
                "result_read_back": "sum of the updated global features (4 bytes), as a training loop reads its loss"}
@@ -863,7 +901,7 @@ def wide_record(args, workload, world, rank, local_rank, dev, steps, warmup, wit
 
         sets = [detached, [torch.empty_like(x) for x in detached]]
         ms_e = pipelined_e2e(dev, host, sets, [lambda: e2e_step(sets[0]), lambda: e2e_step(sets[1])],
-                             lambda fn, k: timed(fn, k)[0], max(3, steps))
+                             lambda fn, k: timed(fn, k)[0], steps)
         e2e = {"value": edges_total / (ms_e * 1e-3), "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4,
                "ms_per_step": ms_e, "pipelined": E2E_NOTE}
     cpu = None

@@ -4,7 +4,7 @@ Restates `softfloor` (/root/reference/src/train.py:21-27) and `loss_function` (s
 pure functions of the edge times (the output of `GNN.edge_prediction`, src/train.py:42), the uniform
 noise the reference draws with `torch.rand_like` (src/train.py:22) and the class table; the constants
 of src/config.py:16-28 are arguments.  Any floating dtype; gradients by autograd, like the reference.
-Only tests/ may import it.  PARITY PIN: tests/golden/loss_cases.pt, produced by oracle/make_golden_loss.py
+Only tests/ may import it.  PARITY PIN: tests/golden/loss_cases_f64.pt / loss_cases_f32.pt, produced by oracle/make_golden_loss.py
 from the UNMODIFIED reference functions (tests/test_oracle_golden.py::test_loss_oracle_matches_reference).
 """
 import math

@@ -127,7 +127,6 @@ def run_gnn_case(ref, S, seed):
 def main():
     ref = load_reference_gnn()
     os.makedirs(OUT_DIR, exist_ok=True)
-    cases = {}
     spec = [
         # name,                F,  S,  T, kind,                   seed, training, extra
         ("dense_train",        10, 40, 12, "dense",                11, True, {}),
@@ -144,10 +143,12 @@ def main():
         ("sparse_eval",        10, 45, 12, "sparse",               25, False, {}),
         ("duplicates_train",   10, 25, 6, "duplicates",            26, True, {}),
     ]
+    os.makedirs(os.path.join(OUT_DIR, "block_cases"), exist_ok=True)
     for name, F, S, T, kind, seed, training, extra in spec:
-        cases[name] = run_block_case(ref, F, S, T, kind, seed, training, **extra)
-        print("block case", name, "E =", cases[name]["edge_index"].shape[1])
-    torch.save(cases, os.path.join(OUT_DIR, "block_cases.pt"))
+        case = run_block_case(ref, F, S, T, kind, seed, training, **extra)
+        # one file per case keeps every golden file under 1 MB
+        torch.save(case, os.path.join(OUT_DIR, "block_cases", name + ".pt"))
+        print("block case", name, "E =", case["edge_index"].shape[1])
     gnn_case = run_gnn_case(ref, S=64, seed=31)
     torch.save(gnn_case, os.path.join(OUT_DIR, "gnn_shipped_weights.pt"))
     for f in os.listdir(OUT_DIR):

@@ -6,7 +6,8 @@ Calls the UNMODIFIED `train.loss_function` (/root/reference/src/train.py:29-80) 
 `gnn` whose `edge_prediction` returns preset edge times (the loss reads the model only through that call,
 src/train.py:42) and with the config globals NFIBERS / NCLASSES overridden for small cases.  The noise the reference
 draws inside `softfloor` (torch.rand_like, src/train.py:22) is reproduced by seeding the default generator identically
-and recorded next to the outputs.  Writes tests/golden/loss_cases.pt.
+and recorded next to the outputs.  Writes tests/golden/loss_cases_f64.pt and loss_cases_f32.pt (one file per
+dtype keeps each under 1 MB).
 """
 import os
 import sys
@@ -19,7 +20,7 @@ sys.path.insert(0, os.path.dirname(HERE))
 from oracle import block_oracle as bo  # noqa: E402
 from oracle.ref_loader import load_reference_train  # noqa: E402
 
-OUT = os.path.join(os.path.dirname(HERE), "tests", "golden", "loss_cases.pt")
+OUT_DIR = os.path.join(os.path.dirname(HERE), "tests", "golden")
 
 
 class _Stub:
@@ -59,12 +60,12 @@ def run_case(train, S, T, seed, dtype, spread):
 
 def main():
     train = load_reference_train()
-    cases = []
-    for S, T, seed, spread in ((50, 12, 1, 6.0), (2000, 12, 2, 7.0), (64, 16, 3, 40.0), (37, 4, 4, 3.0)):
-        for dtype in (torch.float64, torch.float32):
-            cases.append(run_case(train, S, T, seed, dtype, spread))
-    torch.save(cases, OUT)
-    print("wrote %d cases to %s (%.1f KB)" % (len(cases), OUT, os.path.getsize(OUT) / 1e3))
+    for dtype, tag in ((torch.float64, "f64"), (torch.float32, "f32")):
+        cases = [run_case(train, S, T, seed, dtype, spread)
+                 for S, T, seed, spread in ((50, 12, 1, 6.0), (2000, 12, 2, 7.0), (64, 16, 3, 40.0), (37, 4, 4, 3.0))]
+        out = os.path.join(OUT_DIR, "loss_cases_%s.pt" % tag)
+        torch.save(cases, out)
+        print("wrote %d cases to %s (%.1f KB)" % (len(cases), out, os.path.getsize(out) / 1e3))
 
 
 if __name__ == "__main__":

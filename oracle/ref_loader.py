@@ -10,9 +10,9 @@ import sys
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _SHIM = os.path.join(_HERE, "ref_shim")
-# Where the unmodified reference may live: an explicit override, the build container's read-only checkout, or the verbatim
-# copy of src/gnn.py + src/config.py that __graft_entry__.build() vendors under baseline/_ref/ (git-ignored; it travels to
-# the GPU box with the snapshot, which has no /root/reference) -- SURVEY.md section 8c, BASELINE.md section 4.
+# Where the unmodified reference may live: an explicit override (PFS_REFERENCE_ROOT), a checkout of the reference, or a
+# verbatim copy of its src/gnn.py + src/config.py under baseline/_ref/ (git-ignored) -- SURVEY.md section 8c, BASELINE.md
+# section 4.
 VENDORED_ROOT = os.path.join(os.path.dirname(_HERE), "baseline", "_ref")
 
 
@@ -28,25 +28,6 @@ REFERENCE_ROOT = _find_root()
 
 def reference_available():
     return os.path.isfile(os.path.join(REFERENCE_ROOT, "src", "gnn.py"))
-
-
-def vendor_reference(src_root="/root/reference"):
-    """Verbatim copy of the two files the path needs (src/gnn.py, src/config.py) into baseline/_ref/src/, so that the CPU
-    arm of bench.py can time the UNMODIFIED reference on a box without /root/reference.  Returns True when the copy is
-    in place.  Called by __graft_entry__.build() in the build container; never touches tracked files."""
-    import filecmp
-    import shutil
-    ok = True
-    for name in ("gnn.py", "config.py"):
-        src = os.path.join(src_root, "src", name)
-        dst = os.path.join(VENDORED_ROOT, "src", name)
-        if not os.path.isfile(src):
-            ok = ok and os.path.isfile(dst)
-            continue
-        os.makedirs(os.path.dirname(dst), exist_ok=True)
-        if not (os.path.isfile(dst) and filecmp.cmp(src, dst, shallow=False)):
-            shutil.copyfile(src, dst)
-    return ok and os.path.isfile(os.path.join(VENDORED_ROOT, "src", "gnn.py"))
 
 
 @contextlib.contextmanager

@@ -15,7 +15,9 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def golden_block_cases():
     import torch
-    return torch.load(os.path.join(ROOT, "tests", "golden", "block_cases.pt"), map_location="cpu", weights_only=False)
+    d = os.path.join(ROOT, "tests", "golden", "block_cases")      # one file per case, keyed by its name
+    return {f[:-len(".pt")]: torch.load(os.path.join(d, f), map_location="cpu", weights_only=False)
+            for f in sorted(os.listdir(d)) if f.endswith(".pt")}
 
 
 @pytest.fixture(scope="session")

@@ -1,13 +1,12 @@
 """GPU parity of the training-loss kernels (reference src/train.py:21-80; SURVEY.md 8f row N1) against the golden
 vectors of the unmodified reference and against the fp64 oracle: loss terms to rtol 1e-4 (fp32), gradient w.r.t. the
 edge times norm-wise 1e-4, bit-reproducible run to run."""
-import os
-
 import pytest
 import torch
 
 from oracle import block_oracle as bo
 from oracle import loss_oracle as lo
+from tests.util import golden_loss_cases
 
 pytestmark = pytest.mark.gpu
 
@@ -19,8 +18,7 @@ def _dev():
 
 
 def _cases():
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "loss_cases.pt")
-    return [c for c in torch.load(path) if c["time"].dtype == torch.float64]
+    return [c for c in golden_loss_cases() if c["time"].dtype == torch.float64]
 
 
 def _rel(a, b):

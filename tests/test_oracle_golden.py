@@ -1,12 +1,10 @@
 """Pins oracle/block_oracle.py (the CPU restatement) against outputs of the UNMODIFIED reference:
-committed golden vectors (tests/golden, made by oracle/make_golden.py) and, when /root/reference
-is present (build container only), the imported reference modules live."""
+committed golden vectors (tests/golden, made by oracle/make_golden.py)."""
 import pytest
 import torch
 
 from oracle import block_oracle as bo
-from oracle.ref_loader import reference_available, load_reference_gnn
-from tests.util import nerr, run_oracle_block, upstream
+from tests.util import golden_loss_cases, nerr, run_oracle_block
 
 CASES = ["dense_train", "dense_eval", "dense_train_u0", "dense_train_T5", "dense_train_F16", "dense_train_F4",
          "dense_unnormed", "permuted_train", "class_major_train", "shuffled_train", "sparse_train", "sparse_eval",
@@ -45,13 +43,7 @@ def test_double_norm_is_pinned(golden_block_cases):
 
 def test_gnn_shipped_weights_fp64(golden_gnn_case):
     case = golden_gnn_case
-    ck_state = None
-    if reference_available():
-        ck_state = torch.load("/root/reference/params/model_gnn_0.pth", map_location="cpu",
-                              weights_only=False)["model_state"]
-    else:
-        pytest.skip("shipped checkpoint only exists in the build container")
-    sd = bo.cast_state(ck_state, torch.float64)
+    sd = bo.cast_state(case["state"], torch.float64)      # the reference's shipped checkpoint, stored with its outputs
     for training in (True, False):
         x_s, x_t, x_e, u = bo.gnn_forward(sd, 3, case["edge_index"], case["x_s"], case["x_t"], case["x_e"], case["u"],
                                           training=training, buffers={})
@@ -62,24 +54,6 @@ def test_gnn_shipped_weights_fp64(golden_gnn_case):
         assert nerr(x_t, gold["x_t"]) < 1e-9
         assert nerr(u, gold["u"]) < 1e-9
         assert nerr(time, gold["time"]) < 1e-9
-
-
-@pytest.mark.skipif(not reference_available(), reason="/root/reference only exists in the build container")
-def test_restatement_matches_live_reference():
-    ref = load_reference_gnn()
-    torch.manual_seed(5)
-    F, S, T = 10, 37, 12
-    sd = bo.random_block_state(F, seed=77, dtype=torch.float64)
-    blk = ref.Block(F).double()
-    blk.load_state_dict(sd, strict=True)
-    blk.train()
-    edge_index = bo.complete_bipartite(S, T)[:, torch.randperm(S * T)[: S * T // 2]]
-    x_s, x_t = torch.randn(S, F, dtype=torch.float64), torch.randn(T, F, dtype=torch.float64)
-    x_e, u = torch.randn(edge_index.shape[1], F, dtype=torch.float64), torch.randn(1, F, dtype=torch.float64)
-    _, r_s, r_t, r_e, r_u = blk((edge_index, x_s, x_t, x_e, u))
-    o_s, o_t, o_e, o_u = bo.block(sd, "", edge_index, x_s, x_t, x_e, u, training=True, buffers={})
-    for a, b in ((o_s, r_s), (o_t, r_t), (o_e, r_e), (o_u, r_u)):
-        assert nerr(a, b) < 1e-10
 
 
 def test_integer_time_definition():
@@ -94,15 +68,9 @@ def test_integer_time_definition():
 # ---------------------------------------------------------------------------------------------
 # training loss (SURVEY.md section 8f row N1): oracle/loss_oracle.py against the unmodified reference
 # ---------------------------------------------------------------------------------------------
-def _loss_cases():
-    import os
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "loss_cases.pt")
-    return torch.load(path)
-
-
 def test_loss_oracle_matches_reference():
     from oracle import loss_oracle as lo
-    cases = _loss_cases()
+    cases = golden_loss_cases()
     assert len(cases) == 8
     for c in cases:
         S, T = c["S"], c["T"]

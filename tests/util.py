@@ -1,5 +1,14 @@
 """Shared helpers for the parity tests (norm-wise error metric of SURVEY.md section 4.3)."""
+import os
+
 import torch
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def golden_loss_cases():
+    """The reference's training loss on four cases in fp64, then the same four in fp32 (oracle/make_golden_loss.py)."""
+    return [c for tag in ("f64", "f32") for c in torch.load(os.path.join(GOLDEN, "loss_cases_%s.pt" % tag))]
 
 
 def upstream(t):
