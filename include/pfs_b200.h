@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define PFS_ABI_VERSION 5
+#define PFS_ABI_VERSION 6
 
 enum {
     PFS_OK = 0,
@@ -100,8 +100,6 @@ int pfs_profile_report(char* buf, size_t buflen);
 
 /* Workspace (bytes) sufficient for any forward/backward call on this topology. */
 size_t pfs_workspace_bytes(const pfs_topology* topo);
-/* Edge tiles per graph of this topology (rows of the per-tile statistics buffers edge_bn_stat / bn_stat_in). */
-int32_t pfs_stat_tiles(const pfs_topology* topo);
 
 /* -------------------------------------------------------------------------------------------
  * topology (replaces the implicit advanced-indexing / torch_scatter index handling of
@@ -138,10 +136,6 @@ typedef struct pfs_edge_args {
     /* forward outputs */
     float* x_e_out;                              /* [G,E,F] */
     float* bn_save;                              /* [G,4,F]: mean, biased var, combined scale, shift */
-    float* act_save;                             /* optional [G,E,4F]: hidden activations lrelu(h1) in tile (fibre-sorted) order.
-                                                    Non-NULL: the forward stores them and the backward reads them back instead of
-                                                    recomputing the first layer (+16F bytes per edge of HBM for ~30 % fewer
-                                                    instructions in the backward); NULL: recompute */
     /* backward inputs (x_e_out and bn_save as written by the forward) */
     const float* g_out;                          /* dL/dx_e_out [G,E,F] */
     /* backward outputs (overwritten) */
@@ -158,10 +152,6 @@ typedef struct pfs_edge_args {
     float *table_s, *table_t;                    /* optional [G,S,4F], [G,T,4F]: node tables of the first-layer split.  The
                                                     forward writes them here instead of its workspace; a backward given the
                                                     same buffers reads them instead of recomputing them */
-    const float* bn_stat_in;                     /* optional, backward, train mode: [G*tiles][2F] per-tile sums of g_out and
-                                                    g_out (x_e_out - beta) written by the call that produced g_out
-                                                    (pfs_source_args.edge_bn_stat, same topology): the statistics pass over
-                                                    g_out and x_e_out is skipped */
 } pfs_edge_args;
 int pfs_edge_fwd(const pfs_edge_args* a);
 int pfs_edge_bwd(const pfs_edge_args* a);
@@ -185,8 +175,6 @@ typedef struct pfs_source_args {
     float* hidden;                               /* [G,S,10F] saved: lrelu of the node MLP hidden layer */
     float* y_pre;                                /* [G,S,F] saved: node MLP output before the norm */
     float* bn_save;                              /* [G,4,F] */
-    float* act_save;                             /* optional [G,E,2F]: hidden activations of the message MLP (tile order), see pfs_edge_args */
-    float* msg_save;                             /* optional [G,E,2F]: the messages m; both or neither */
     const float* g_out;                          /* dL/dx_s_out [G,S,F] */
     const float* g_x_e_add;                      /* optional [G,E,F]: g_x_e = (this module's dL/dx_e) + g_x_e_add, fused into the store */
     float *g_x_s, *g_x_t, *g_x_e, *g_u;
@@ -198,11 +186,6 @@ typedef struct pfs_source_args {
                                                     x_e then holds the pre-norm z, and the edge pass stores
                                                     x_e' = scale z + shift back into x_e_norm_out as it goes */
     float* x_e_norm_out;                         /* [G,E,F], may alias x_e (every row is read and written by one thread) */
-    const float* edge_bn_shift;                  /* optional, backward: the EdgeModel's norm.bias [F] ... */
-    float* edge_bn_stat;                         /* ... and [G*tiles][2F] (tiles = pfs_stat_tiles(topo)): the edge pass, which
-                                                    stores the complete gradient of x_e (its own + g_x_e_add), also emits the
-                                                    per-tile sums of g and g (x_e - shift) the EdgeModel's BatchNorm backward
-                                                    needs (pfs_edge_args.bn_stat_in) */
 } pfs_source_args;
 int pfs_source_fwd(const pfs_source_args* a);
 int pfs_source_bwd(const pfs_source_args* a);
@@ -225,7 +208,6 @@ typedef struct pfs_target_args {
     float* act_sum;                              /* [G,T,2F] saved: per-class sum of the hidden activations */
     float* y_pre;                                /* [G,T,F] saved */
     float* bn_save;                              /* [G,4,F] */
-    float* act_save;                             /* optional [G,E,2F]: hidden activations of the message MLP (tile order), see pfs_edge_args */
     const float* g_out;                          /* dL/dx_t_out [G,T,F] */
     const float* g_x_e_add;                      /* optional [G,E,F]: g_x_e = (this module's dL/dx_e) + g_x_e_add, fused into the store */
     float *g_x_s, *g_x_t, *g_x_e, *g_u;

@@ -18,7 +18,7 @@ HEADER = os.path.join(os.path.dirname(_HERE), "include", "pfs_b200.h")
 PFS_LAYOUT_DENSE = 0
 PFS_LAYOUT_CSR = 1
 PFS_TILE_EDGES = 256
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 _P = ct.c_void_p
 
@@ -46,11 +46,11 @@ class EdgeArgs(ct.Structure):
         (_P, "x_s x_t x_e u w1 b1 w2 b2 gamma beta running_mean running_var num_batches_tracked"),
         (ct.c_int32, "training normed"),
         (ct.c_float, "eps momentum"),
-        (_P, "x_e_out bn_save act_save g_out g_x_s g_x_t g_x_e g_u g_w1 g_b1 g_w2 g_b2 g_gamma g_beta workspace"),
+        (_P, "x_e_out bn_save g_out g_x_s g_x_t g_x_e g_u g_w1 g_b1 g_w2 g_b2 g_gamma g_beta workspace"),
         (ct.c_size_t, "workspace_bytes"),
         (_P, "stream"),
         (ct.c_int32, "defer_affine reserved0"),
-        (_P, "table_s table_t bn_stat_in"),
+        (_P, "table_s table_t"),
     ])
 
 
@@ -60,11 +60,11 @@ class SourceArgs(ct.Structure):
         (_P, "x_s x_t x_e u w1 b1 w2 b2 w3 b3 w4 b4 gamma beta running_mean running_var num_batches_tracked"),
         (ct.c_int32, "training normed"),
         (ct.c_float, "eps momentum"),
-        (_P, "x_s_out moments hidden y_pre bn_save act_save msg_save g_out g_x_e_add g_x_s g_x_t g_x_e g_u "
+        (_P, "x_s_out moments hidden y_pre bn_save g_out g_x_e_add g_x_s g_x_t g_x_e g_u "
              "g_w1 g_b1 g_w2 g_b2 g_w3 g_b3 g_w4 g_b4 g_gamma g_beta workspace"),
         (ct.c_size_t, "workspace_bytes"),
         (_P, "stream"),
-        (_P, "x_e_affine x_e_norm_out edge_bn_shift edge_bn_stat"),
+        (_P, "x_e_affine x_e_norm_out"),
     ])
 
 
@@ -74,7 +74,7 @@ class TargetArgs(ct.Structure):
         (_P, "x_s x_t x_e u w1 b1 w2 b2 w3 b3 w4 b4 gamma beta running_mean running_var num_batches_tracked"),
         (ct.c_int32, "training normed"),
         (ct.c_float, "eps momentum"),
-        (_P, "x_t_out act_sum y_pre bn_save act_save g_out g_x_e_add g_x_s g_x_t g_x_e g_u "
+        (_P, "x_t_out act_sum y_pre bn_save g_out g_x_e_add g_x_s g_x_t g_x_e g_u "
              "g_w1 g_b1 g_w2 g_b2 g_w3 g_b3 g_w4 g_b4 g_gamma g_beta workspace"),
         (ct.c_size_t, "workspace_bytes"),
         (_P, "stream"),
@@ -150,7 +150,6 @@ SYMBOLS = {
     "pfs_profile_enable": (ct.c_int, [ct.c_int]),
     "pfs_profile_report": (ct.c_int, [ct.c_char_p, ct.c_size_t]),
     "pfs_workspace_bytes": (ct.c_size_t, [ct.POINTER(TopologyStruct)]),
-    "pfs_stat_tiles": (_I32, [ct.POINTER(TopologyStruct)]),
     "pfs_detect_dense": (ct.c_int, [_P, _I64, _I32, _I32, _P, _P]),
     "pfs_build_topology_temp_bytes": (ct.c_size_t, [_I64, _I32, _I32]),
     "pfs_build_topology": (ct.c_int, [_P, _I64, _I32, _I32] + [_P] * 9 + [_P, ct.c_size_t, _P]),

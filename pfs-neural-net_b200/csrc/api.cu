@@ -12,10 +12,8 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #include "edge_model.cuh"
-#include "edge_fwd_tc.cuh"
 #include "node_ops.cuh"
 #include "source_model.cuh"
-#include "source_node_c.cuh"
 #include "source_node_mma.cuh"
 #include "source_node_bwd_mma.cuh"
 #include "target_model.cuh"
@@ -190,7 +188,14 @@ int dense_ntiles(int S, int T) {
     const int fpt = dense_fpt(T);
     return fpt > 0 ? (S + fpt - 1) / fpt : 0;
 }
-// node tiles: constant-bank kernels (Fdim <= 10) use 128-fibre tiles, the shared-memory kernels node_rows<F>()
+// node-MLP route per Fdim: 4, 8 and 10 on the tensor-core kernels with W4 in the constant bank (source_node_mma.cuh,
+// source_node_bwd_mma.cuh), 16 on the shared-memory kernels (source_model.cuh)
+template <int F> constexpr bool node_route_mma(bool mma) {
+    return SourceNodeConst<F>::fits == mma && SourceNodeMma<F>::fits == mma && SourceNodeBwdMma<F>::fits == mma;
+}
+static_assert(node_route_mma<4>(true) && node_route_mma<8>(true) && node_route_mma<10>(true) && node_route_mma<16>(false),
+              "node-MLP kernel route per Fdim");
+// node tiles: the tensor-core forward uses 128-fibre tiles, the shared-memory kernels node_rows<F>()
 template <int F> constexpr int node_tile_rows() { return SourceNodeConst<F>::fits ? kNodeRowsC : node_rows<F>(); }
 template <int F> int node_ntiles(int S) { return (S + node_tile_rows<F>() - 1) / node_tile_rows<F>(); }
 
@@ -258,48 +263,6 @@ int run_prep(int G, const TableJob* jobs, int njobs, const float* W, int ldw, co
     if (pl.n > 0)
         PFS_CUDA(cudaMemcpyToSymbolAsync(c_w, wstage, sizeof(float) * (size_t)nfloats, 0, cudaMemcpyDeviceToDevice, st));
     return PFS_OK;
-}
-
-// PFS_NODE_MMA=0 switches the fibre MLP back from the tcgen05 kernel to the FMA kernel (A/B runs)
-bool node_mma_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("PFS_NODE_MMA");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
-}
-
-// PFS_NODE_BWD_MMA=0 keeps the tensor-core forward but runs the fibre MLP backward on the FMA kernel
-bool node_bwd_mma_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("PFS_NODE_BWD_MMA");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1 && node_mma_enabled();
-}
-
-// PFS_EDGE_TC=1 runs the EdgeModel forward of the dense layout on the tcgen05 kernel (edge_fwd_tc.cuh) instead of the
-// FFMA2 kernel.  Off by default: measured at C3 (profiles/r02_edge_tc_vs_fma.txt) the tensor-core version takes 0.75 ms
-// against 0.40 ms -- at K = 10 / 40, N = 40 / 10 the MMAs are bound by re-reading the 128-row A operand from shared
-// memory and by the per-tile issue -> commit -> tcgen05.ld round trips, not by the tensor pipe.
-bool edge_tc_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("PFS_EDGE_TC");
-        v = (e && e[0] == '1') ? 1 : 0;
-    }
-    return v == 1;
-}
-
-bool edge_bwd_lean_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("PFS_EDGE_BWD_LEAN");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
 }
 
 // staging geometry of the edge kernels (common.cuh: TileStage)
@@ -509,31 +472,10 @@ int edge_fwd_impl(const pfs_edge_args& a, const Topo& tp) {
     const int max_fib = max_fibres_per_tile(tp);
     const bool sc = stage_class_table(tp, H);
     size_t smem = 0;
-    // dense layout: both MLP layers on tcgen05 (edge_fwd_tc.cuh) when the tile's node-table rows fit its register
-    // prefetch (2 float4 of P_s rows and 1 of P_t per thread)
-    using TC = EdgeFwdTc<F>;
-    const bool tc = TC::fits && tp.layout == PFS_LAYOUT_DENSE && edge_tc_enabled() && max_fib * (H / 4) <= 2 * kThreads &&
-                    tp.T * (H / 4) <= kThreads && sizeof(float) * TC::floats(max_fib, tp.T) <= kSmemLimit;
-    int nbuf = 1;
-    if (tc) {
-        smem = sizeof(float) * TC::floats(max_fib, tp.T);
-        PFS_TRY(allow_smem(k_edge_fwd_tc<F>, smem));
-    } else {
-        nbuf = pick_nbuf([&](int nb) { return sizeof(float) * TileStage<F, 1, H, H>::floats(max_fib, tp.T, sc, nb); }, smem);
-        if (!nbuf) return fail(PFS_ERR_UNSUPPORTED, "edge_fwd: tile staging does not fit shared memory");
-        PFS_TRY(allow_smem(k_edge_fwd<F>, smem));
-    }
-    // the occupancy calculator reports 1 CTA per SM for a kernel that allocates tensor memory whatever its footprint
-    // (measured: 128 registers, 99 KB -> 1; the FFMA2 kernel with 128 registers, 113 KB -> 2); the tcgen05 kernel takes
-    // 128 of the 512 TMEM columns, so two (three where shared memory allows) CTAs do fit
-    int grid;
-    if (tc) {
-        const int per_sm = smem <= 75 * 1024 ? 3 : smem <= 113 * 1024 ? 2 : 1;
-        grid = per_sm * num_sms();
-        if (grid > total) grid = total;
-    } else {
-        grid = persistent_grid(k_edge_fwd<F>, smem, total);
-    }
+    const int nbuf = pick_nbuf([&](int nb) { return sizeof(float) * TileStage<F, 1, H, H>::floats(max_fib, tp.T, sc, nb); }, smem);
+    if (!nbuf) return fail(PFS_ERR_UNSUPPORTED, "edge_fwd: tile staging does not fit shared memory");
+    PFS_TRY(allow_smem(k_edge_fwd<F>, smem));
+    const int grid = persistent_grid(k_edge_fwd<F>, smem, total);
     const int nrec = chunk_records(grid, total, tp.ntiles);
     Bump ws(a.workspace, a.workspace_bytes);
     float* uvec = ws.f((size_t)tp.G * H);
@@ -547,22 +489,15 @@ int edge_fwd_impl(const pfs_edge_args& a, const Topo& tp) {
     TableJob jobs[2];
     edge_table_jobs<F>(a, tp, Ps, Pt, jobs);
     PackList pl{};
-    if (!tc) {
-        pl.it[0] = PackItem{a.w1, H, 2 * F, F, H, 1, 0};            // W1_e input-major [F][H]
-        pl.it[1] = PackItem{a.w2, H, 0, H, F, 1, F * H};            // W2 input-major [H][F]
-        pl.it[2] = PackItem{a.b2, 1, 0, 1, F, 0, 2 * F * H};        // b2
-        pl.n = 3;
-    }
+    pl.it[0] = PackItem{a.w1, H, 2 * F, F, H, 1, 0};            // W1_e input-major [F][H]
+    pl.it[1] = PackItem{a.w2, H, 0, H, F, 1, F * H};            // W2 input-major [H][F]
+    pl.it[2] = PackItem{a.b2, 1, 0, 1, F, 0, 2 * F * H};        // b2
+    pl.n = 3;
     PFS_TRY((run_prep<F, H>(tp.G, jobs, 2, a.w1, H, a.u, pl, 2 * F * H + F, wstage, st)));
     const bool stats = a.normed && a.training;
-    EdgeFwdParams p{tp, a.x_e, Ps, Pt, a.w1, a.w2, a.b2, a.x_e_out, stats ? part : nullptr, max_fib, sc ? 1 : 0, nrec, nbuf, a.act_save};
-    if (tc) {
-        k_edge_fwd_tc<F><<<grid, kThreads, smem, st>>>(p);     // weights go straight from global into the MMA operands
-        PFS_LAUNCH_CHECK("k_edge_fwd_tc");
-    } else {
-        k_edge_fwd<F><<<grid, kThreads, smem, st>>>(p);
-        PFS_LAUNCH_CHECK("k_edge_fwd");
-    }
+    EdgeFwdParams p{tp, a.x_e, Ps, Pt, a.w1, a.w2, a.b2, a.x_e_out, stats ? part : nullptr, max_fib, sc ? 1 : 0, nrec, nbuf};
+    k_edge_fwd<F><<<grid, kThreads, smem, st>>>(p);
+    PFS_LAUNCH_CHECK("k_edge_fwd");
     if (a.normed) {
         PFS_REQUIRE(a.gamma && a.beta && a.bn_save, "normed edge model needs gamma, beta, bn_save");
         PFS_TRY(bn_forward_tail(F, tp.G, tp.E, part, tp.ntiles, 1, a.training, a.gamma, a.beta, a.running_mean,
@@ -582,11 +517,10 @@ int edge_bwd_impl(const pfs_edge_args& a, const Topo& tp) {
     const int mode = !a.normed ? 0 : (a.training ? 1 : 2);
     using SM = EdgeBwdSmem<F>;
     // k_edge_bwd2 (two CTAs per SM: x_e staged only, hidden layer in two halves, shared accumulator registers) where
-    // its tiles fit 113 KB; PFS_EDGE_BWD_LEAN=0 selects the double-buffered one-CTA-per-SM kernel (A/B runs).
+    // its tiles fit 113 KB, else the double-buffered one-CTA-per-SM k_edge_bwd (Fdim 16).
     // Measured at C3: 1.21 ms against 1.60 ms.
-    const bool lean = SM::lean_fits && edge_bwd_lean_enabled();
-    const bool saved = lean && a.act_save != nullptr;      // hidden activations saved by the forward: no recompute, no node tables
-    auto kern = lean ? (saved ? k_edge_bwd2<F, true> : k_edge_bwd2<F, false>) : k_edge_bwd<F>;
+    constexpr bool lean = SM::lean_fits;
+    auto kern = lean ? k_edge_bwd2<F> : k_edge_bwd<F>;
     const int max_fib = max_fibres_per_tile(tp);
     const bool sc = stage_class_table(tp, H);
     size_t smem_bwd = SM::bytes_lean;
@@ -628,24 +562,20 @@ int edge_bwd_impl(const pfs_edge_args& a, const Topo& tp) {
         pl.it[1] = PackItem{a.w2, H, 0, H, F, 0, CW::kW2o};         // W2 as stored [F][H]
         pl.it[2] = PackItem{a.w1, H, 2 * F, F, H, 0, CW::kW1o};     // W1_e as stored [H][F]
         pl.n = 3;
-        PFS_TRY((run_prep<F, H>(tp.G, jobs, (saved || cached) ? 0 : 2, a.w1, H, a.u, pl, CW::kFloats, wstage, st)));
+        PFS_TRY((run_prep<F, H>(tp.G, jobs, cached ? 0 : 2, a.w1, H, a.u, pl, CW::kFloats, wstage, st)));
     }
     const int n = tp.G * F;
-    // statistics of the incoming gradient taken by the kernel that stored it (pfs_source_bwd, edge_bn_stat): train mode only
-    const bool stats_in = a.bn_stat_in != nullptr && mode == 1;
-    k_edge_bn_bwd_coef<<<(n + 127) / 128, 128, 0, st>>>(0, mode, 0, F, tp.G, tp.ntiles, tp.E, a.bn_save, a.gamma, a.beta,
+    k_edge_bn_bwd_coef<<<(n + 127) / 128, 128, 0, st>>>(0, mode, F, tp.G, tp.ntiles, tp.E, a.bn_save, a.gamma, a.beta,
                                                          a.running_mean, a.running_var, a.eps, statsum, coef, dgb);
     PFS_LAUNCH_CHECK("k_edge_bn_bwd_coef/0");
     if (mode != 0) {
-        if (!stats_in) {
-            EdgeBnStatParams sp{tp, a.x_e_out, a.g_out, coef, statp};
-            const int g2 = persistent_grid(k_edge_bn_bwd_stats<F>, 0, total);
-            k_edge_bn_bwd_stats<F><<<g2, kThreads, 0, st>>>(sp);
-            PFS_LAUNCH_CHECK("k_edge_bn_bwd_stats");
-        }
-        k_tile_partial_sums<<<tp.G, 256, 0, st>>>(stats_in ? a.bn_stat_in : statp, tp.ntiles, 2 * F, statsum);
+        EdgeBnStatParams sp{tp, a.x_e_out, a.g_out, coef, statp};
+        const int g2 = persistent_grid(k_edge_bn_bwd_stats<F>, 0, total);
+        k_edge_bn_bwd_stats<F><<<g2, kThreads, 0, st>>>(sp);
+        PFS_LAUNCH_CHECK("k_edge_bn_bwd_stats");
+        k_tile_partial_sums<<<tp.G, 256, 0, st>>>(statp, tp.ntiles, 2 * F, statsum);
         PFS_LAUNCH_CHECK("k_tile_partial_sums");
-        k_edge_bn_bwd_coef<<<(n + 127) / 128, 128, 0, st>>>(1, mode, stats_in ? 1 : 0, F, tp.G, tp.ntiles, tp.E, a.bn_save,
+        k_edge_bn_bwd_coef<<<(n + 127) / 128, 128, 0, st>>>(1, mode, F, tp.G, tp.ntiles, tp.E, a.bn_save,
                                                              a.gamma, a.beta, a.running_mean, a.running_var, a.eps, statsum,
                                                              coef, dgb);
         PFS_LAUNCH_CHECK("k_edge_bn_bwd_coef/1");
@@ -653,8 +583,7 @@ int edge_bwd_impl(const pfs_edge_args& a, const Topo& tp) {
     }
     const bool dense = tp.layout == PFS_LAYOUT_DENSE;
     EdgeBwdParams p{tp, a.x_e, a.x_e_out, a.g_out, Ps, Pt, coef, a.g_x_e, dPs,
-                    dense ? stage : nullptr, dense ? nullptr : stage, wpart, pstride, max_fib, sc ? 1 : 0, nbuf,
-                    saved ? a.act_save : nullptr};
+                    dense ? stage : nullptr, dense ? nullptr : stage, wpart, pstride, max_fib, sc ? 1 : 0, nbuf};
     kern<<<grid, kThreads, smem_bwd, st>>>(p);
     if (lean) {
         PFS_LAUNCH_CHECK("k_edge_bwd2");
@@ -702,19 +631,16 @@ int source_fwd_impl(const pfs_source_args& a, const Topo& tp) {
         int nfloats = MsgEdgeConst<F>::kFloats;
         if constexpr (SourceNodeConst<F>::fits) {
             using CW = SourceNodeConst<F>;
-            constexpr int J = 10 * F, K9 = 9 * F;
-            const bool mma = SourceNodeMma<F>::fits && node_mma_enabled();
+            constexpr int J = 10 * F;
             pl.it[pl.n++] = PackItem{a.w4, J, 0, J, F, 1, CW::kW4t};       // W4 input-major [J][F]
             pl.it[pl.n++] = PackItem{a.b4, 1, 0, 1, F, 0, CW::kB4};
-            if (!mma) pl.it[pl.n++] = PackItem{a.w3, J, 0, K9, J, 1, CW::kW3t};      // W3[:, :9F] input-major [K9][J] (FMA kernel)
-            nfloats = mma ? CW::kFwdMmaFloats : CW::kFwdFloats;
+            nfloats = CW::kFwdMmaFloats;
         }
         PFS_TRY((run_prep<F, M>(tp.G, jobs, 1, a.w1, M, a.u, pl, nfloats, wstage, st)));
     }
     {
-        PFS_REQUIRE((a.act_save == nullptr) == (a.msg_save == nullptr), "act_save and msg_save go together");
         if (a.x_e_affine) PFS_REQUIRE(a.x_e_norm_out, "x_e_affine needs x_e_norm_out");
-        SourceEdgeFwdParams p{tp, a.x_e, Qt, a.w1, a.w2, a.b2, a.moments, a.act_save, a.msg_save, a.x_e_affine, a.x_e_norm_out};
+        SourceEdgeFwdParams p{tp, a.x_e, Qt, a.w1, a.w2, a.b2, a.moments, a.x_e_affine, a.x_e_norm_out};
         const int grid = persistent_grid(k_source_edge_fwd<F>, 0, total);
         k_source_edge_fwd<F><<<grid, kThreads, 0, st>>>(p);
         PFS_LAUNCH_CHECK("k_source_edge_fwd");
@@ -724,22 +650,13 @@ int source_fwd_impl(const pfs_source_args& a, const Topo& tp) {
         SourceNodeFwdParams p{tp.G, tp.S, a.x_s, a.u, a.moments, a.w3, a.b3, a.w4, a.b4, a.hidden, a.y_pre,
                               stats ? partn : nullptr, ntn};
         if constexpr (SourceNodeConst<F>::fits) {
-            using SM = SourceNodeFwdSmemC<F>;
-            if (SourceNodeMma<F>::fits && node_mma_enabled()) {
-                // first layer on tcgen05 (3xTF32), see source_node_mma.cuh
-                auto kern = k_source_node_fwd_mma<F>;
-                constexpr size_t smem = SourceNodeMma<F>::bytes;
-                PFS_TRY(allow_smem(kern, smem));
-                const int grid = persistent_grid(kern, smem, (long long)ntn * tp.G, kNodeThreadsC);
-                kern<<<grid, kNodeThreadsC, smem, st>>>(p);
-                PFS_LAUNCH_CHECK("k_source_node_fwd_mma");
-            } else {
-                auto kern = k_source_node_fwd_c<F>;
-                PFS_TRY(allow_smem(kern, SM::bytes));
-                const int grid = persistent_grid(kern, SM::bytes, (long long)ntn * tp.G, kNodeThreadsC);
-                kern<<<grid, kNodeThreadsC, SM::bytes, st>>>(p);
-                PFS_LAUNCH_CHECK("k_source_node_fwd");
-            }
+            // first layer on tcgen05 (3xTF32), see source_node_mma.cuh
+            auto kern = k_source_node_fwd_mma<F>;
+            constexpr size_t smem = SourceNodeMma<F>::bytes;
+            PFS_TRY(allow_smem(kern, smem));
+            const int grid = persistent_grid(kern, smem, (long long)ntn * tp.G, kNodeThreadsC);
+            kern<<<grid, kNodeThreadsC, smem, st>>>(p);
+            PFS_LAUNCH_CHECK("k_source_node_fwd_mma");
         } else {
             using SM = SourceNodeFwdSmem<F>;
             auto kern = k_source_node_fwd<F>;
@@ -768,26 +685,15 @@ int source_bwd_impl(const pfs_source_args& a, const Topo& tp) {
     const int total = tp.ntiles * tp.G;
     int ntn = node_ntiles<F>(tp.S);
     const int mode = !a.normed ? 0 : (a.training ? 1 : 2);
-    using SME = SourceEdgeBwdSmem<F>;
-    constexpr bool kNodeC = SourceNodeConst<F>::fits;
+    constexpr size_t smem_e = SourceEdgeBwdSmem<F>::bytes;
     constexpr bool kNodeMma = SourceNodeBwdMma<F>::fits;
-    const bool use_mma = kNodeMma && node_bwd_mma_enabled();
-    const bool saved = a.act_save != nullptr && a.msg_save != nullptr;
-    const bool stats = a.edge_bn_stat != nullptr;
-    auto ke = saved ? k_source_edge_bwd<F, true, false> : stats ? k_source_edge_bwd<F, false, true> : k_source_edge_bwd<F, false, false>;
-    if (stats && saved) return fail(PFS_ERR_UNSUPPORTED, "edge_bn_stat together with saved activations");
-    const size_t smem_e = stats ? SME::bytes_stats : SME::bytes;
+    auto ke = k_source_edge_bwd<F>;
     PFS_TRY(allow_smem(ke, smem_e));
     int gridn = 0;
-    if (use_mma) {
-        if constexpr (kNodeMma) {
-            ntn = (tp.S + kNodeRowsB - 1) / kNodeRowsB;        // 64-fibre tiles
-            PFS_TRY(allow_smem(k_source_node_bwd_mma<F>, SourceNodeBwdMma<F>::bytes));
-            gridn = persistent_grid(k_source_node_bwd_mma<F>, SourceNodeBwdMma<F>::bytes, (long long)ntn * tp.G, kNodeThreadsC);
-        }
-    } else if constexpr (kNodeC) {
-        PFS_TRY(allow_smem(k_source_node_bwd_c<F>, SourceNodeBwdSmemC<F>::bytes));
-        gridn = persistent_grid(k_source_node_bwd_c<F>, SourceNodeBwdSmemC<F>::bytes, (long long)ntn * tp.G, kNodeThreadsC);
+    if constexpr (kNodeMma) {
+        ntn = (tp.S + kNodeRowsB - 1) / kNodeRowsB;        // 48-fibre tiles
+        PFS_TRY(allow_smem(k_source_node_bwd_mma<F>, SourceNodeBwdMma<F>::bytes));
+        gridn = persistent_grid(k_source_node_bwd_mma<F>, SourceNodeBwdMma<F>::bytes, (long long)ntn * tp.G, kNodeThreadsC);
     } else {
         PFS_TRY(allow_smem(k_source_node_bwd<F>, SourceNodeBwdSmem<F>::bytes));
         gridn = persistent_grid(k_source_node_bwd<F>, SourceNodeBwdSmem<F>::bytes, (long long)ntn * tp.G);
@@ -811,23 +717,18 @@ int source_bwd_impl(const pfs_source_args& a, const Topo& tp) {
     float* wstage = ws.f(kConstFloats);
     if (!ws.ok) return fail(PFS_ERR_WORKSPACE, "source_bwd: workspace too small (%zu B)", a.workspace_bytes);
     {
-        // one prologue for the whole backward: Q_t (unless the activations were saved), the node-MLP weights and the
-        // message-MLP weights (disjoint regions of the constant bank), one upload
+        // one prologue for the whole backward: Q_t, the node-MLP weights and the message-MLP weights (disjoint regions
+        // of the constant bank), one upload
         TableJob jobs[2] = {TableJob{a.x_t, tp.T, 0, -1, a.b1, Qt}, TableJob{}};
         PackList pl{};
         add_msg_weights<F>(pl, a.w1, a.w2, a.b2);
-        if (a.edge_bn_stat) {
-            PFS_REQUIRE(a.edge_bn_shift, "edge_bn_stat needs edge_bn_shift");
-            pl.it[pl.n++] = PackItem{a.edge_bn_shift, 1, 0, 1, F, 0, MsgEdgeConst<F>::kEB};
-        }
         int nfloats = MsgEdgeConst<F>::kFloats;
-        if constexpr (kNodeC) {
+        if constexpr (kNodeMma) {
             using CW = SourceNodeConst<F>;
             pl.it[pl.n++] = PackItem{a.w4, J, 0, J, F, 0, CW::kW4o};       // W4 as stored [F][J]
-            if (!use_mma) pl.it[pl.n++] = PackItem{a.w3, J, 0, K9, J, 0, CW::kW3o};      // W3[:, :9F] as stored [J][K9] (FMA kernel)
-            nfloats = use_mma ? CW::kBwdMmaFloats : CW::kBwdFloats;
+            nfloats = CW::kBwdMmaFloats;
         }
-        PFS_TRY((run_prep<F, M>(tp.G, jobs, saved ? 0 : 1, a.w1, M, a.u, pl, nfloats, wstage, st)));
+        PFS_TRY((run_prep<F, M>(tp.G, jobs, 1, a.w1, M, a.u, pl, nfloats, wstage, st)));
     }
     if (mode != 0) {
         int nchunk = (tp.S + 4095) / 4096;           // one CTA per 4096 fibres of a graph (1 for the C3 graphs)
@@ -845,20 +746,10 @@ int source_bwd_impl(const pfs_source_args& a, const Topo& tp) {
     {
         SourceNodeBwdParams p{tp.G, tp.S, ntn, mode, a.eps, a.x_s, a.moments, a.hidden, a.y_pre, a.g_out, a.bn_save,
                               bnstat, a.w3, a.w4, a.g_x_s, coefA, tot3p, wpn, pstride_n};
-        if constexpr (kNodeC) {
-            bool launched = false;
-            if constexpr (kNodeMma) {
-                if (use_mma) {
-                    // both 9F x 10F contractions on tcgen05 (3xTF32), see source_node_bwd_mma.cuh
-                    k_source_node_bwd_mma<F><<<gridn, kNodeThreadsC, SourceNodeBwdMma<F>::bytes, st>>>(p);
-                    PFS_LAUNCH_CHECK("k_source_node_bwd_mma");
-                    launched = true;
-                }
-            }
-            if (!launched) {
-                k_source_node_bwd_c<F><<<gridn, kNodeThreadsC, SourceNodeBwdSmemC<F>::bytes, st>>>(p);
-                PFS_LAUNCH_CHECK("k_source_node_bwd");
-            }
+        if constexpr (kNodeMma) {
+            // both 9F x 10F contractions on tcgen05 (3xTF32), see source_node_bwd_mma.cuh
+            k_source_node_bwd_mma<F><<<gridn, kNodeThreadsC, SourceNodeBwdMma<F>::bytes, st>>>(p);
+            PFS_LAUNCH_CHECK("k_source_node_bwd_mma");
         } else {
             k_source_node_bwd<F><<<gridn, kThreads, SourceNodeBwdSmem<F>::bytes, st>>>(p);
             PFS_LAUNCH_CHECK("k_source_node_bwd");
@@ -877,8 +768,7 @@ int source_bwd_impl(const pfs_source_args& a, const Topo& tp) {
     {
         const bool dense = tp.layout == PFS_LAYOUT_DENSE;
         SourceEdgeBwdParams p{tp, a.x_e, Qt, a.w1, a.w2, a.b2, a.moments, coefA, a.g_x_e, a.g_x_e_add,
-                              dense ? stage : nullptr, dense ? nullptr : stage, wpe, pstride_e, a.act_save, a.msg_save,
-                              a.edge_bn_stat};
+                              dense ? stage : nullptr, dense ? nullptr : stage, wpe, pstride_e};
         ke<<<gride, kThreads, smem_e, st>>>(p);
         PFS_LAUNCH_CHECK("k_source_edge_bwd");
     }
@@ -934,7 +824,7 @@ int target_fwd_impl(const pfs_target_args& a, const Topo& tp) {
     }
     {
         const bool dense = tp.layout == PFS_LAYOUT_DENSE;
-        TargetEdgeFwdParams p{tp, a.x_e, Rs, a.w1, dense ? stage : nullptr, dense ? nullptr : stage, a.act_save};
+        TargetEdgeFwdParams p{tp, a.x_e, Rs, a.w1, dense ? stage : nullptr, dense ? nullptr : stage};
         const int grid = persistent_grid(k_target_edge_fwd<F>, 0, total);
         k_target_edge_fwd<F><<<grid, kThreads, 0, st>>>(p);
         PFS_LAUNCH_CHECK("k_target_edge_fwd");
@@ -963,8 +853,7 @@ int target_bwd_impl(const pfs_target_args& a, const Topo& tp) {
     prof_mark(nullptr, st);
     const int total = tp.ntiles * tp.G;
     using SM = TargetEdgeBwdSmem<F>;
-    const bool saved = a.act_save != nullptr;
-    auto ke = saved ? k_target_edge_bwd<F, true> : k_target_edge_bwd<F, false>;
+    auto ke = k_target_edge_bwd<F>;
     PFS_TRY(allow_smem(ke, SM::bytes));
     const int gride = persistent_grid(ke, SM::bytes, total);
     constexpr int pstride_e = M * F;
@@ -1007,10 +896,10 @@ int target_bwd_impl(const pfs_target_args& a, const Topo& tp) {
         TableJob jobs[2] = {TableJob{a.x_s, tp.S, 0, -1, a.b1, Rs}, TableJob{}};
         PackList pl{};
         add_msg_weights<F>(pl, a.w1, nullptr, nullptr);
-        PFS_TRY((run_prep<F, M>(tp.G, jobs, (saved || cached) ? 0 : 1, a.w1, M, a.u, pl, MsgEdgeConst<F>::kFloats, wstage, st)));
+        PFS_TRY((run_prep<F, M>(tp.G, jobs, cached ? 0 : 1, a.w1, M, a.u, pl, MsgEdgeConst<F>::kFloats, wstage, st)));
     }
     {
-        TargetEdgeBwdParams p{tp, a.x_e, Rs, a.w1, dasum, a.g_x_e, a.g_x_e_add, dRs, wpe, pstride_e, a.act_save};
+        TargetEdgeBwdParams p{tp, a.x_e, Rs, a.w1, dasum, a.g_x_e, a.g_x_e_add, dRs, wpe, pstride_e};
         ke<<<gride, kThreads, SM::bytes, st>>>(p);
         PFS_LAUNCH_CHECK("k_target_edge_bwd");
     }
@@ -1196,11 +1085,6 @@ size_t pfs_workspace_bytes(const pfs_topology* t) {
     fl += G * 64 * 2 * F + 64;                                   // chunk partials of the node BatchNorm backward sums
     fl += 4096;
     return fl * sizeof(float) + 64 * 256;
-}
-
-int32_t pfs_stat_tiles(const pfs_topology* t) {
-    if (!t) return 0;
-    return t->layout == PFS_LAYOUT_DENSE ? dense_ntiles(t->S, t->T) : t->ntiles;
 }
 
 int pfs_detect_dense(const int64_t* edge_index, int64_t E, int32_t S, int32_t T, int32_t* flag_dev, void* stream) {

@@ -477,8 +477,7 @@ template <int F>
 struct MsgEdgeConst {
     static constexpr int M = 2 * F;
     static constexpr int kW1t = 0, kW2t = F * M, kW2o = F * M + M * M, kW1o = F * M + 2 * M * M,
-                         kB2 = 2 * F * M + 2 * M * M, kEB = 2 * F * M + 2 * M * M + M,      // kEB: EdgeModel norm.bias [F]
-                         kFloats = 2 * F * M + 2 * M * M + M + F;
+                         kB2 = 2 * F * M + 2 * M * M, kFloats = 2 * F * M + 2 * M * M + M;
 };
 
 // packs dst[k * J + j] = W[j * ld + koff + k] (input-major) or dst[j * K + k] (output-major)

@@ -26,7 +26,6 @@ struct EdgeFwdParams {
     int stage_class;    // 1: the class table P_t is staged in shared memory too
     int nrec;           // statistics records per CTA (chunk_records)
     int nbuf;           // staging buffers (2 = prefetch the next tile)
-    float* act_save;    // [G,E(q),4F] hidden activations for the backward, or null
 };
 
 template <int F>
@@ -67,7 +66,6 @@ __global__ void __launch_bounds__(kThreads, 2) k_edge_fwd(const EdgeFwdParams p)
             dense_acc_c<F, H, kW1>(x, h);
 #pragma unroll
             for (int j = 0; j < H; ++j) h[j] = lrelu(h[j]);
-            if (p.act_save) store_row<H>(p.act_save + ((size_t)t.g * tp.E + t.q0 + threadIdx.x) * H, h);
 #pragma unroll
             for (int j = 0; j < F; ++j) z[j] = c_w[kB2 + j];
             dense_acc_c<H, F, kW2>(h, z);
@@ -157,9 +155,7 @@ __global__ void __launch_bounds__(kThreads) k_edge_bn_bwd_stats(const EdgeBnStat
 //   stage 1 (after it): fills c1 = mean g, c2 = mean(g xhat1) * kappa and the per-graph
 //            gamma / beta gradients dgb[g][0..F) , dgb[g][F..2F)
 // mode: 0 = not normed, 1 = train, 2 = eval
-// unscaled (stage 1, train mode): sums[.][F..2F) holds sum g (x_e_out - beta) (the statistics a previous kernel took
-// while it stored g, pfs_edge_args.bn_stat_in) instead of sum g xhat1; the factor inv is applied here
-__global__ void k_edge_bn_bwd_coef(int stage, int mode, int unscaled, int F, int G, int ntiles, long long n_rows,
+__global__ void k_edge_bn_bwd_coef(int stage, int mode, int F, int G, int ntiles, long long n_rows,
                                    const float* __restrict__ save, const float* __restrict__ gamma,
                                    const float* __restrict__ beta, const float* __restrict__ rm,
                                    const float* __restrict__ rv, float eps, const double* __restrict__ sums,
@@ -204,8 +200,7 @@ __global__ void k_edge_bn_bwd_coef(int stage, int mode, int unscaled, int F, int
         return;
     }
     const double sg = sums[(size_t)g * 2 * F + f];
-    double sgx = sums[(size_t)g * 2 * F + F + f];
-    if (unscaled) sgx *= (gm != 0.0) ? 1.0 / (gm * gm * r2) : 0.0;
+    const double sgx = sums[(size_t)g * 2 * F + F + f];
     const double n = (double)n_rows;
     const double gbar = sg / n, mgx = sgx / n;
     const double sc = gm * r2, q = var * r1 * r1;
@@ -228,7 +223,6 @@ struct EdgeBwdParams {
     float* wpartial;                 // [ncta][pstride]: dW1_e [4F*F], dW2 [F*4F], db2 [F]
     int pstride;
     int max_fib, stage_class, nbuf;
-    const float* act_save;           // [G,E(q),4F] hidden activations saved by the forward (k_edge_bwd2<F, true>)
 };
 
 // constant-bank layout of the edge backward (floats): W1_e input-major [F][H] (recompute h),
@@ -370,9 +364,7 @@ __global__ void __launch_bounds__(kThreads) k_edge_bwd(const EdgeBwdParams p) {
 //   * the two weight-gradient accumulations run on the two halves of the CTA and SHARE one register array;
 //   * db2 = sum dz is taken from the staged dz rows instead of a per-thread running sum.
 // ------------------------------------------------------------------------------------------
-// SAVED: ps points at the edge's saved activation row a1 = lrelu(h1) (lrelu' is read off its sign: a1 > 0 <=> h1 > 0)
-// instead of the node-table rows; the first layer is not recomputed
-template <int F, int HALF, bool SAVED>
+template <int F, int HALF>
 __device__ __forceinline__ void edge_bwd_half(const EdgeBwdParams& p, const float* __restrict__ ps, const float* __restrict__ pt,
                                               const float (&x)[F], const float (&dz)[F], float (&dx)[F], float* A1row,
                                               float* DHrow, float* dh_row_out) {
@@ -380,17 +372,15 @@ __device__ __forceinline__ void edge_bwd_half(const EdgeBwdParams& p, const floa
     using CW = EdgeBwdConst<F>;
     float hh[HH], da[HH];
     load_row<HH>(ps + HALF * HH, hh);
-    if constexpr (!SAVED) {
-        add_row<HH>(pt + HALF * HH, hh);
-        dense_acc_c<F, HH, CW::kW1t + HALF * HH, H>(x, hh);
-    }
+    add_row<HH>(pt + HALF * HH, hh);
+    dense_acc_c<F, HH, CW::kW1t + HALF * HH, H>(x, hh);
 #pragma unroll
     for (int k = 0; k < HH; ++k) da[k] = 0.f;
     dense_acc_c<F, HH, CW::kW2o + HALF * HH, H>(dz, da);
 #pragma unroll
     for (int k = 0; k < HH; ++k) {
         da[k] *= dlrelu(hh[k]);      // dh
-        if constexpr (!SAVED) hh[k] = lrelu(hh[k]);        // a1
+        hh[k] = lrelu(hh[k]);        // a1
     }
     store_row_smem<HH>(A1row + HALF * HH, hh);
     store_row_smem<HH>(DHrow + HALF * HH, da);
@@ -398,7 +388,7 @@ __device__ __forceinline__ void edge_bwd_half(const EdgeBwdParams& p, const floa
     if (dh_row_out) store_row<HH>(dh_row_out + HALF * HH, da);
 }
 
-template <int F, bool SAVED>
+template <int F>
 __global__ void __launch_bounds__(kThreads, 2) k_edge_bwd2(const EdgeBwdParams p) {
     constexpr int H = 4 * F;
     using SM = EdgeBwdSmem<F>;
@@ -437,7 +427,6 @@ __global__ void __launch_bounds__(kThreads, 2) k_edge_bwd2(const EdgeBwdParams p
             bulk_prefetch_l2(p.x_e + off, bytes);
             bulk_prefetch_l2(p.xe2 + off, bytes);
             bulk_prefetch_l2(p.gout + off, bytes);
-            if (SAVED) bulk_prefetch_l2(p.act_save + off * 4, bytes * 4);
         }
         __syncthreads();
         const float* XE = stg.edge(b, 0);
@@ -460,12 +449,11 @@ __global__ void __launch_bounds__(kThreads, 2) k_edge_bwd2(const EdgeBwdParams p
             store_row_smem<F>(DZ + threadIdx.x * LDF, dz);
 #pragma unroll
             for (int k = 0; k < F; ++k) dx[k] = 0.f;
-            const float* ps = SAVED ? p.act_save + ((size_t)t.g * tp.E + t.q0 + threadIdx.x) * H
-                                    : p.Ps + ((size_t)t.g * tp.S + er.src) * H;
-            const float* pt = SAVED ? nullptr : p.Pt + ((size_t)t.g * tp.T + er.tgt) * H;
+            const float* ps = p.Ps + ((size_t)t.g * tp.S + er.src) * H;
+            const float* pt = p.Pt + ((size_t)t.g * tp.T + er.tgt) * H;
             float* dho = p.dh_rows ? p.dh_rows + ((size_t)t.g * tp.E + t.q0 + threadIdx.x) * H : nullptr;
-            edge_bwd_half<F, 0, SAVED>(p, ps, pt, x, dz, dx, A1 + threadIdx.x * LDH, DH + threadIdx.x * LDH, dho);
-            edge_bwd_half<F, 1, SAVED>(p, ps, pt, x, dz, dx, A1 + threadIdx.x * LDH, DH + threadIdx.x * LDH, dho);
+            edge_bwd_half<F, 0>(p, ps, pt, x, dz, dx, A1 + threadIdx.x * LDH, DH + threadIdx.x * LDH, dho);
+            edge_bwd_half<F, 1>(p, ps, pt, x, dz, dx, A1 + threadIdx.x * LDH, DH + threadIdx.x * LDH, dho);
             store_row<F>(p.g_x_e + row, dx);
         }
         __syncthreads();

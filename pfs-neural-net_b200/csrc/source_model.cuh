@@ -28,8 +28,6 @@ struct SourceEdgeFwdParams {
     const float* Qt;       // [G,T,2F] = x_t . W1[:, :F]^T + b1
     const float *w1, *w2, *b2;
     float* moments;        // [G,S,5,2F]: mean, E[m^2], c2, c3, c4
-    float* act_save;       // [G,E(q),2F] hidden activations for the backward, or null
-    float* msg_save;       // [G,E(q),2F] messages for the backward, or null
     const float* xaff;     // [G,4,F] (rows 2, 3: scale, shift) of a deferred EdgeModel norm, or null: xe2 then holds z
     float* xe_norm_out;    // [G,E,F] where x_e' = scale z + shift is stored (may alias xe2)
 };
@@ -62,11 +60,6 @@ __global__ void __launch_bounds__(kThreads) k_source_edge_fwd(const SourceEdgeFw
                 m[j] = c_w[CW::kB2 + j];
             }
             dense_acc_c<M, M, CW::kW2t>(h, m);
-            if (p.act_save) {
-                const size_t q = ((size_t)t.g * tp.E + t.q0 + threadIdx.x) * M;
-                store_row<M>(p.act_save + q, h);
-                store_row<M>(p.msg_save + q, m);
-            }
 #pragma unroll
             for (int j = 0; j < M; ++j) MT[j * LDT + threadIdx.x] = m[j];
         }
@@ -480,9 +473,6 @@ struct SourceEdgeBwdParams {
     float* dhs_rows;                // general: [G,E(q),2F]
     float* wpartial;                // [ncta][pstride]: dW1_e [2F*F], dW2 [2F*2F], db2 [2F]
     int pstride;
-    const float *act_save, *msg_save;   // [G,E(q),2F] each, saved by the forward (k_source_edge_bwd<F, true>)
-    float* bn_stat_part;            // optional [G*ntiles][2F]: per-tile sums of g and g (x_e' - beta) over the STORED gradient
-                                    // rows (the EdgeModel's BatchNorm-backward statistics, beta in the constant bank at kEB)
 };
 
 template <int F>
@@ -492,14 +482,9 @@ struct SourceEdgeBwdSmem {
     static constexpr int kWeights = 0;   // the weights live in the constant bank (MsgEdgeConst)
     static constexpr int kTiles = kTile * (3 * LDM + LDF);
     static constexpr size_t bytes = sizeof(float) * (kWeights + kTiles);
-    static constexpr size_t bytes_stats = bytes + sizeof(float) * kTile * 2 * F;   // + the [g | g (x - beta)] rows of bn_stat_part
 };
 
-// SAVED: the hidden activations a = lrelu(h) and the messages m are read back (act_save / msg_save of the forward)
-// instead of being recomputed; lrelu' is read off the sign of a
-// STATS: also emit bn_stat_part (opt-in, PFS_FUSE_BN_STATS=1: measured at C3 it does not pay -- the extra staging and
-// reduction cost this kernel 0.10 ms, the statistics kernel it replaces takes 0.11 ms, profiles/r02_bn_stat_fusion.txt)
-template <int F, bool SAVED, bool STATS = false>
+template <int F>
 __global__ void __launch_bounds__(kThreads, (F <= 10 ? 2 : 1)) k_source_edge_bwd(const SourceEdgeBwdParams p) {
     using SM = SourceEdgeBwdSmem<F>;
     constexpr int M = 2 * F, LDM = SM::LDM, LDF = SM::LDF;
@@ -509,7 +494,6 @@ __global__ void __launch_bounds__(kThreads, (F <= 10 ? 2 : 1)) k_source_edge_bwd
     float* AS = DM + kTile * LDM;
     float* DHS = AS + kTile * LDM;
     float* XE = DHS + kTile * LDM;   // [kTile][LDF]
-    float* GS = XE + kTile * LDF;    // [kTile][2F]
     using AccW2 = OuterAcc<M, M, 4, F / 2, 0, 160>;            // dW2[j][k]   = sum dm_j as_k
     using AccW1 = OuterAcc<M, F, 4, F / 2, 160, 96>;           // dW1_e[j][k] = sum dhs_j x_k
     AccW2 accw2;
@@ -531,33 +515,20 @@ __global__ void __launch_bounds__(kThreads, (F <= 10 ? 2 : 1)) k_source_edge_bwd
             if (p.g_add) bulk_prefetch_l2(p.g_add + off, bytes);
             bulk_prefetch_l2(p.coefA + frow * 4 * M, (size_t)tn.nfib * 4 * M * sizeof(float));
             bulk_prefetch_l2(p.moments + frow * 5 * M, (size_t)tn.nfib * 5 * M * sizeof(float));
-            if (SAVED) {
-                bulk_prefetch_l2(p.act_save + off * 2, bytes * 2);
-                bulk_prefetch_l2(p.msg_save + off * 2, bytes * 2);
-            }
         }
         if (threadIdx.x < t.ne) {
             const EdgeRef er = get_edge(tp, t, threadIdx.x);
             const size_t row = ((size_t)t.g * tp.E + er.e) * F;
-            float x[F], h[M], m[M];
+            float x[F], h[M], a[M], m[M];
             load_row<F>(p.xe2 + row, x);
-            float a[M];
-            if constexpr (SAVED) {
-                const size_t q = ((size_t)t.g * tp.E + t.q0 + threadIdx.x) * M;
-                load_row<M>(p.act_save + q, a);
-                load_row<M>(p.msg_save + q, m);
+            load_row<M>(p.Qt + ((size_t)t.g * tp.T + er.tgt) * M, h);
+            dense_acc_c<F, M, CW::kW1t>(x, h);
 #pragma unroll
-                for (int j = 0; j < M; ++j) h[j] = a[j];          // only the sign is used below
-            } else {
-                load_row<M>(p.Qt + ((size_t)t.g * tp.T + er.tgt) * M, h);
-                dense_acc_c<F, M, CW::kW1t>(x, h);
-#pragma unroll
-                for (int j = 0; j < M; ++j) {
-                    a[j] = lrelu(h[j]);
-                    m[j] = c_w[CW::kB2 + j];
-                }
-                dense_acc_c<M, M, CW::kW2t>(a, m);
+            for (int j = 0; j < M; ++j) {
+                a[j] = lrelu(h[j]);
+                m[j] = c_w[CW::kB2 + j];
             }
+            dense_acc_c<M, M, CW::kW2t>(a, m);
             // dm = (A0 + A1 m + A2 d^2 + A3 d^3) / count
             int e0, n;
             fibre_range(tp, t, er.src - t.fibre0, e0, n);
@@ -606,49 +577,12 @@ __global__ void __launch_bounds__(kThreads, (F <= 10 ? 2 : 1)) k_source_edge_bwd
             dense_acc_c<M, F, CW::kW1o>(da, dx);
             if (p.g_add) add_row<F>(p.g_add + row, dx);
             store_row<F>(p.g_x_e + row, dx);
-            if constexpr (STATS) {     // dx is now the whole gradient of x_e': its BatchNorm-backward statistics ride along
-                float xr[F], gs[M];
-                {   // own row back from the staged tile (rows of LDF floats are 8-byte aligned only)
-                    const float2* q = reinterpret_cast<const float2*>(XE + threadIdx.x * LDF);
-#pragma unroll
-                    for (int k = 0; k < F / 2; ++k) {
-                        const float2 v = q[k];
-                        xr[2 * k] = v.x; xr[2 * k + 1] = v.y;
-                    }
-                }
-#pragma unroll
-                for (int k = 0; k < F; ++k) {
-                    gs[k] = dx[k];
-                    gs[F + k] = dx[k] * (xr[k] - c_w[CW::kEB + k]);
-                }
-                store_row_smem<M>(GS + threadIdx.x * M, gs);
-            }
             if (p.dhs_rows) store_row<M>(p.dhs_rows + ((size_t)t.g * tp.E + t.q0 + threadIdx.x) * M, da);
         }
         __syncthreads();
         accw2.accumulate(DM, LDM, AS, LDM, t.ne);
         accw1.accumulate(DHS, LDM, XE, LDF, t.ne);
         if (p.class_part) tile_class_sums<M, LDM>(tp, t, DHS, p.class_part + (size_t)tile * tp.T * M);
-        if (STATS && (int)threadIdx.x >= kThreads - 8 * M) {
-            // column sums of GS over the tile: 8 row parts per column in adjacent lanes (whole warps: 8 * 2F threads,
-            // M % 4 == 0; the upper threads of the CTA, whose outer product is the shorter one), three shuffles, fixed order
-            const int tt = (int)threadIdx.x - (kThreads - 8 * M);
-            const int part = tt & 7, col = tt >> 3;
-            float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-            int r = part;
-            for (; r + 24 < t.ne; r += 32) {
-                s0 += GS[r * M + col];
-                s1 += GS[(r + 8) * M + col];
-                s2 += GS[(r + 16) * M + col];
-                s3 += GS[(r + 24) * M + col];
-            }
-            for (; r < t.ne; r += 8) s0 += GS[r * M + col];
-            float sum = (s0 + s1) + (s2 + s3);
-            sum += __shfl_xor_sync(0xffffffffu, sum, 1);
-            sum += __shfl_xor_sync(0xffffffffu, sum, 2);
-            sum += __shfl_xor_sync(0xffffffffu, sum, 4);
-            if (part == 0) p.bn_stat_part[(size_t)tile * M + col] = sum;
-        }
         __syncthreads();
     }
     float* out = p.wpartial + (size_t)blockIdx.x * p.pstride;

@@ -22,7 +22,7 @@
 //     BatchNorm backward of the upstream gradient and the moment-polynomial coefficients.
 #pragma once
 #include <cfloat>
-#include "source_node_c.cuh"
+#include "source_node_mma.cuh"
 #include "tc_ptx.cuh"
 
 namespace pfs {

@@ -14,10 +14,32 @@
 //     epilogue (bias, LeakyReLU, hidden store, second layer, BatchNorm tile statistics).
 #pragma once
 #include <cfloat>
-#include "source_node_c.cuh"
+#include "source_model.cuh"
 #include "tc_ptx.cuh"
 
 namespace pfs {
+
+constexpr int kNodeThreadsC = 320;   // 10 warps
+constexpr int kNodeRowsC = 128;      // fibres per node tile of the forward
+
+// Constant-bank layout of the node kernels (floats; common.cuh: c_w).  The node-MLP constants sit ABOVE the
+// message-MLP constants (MsgEdgeConst, at most 2 * 16 * 32 + 2 * 32 * 32 + 32 floats at Fdim 16) so that one upload
+// per module call serves the edge kernel and the node kernel.  W3 itself goes to shared memory as the MMA operand.
+template <int F>
+struct SourceNodeConst {
+    static constexpr int K9 = 9 * F, J = 10 * F;
+    static constexpr int kBase = 4096;
+    // forward: W4 input-major [J][F] (y_f += W4[f][j] a_j), b4 [F]
+    static constexpr int kW4t = kBase, kB4 = kBase + J * F, kFwdMmaFloats = kBase + J * F + F;
+    // backward: W4 as stored [F][J] (dh3_j += W4[f][j] dy_f)
+    static constexpr int kW4o = kBase, kBwdMmaFloats = kBase + F * J;
+    // The tensor-core node kernels serve the widths at which the whole node MLP, W3 [J][9F] included, fits the bank
+    // above kBase: Fdim 4, 8 and 10.  Fdim 16 runs the shared-memory kernels of source_model.cuh.  This predicate also
+    // picks the node tile size and the workspace carve (api.cu: node_tile_rows).
+    static constexpr bool fits = kBase + J * F + F + K9 * J <= kConstFloats;
+};
+
+__device__ __forceinline__ int warp_index_uniform() { return __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0); }
 
 template <int F>
 struct SourceNodeMma {

@@ -18,7 +18,6 @@ struct TargetEdgeFwdParams {
     const float* w1;        // [2F,2F]
     float* class_part;      // dense: [G,ntiles,T,2F]
     float* act_rows;        // general: [G,E(q),2F]
-    float* act_save;        // [G,E(q),2F] hidden activations for the backward, or null
 };
 
 template <int F>
@@ -38,7 +37,6 @@ __global__ void __launch_bounds__(kThreads) k_target_edge_fwd(const TargetEdgeFw
             dense_acc_c<F, M, CW::kW1t>(x, h);
 #pragma unroll
             for (int j = 0; j < M; ++j) h[j] = lrelu(h[j]);
-            if (p.act_save) store_row<M>(p.act_save + ((size_t)t.g * tp.E + t.q0 + threadIdx.x) * M, h);
             if (p.act_rows) {
                 store_row<M>(p.act_rows + ((size_t)t.g * tp.E + t.q0 + threadIdx.x) * M, h);
             } else {
@@ -335,7 +333,6 @@ struct TargetEdgeBwdParams {
     float* dRs;             // [G,S,2F]
     float* wpartial;        // [ncta][pstride]: dW1_e [2F*F]
     int pstride;
-    const float* act_save;  // [G,E(q),2F] hidden activations saved by the forward (k_target_edge_bwd<F, true>)
 };
 
 template <int F>
@@ -349,8 +346,7 @@ struct TargetEdgeBwdSmem {
     static constexpr size_t bytes = sizeof(float) * kFloats;
 };
 
-// SAVED: the hidden activation is read back (act_save of the forward; lrelu' from its sign) instead of recomputed
-template <int F, bool SAVED>
+template <int F>
 __global__ void __launch_bounds__(kThreads) k_target_edge_bwd(const TargetEdgeBwdParams p) {
     using SM = TargetEdgeBwdSmem<F>;
     constexpr int M = 2 * F, LDM = SM::LDM, LDF = SM::LDF;
@@ -370,20 +366,15 @@ __global__ void __launch_bounds__(kThreads) k_target_edge_bwd(const TargetEdgeBw
             const size_t off = ((size_t)tn.g * tp.E + tn.q0) * F, bytes = (size_t)tn.ne * F * sizeof(float);
             bulk_prefetch_l2(p.xe2 + off, bytes);
             if (p.g_add) bulk_prefetch_l2(p.g_add + off, bytes);
-            if (SAVED) bulk_prefetch_l2(p.act_save + off * 2, bytes * 2);
-            else bulk_prefetch_l2(p.Rs + ((size_t)tn.g * tp.S + tn.fibre0) * M, (size_t)tn.nfib * M * sizeof(float));
+            bulk_prefetch_l2(p.Rs + ((size_t)tn.g * tp.S + tn.fibre0) * M, (size_t)tn.nfib * M * sizeof(float));
         }
         if (threadIdx.x < t.ne) {
             const EdgeRef er = get_edge(tp, t, threadIdx.x);
             const size_t row = ((size_t)t.g * tp.E + er.e) * F;
             float x[F], h[M], d[M];
             load_row<F>(p.xe2 + row, x);
-            if constexpr (SAVED) {
-                load_row<M>(p.act_save + ((size_t)t.g * tp.E + t.q0 + threadIdx.x) * M, h);
-            } else {
-                load_row<M>(p.Rs + ((size_t)t.g * tp.S + er.src) * M, h);
-                dense_acc_c<F, M, CW::kW1t>(x, h);
-            }
+            load_row<M>(p.Rs + ((size_t)t.g * tp.S + er.src) * M, h);
+            dense_acc_c<F, M, CW::kW1t>(x, h);
             load_row<M>(p.dasum + ((size_t)t.g * tp.T + er.tgt) * M, d);
 #pragma unroll
             for (int j = 0; j < M; ++j) d[j] *= dlrelu(h[j]);

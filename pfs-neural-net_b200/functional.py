@@ -12,30 +12,8 @@ import torch
 
 from . import _abi
 
-import os
-
 BN_EPS = 1e-5
 BN_MOMENTUM = 0.1
-# PFS_SAVE_ACT=1 keeps the per-edge hidden activations (and the SModel messages) of a training forward for the backward
-# instead of recomputing them (+16F + 16F + 8F bytes per edge of HBM, ~30 % fewer instructions in the three backward edge
-# kernels).  OFF by default -- measured at C3 (profiles/r02_save_act_vs_recompute.txt) it LOSES: the forward kernels slow
-# down by the extra row stores (k_edge_fwd 0.40 -> 0.70 ms, k_source_edge_fwd 0.34 -> 0.48, k_target_edge_fwd 0.15 ->
-# 0.22) and the backward kernels do not speed up (k_edge_bwd2 1.19 -> 1.24 ms): they wait on their per-thread row loads,
-# of which there are now more, not on instruction issue.  Step 5.38 -> 5.82 ms.
-SAVE_ACT = os.environ.get("PFS_SAVE_ACT", "0") == "1"
-# PFS_KEEP_TABLES=0: the backward recomputes the node tables of the first-layer split (P_s, P_t, R_s) instead of reading the
-# forward's; PFS_DEFER_AFFINE=0: the EdgeModel applies its norm itself inside a Block too (A/B runs)
-KEEP_TABLES = os.environ.get("PFS_KEEP_TABLES", "1") == "1"
-DEFER_AFFINE = os.environ.get("PFS_DEFER_AFFINE", "1") == "1"
-# PFS_FUSE_BN_STATS=1: the SModel backward, which stores the complete gradient of x_e', also takes the statistics the
-# EdgeModel's BatchNorm backward needs from it (pfs_source_args.edge_bn_stat -> pfs_edge_args.bn_stat_in) instead of a pass
-# of its own over g and x_e'.  OFF by default: measured at C3 it does not pay (profiles/r02_bn_stat_fusion.txt).
-FUSE_BN_STATS = os.environ.get("PFS_FUSE_BN_STATS", "0") == "1"
-
-
-def _want_save(ctx):
-    """a backward will follow (some input needs a gradient and grad mode was on at apply time)"""
-    return SAVE_ACT and any(ctx.needs_input_grad)
 RMS_EPS = float(torch.finfo(torch.float32).eps)    # nn.RMSNorm(eps=None), reference src/gnn.py:203
 
 
@@ -89,24 +67,14 @@ class XeGradBus:
     (`g_x_e_add` of pfs_target_bwd / pfs_source_bwd) and marks it used; `XeFanout.backward` adds whatever was not
     fused, so every combination of used / unused branches gives the same sum.  In a training step autograd runs
     the output tap first, then TModel, then SModel, and nothing is left for it to add."""
-    __slots__ = ("g_o", "g_t", "o_used", "t_used", "edge_beta", "stat", "stat_for")
+    __slots__ = ("g_o", "g_t", "o_used", "t_used")
 
     def __init__(self):
-        self.edge_beta = None        # EdgeModel norm.bias when that norm runs in train mode (set by Block.forward)
-        self.stat = self.stat_for = None
         self.clear()
 
     def clear(self):
         self.g_o = self.g_t = None
         self.o_used = self.t_used = False
-
-    def take_stats(self, g):
-        """BatchNorm-backward statistics of `g` if the SModel backward took them while it stored exactly this tensor."""
-        st, key = self.stat, self.stat_for
-        self.stat = self.stat_for = None
-        if st is not None and key == (g.data_ptr(), g._version, tuple(g.shape)):
-            return st
-        return None
 
     def addend_for_target(self, like):
         if (self.g_o is not None and not self.o_used and self.g_o.numel() == like.numel()
@@ -169,44 +137,41 @@ class EdgeFunction(torch.autograd.Function):
     """EdgeModel (reference src/gnn.py:73-101) -> pfs_edge_fwd / pfs_edge_bwd."""
 
     @staticmethod
-    def forward(ctx, topo, training, normed, x_s, x_t, x_e, u, w1, b1, w2, b2, gamma, beta, rm, rv, nbt, defer=None, bus=None):
+    def forward(ctx, topo, training, normed, x_s, x_t, x_e, u, w1, b1, w2, b2, gamma, beta, rm, rv, nbt, defer=None):
         """`defer`: a dict handed in by Block.forward.  When the module is normed the BatchNorm affine is NOT applied here:
         the returned tensor holds the pre-norm z, defer["affine"] the per-graph (scale, shift), and the next consumer
         (SourceFunction with edge_affine=...) normalises the rows in place while it reads them."""
         dev = _dev_check(x_s, x_t, x_e, u, w1, b1, w2, b2, gamma, beta, rm, rv)
-        ctx.save_act = _want_save(ctx)
         x_s, x_t, x_e, u, w1, b1, w2, b2, gamma, beta = (_c(t) for t in (x_s, x_t, x_e, u, w1, b1, w2, b2, gamma, beta))
         G, F = _check_shapes(topo, x_s, x_t, x_e, u)
         lib = _abi.load_library()
         out = torch.empty_like(x_e)
         bn_save = torch.empty(G, 4, F, device=dev, dtype=torch.float32) if normed else None
-        act = torch.empty(G, topo.E, 4 * F, device=dev, dtype=torch.float32) if ctx.save_act else None
         # node tables of the first-layer split, kept for the backward when one will follow (it then skips their recomputation)
-        keep = KEEP_TABLES and any(ctx.needs_input_grad) and not ctx.save_act
+        keep = any(ctx.needs_input_grad)
         tab_s = torch.empty(G, topo.S, 4 * F, device=dev, dtype=torch.float32) if keep else None
         tab_t = torch.empty(G, topo.T, 4 * F, device=dev, dtype=torch.float32) if keep else None
         a = _abi.EdgeArgs()
         ws = _fill_common(a, topo, G, F, dict(x_s=x_s, x_t=x_t, x_e=x_e, u=u, w1=w1, b1=b1, w2=w2, b2=b2, gamma=gamma,
                                               beta=beta, running_mean=rm, running_var=rv, num_batches_tracked=nbt,
-                                              x_e_out=out, bn_save=bn_save, act_save=act, table_s=tab_s, table_t=tab_t))
+                                              x_e_out=out, bn_save=bn_save, table_s=tab_s, table_t=tab_t))
         a.training, a.normed, a.eps, a.momentum = int(training), int(normed), BN_EPS, BN_MOMENTUM
-        deferred = defer is not None and bool(normed) and DEFER_AFFINE
+        deferred = defer is not None and bool(normed)
         a.defer_affine = int(deferred)
         with torch.cuda.device(dev):
             a.stream = _stream(dev)
             _abi.check(lib.pfs_edge_fwd(ct.byref(a)), "pfs_edge_fwd")
         if deferred:
             defer["affine"] = bn_save
-        ctx.bus = bus
         ctx.topo, ctx.training, ctx.normed = topo, training, normed
         ctx.buffers = (rm, rv)
-        ctx.save_for_backward(x_s, x_t, x_e, u, w1, b1, w2, b2, gamma, beta, out, bn_save, act, tab_s, tab_t)
+        ctx.save_for_backward(x_s, x_t, x_e, u, w1, b1, w2, b2, gamma, beta, out, bn_save, tab_s, tab_t)
         del ws
         return out
 
     @staticmethod
     def backward(ctx, g):
-        x_s, x_t, x_e, u, w1, b1, w2, b2, gamma, beta, out, bn_save, act, tab_s, tab_t = ctx.saved_tensors
+        x_s, x_t, x_e, u, w1, b1, w2, b2, gamma, beta, out, bn_save, tab_s, tab_t = ctx.saved_tensors
         topo, dev = ctx.topo, x_e.device
         G, F = x_s.shape[0], x_s.shape[2]
         lib = _abi.load_library()
@@ -219,9 +184,7 @@ class EdgeFunction(torch.autograd.Function):
         a = _abi.EdgeArgs()
         rm, rv = ctx.buffers
         named = dict(x_s=x_s, x_t=x_t, x_e=x_e, u=u, w1=w1, b1=b1, w2=w2, b2=b2, gamma=gamma, beta=beta,
-                     running_mean=rm, running_var=rv, x_e_out=out, bn_save=bn_save, act_save=act, g_out=g,
-                     table_s=tab_s, table_t=tab_t,
-                     bn_stat_in=ctx.bus.take_stats(g) if (ctx.bus is not None and ctx.normed and ctx.training) else None)
+                     running_mean=rm, running_var=rv, x_e_out=out, bn_save=bn_save, g_out=g, table_s=tab_s, table_t=tab_t)
         named.update(gr)
         ws = _fill_common(a, topo, G, F, named)
         a.training, a.normed, a.eps, a.momentum = int(ctx.training), int(ctx.normed), BN_EPS, BN_MOMENTUM
@@ -230,7 +193,7 @@ class EdgeFunction(torch.autograd.Function):
             _abi.check(lib.pfs_edge_bwd(ct.byref(a)), "pfs_edge_bwd")
         del ws
         return (None, None, None, gr["g_x_s"], gr["g_x_t"], gr["g_x_e"], gr["g_u"], gr["g_w1"], gr["g_b1"],
-                gr["g_w2"], gr["g_b2"], gr["g_gamma"], gr["g_beta"], None, None, None, None, None)
+                gr["g_w2"], gr["g_b2"], gr["g_gamma"], gr["g_beta"], None, None, None, None)
 
 
 class SourceFunction(torch.autograd.Function):
@@ -242,7 +205,6 @@ class SourceFunction(torch.autograd.Function):
         """`edge_affine`: bn_save of an EdgeFunction run with a deferred norm -- x_e then holds the pre-norm z and is
         normalised IN PLACE by the edge pass of this call (every row is read and written by the same thread)."""
         dev = _dev_check(x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta, rm, rv)
-        save_act = _want_save(ctx)
         if edge_affine is not None and not x_e.is_contiguous():
             raise _abi.PfsError("deferred edge norm needs a contiguous x_e")
         (x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta) = (
@@ -251,8 +213,6 @@ class SourceFunction(torch.autograd.Function):
         lib = _abi.load_library()
         f32 = dict(device=dev, dtype=torch.float32)
         out = torch.empty_like(x_s)
-        act = torch.empty(G, topo.E, 2 * F, **f32) if save_act else None
-        msg = torch.empty(G, topo.E, 2 * F, **f32) if save_act else None
         moments = torch.empty(G, topo.S, 5, 2 * F, **f32)
         hidden = torch.empty(G, topo.S, 10 * F, **f32)
         y_pre = torch.empty(G, topo.S, F, **f32)
@@ -261,7 +221,7 @@ class SourceFunction(torch.autograd.Function):
         ws = _fill_common(a, topo, G, F, dict(
             x_s=x_s, x_t=x_t, x_e=x_e, u=u, w1=w1, b1=b1, w2=w2, b2=b2, w3=w3, b3=b3, w4=w4, b4=b4, gamma=gamma,
             beta=beta, running_mean=rm, running_var=rv, num_batches_tracked=nbt, x_s_out=out, moments=moments,
-            hidden=hidden, y_pre=y_pre, bn_save=bn_save, act_save=act, msg_save=msg,
+            hidden=hidden, y_pre=y_pre, bn_save=bn_save,
             x_e_affine=edge_affine, x_e_norm_out=x_e if edge_affine is not None else None))
         a.training, a.normed, a.eps, a.momentum = int(training), int(normed), BN_EPS, BN_MOMENTUM
         with torch.cuda.device(dev):
@@ -271,14 +231,14 @@ class SourceFunction(torch.autograd.Function):
         ctx.bus = bus
         ctx.buffers = (rm, rv)
         ctx.save_for_backward(x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta, moments, hidden, y_pre,
-                              bn_save, act, msg)
+                              bn_save)
         del ws
         return out
 
     @staticmethod
     def backward(ctx, g):
         (x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta, moments, hidden, y_pre,
-         bn_save, act, msg) = ctx.saved_tensors
+         bn_save) = ctx.saved_tensors
         topo, dev = ctx.topo, x_e.device
         G, F = x_s.shape[0], x_s.shape[2]
         lib = _abi.load_library()
@@ -292,18 +252,9 @@ class SourceFunction(torch.autograd.Function):
         rm, rv = ctx.buffers
         named = dict(x_s=x_s, x_t=x_t, x_e=x_e, u=u, w1=w1, b1=b1, w2=w2, b2=b2, w3=w3, b3=b3, w4=w4, b4=b4,
                      gamma=gamma, beta=beta, running_mean=rm, running_var=rv, moments=moments, hidden=hidden,
-                     y_pre=y_pre, bn_save=bn_save, act_save=act, msg_save=msg, g_out=g)
+                     y_pre=y_pre, bn_save=bn_save, g_out=g)
         add = ctx.bus.addend_for_source(x_e) if ctx.bus is not None else None
         named.update(gr, g_x_e_add=add)
-        # the stored g_x_e is the complete gradient of x_e' when the other two branches were fused in: its BatchNorm-backward
-        # statistics for the EdgeModel ride along (EdgeFunction.backward checks that it receives exactly this tensor)
-        stat = None
-        bus = ctx.bus
-        if (FUSE_BN_STATS and bus is not None and bus.edge_beta is not None and bus.o_used and bus.t_used
-                and bus.edge_beta.is_cuda and bus.edge_beta.dtype == torch.float32):
-            t = topo.struct(G, F)
-            stat = torch.empty(G * lib.pfs_stat_tiles(ct.byref(t)), 2 * F, device=dev, dtype=torch.float32)
-            named.update(edge_bn_shift=bus.edge_beta.detach().contiguous(), edge_bn_stat=stat)
         a = _abi.SourceArgs()
         ws = _fill_common(a, topo, G, F, named)
         a.training, a.normed, a.eps, a.momentum = int(ctx.training), int(ctx.normed), BN_EPS, BN_MOMENTUM
@@ -311,9 +262,6 @@ class SourceFunction(torch.autograd.Function):
             a.stream = _stream(dev)
             _abi.check(lib.pfs_source_bwd(ct.byref(a)), "pfs_source_bwd")
         del ws
-        if stat is not None:
-            g_e = gr["g_x_e"]
-            bus.stat, bus.stat_for = stat, (g_e.data_ptr(), g_e._version, tuple(g_e.shape))
         return (None, None, None, gr["g_x_s"], gr["g_x_t"], gr["g_x_e"], gr["g_u"], gr["g_w1"], gr["g_b1"],
                 gr["g_w2"], gr["g_b2"], gr["g_w3"], gr["g_b3"], gr["g_w4"], gr["g_b4"], gr["g_gamma"], gr["g_beta"],
                 None, None, None, None, None)
@@ -325,24 +273,22 @@ class TargetFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, topo, training, normed, x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta, rm, rv, nbt, bus=None):
         dev = _dev_check(x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta, rm, rv)
-        save_act = _want_save(ctx)
         (x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta) = (
             _c(t) for t in (x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta))
         G, F = _check_shapes(topo, x_s, x_t, x_e, u)
         lib = _abi.load_library()
         f32 = dict(device=dev, dtype=torch.float32)
         out = torch.empty_like(x_t)
-        act = torch.empty(G, topo.E, 2 * F, **f32) if save_act else None
         act_sum = torch.empty(G, topo.T, 2 * F, **f32)
         y_pre = torch.empty(G, topo.T, F, **f32)
         bn_save = torch.empty(G, 4, F, **f32) if normed else None
-        keep = KEEP_TABLES and any(ctx.needs_input_grad) and not save_act
+        keep = any(ctx.needs_input_grad)
         tab_s = torch.empty(G, topo.S, 2 * F, **f32) if keep else None
         a = _abi.TargetArgs()
         ws = _fill_common(a, topo, G, F, dict(
             x_s=x_s, x_t=x_t, x_e=x_e, u=u, w1=w1, b1=b1, w2=w2, b2=b2, w3=w3, b3=b3, w4=w4, b4=b4, gamma=gamma,
             beta=beta, running_mean=rm, running_var=rv, num_batches_tracked=nbt, x_t_out=out, act_sum=act_sum,
-            y_pre=y_pre, bn_save=bn_save, act_save=act, table_s=tab_s))
+            y_pre=y_pre, bn_save=bn_save, table_s=tab_s))
         a.training, a.normed, a.eps, a.momentum = int(training), int(normed), BN_EPS, BN_MOMENTUM
         with torch.cuda.device(dev):
             a.stream = _stream(dev)
@@ -350,13 +296,13 @@ class TargetFunction(torch.autograd.Function):
         ctx.topo, ctx.training, ctx.normed = topo, training, normed
         ctx.bus = bus
         ctx.buffers = (rm, rv)
-        ctx.save_for_backward(x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta, act_sum, y_pre, bn_save, act, tab_s)
+        ctx.save_for_backward(x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta, act_sum, y_pre, bn_save, tab_s)
         del ws
         return out
 
     @staticmethod
     def backward(ctx, g):
-        (x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta, act_sum, y_pre, bn_save, act, tab_s) = ctx.saved_tensors
+        (x_s, x_t, x_e, u, w1, b1, w2, b2, w3, b3, w4, b4, gamma, beta, act_sum, y_pre, bn_save, tab_s) = ctx.saved_tensors
         topo, dev = ctx.topo, x_e.device
         G, F = x_s.shape[0], x_s.shape[2]
         lib = _abi.load_library()
@@ -370,7 +316,7 @@ class TargetFunction(torch.autograd.Function):
         rm, rv = ctx.buffers
         named = dict(x_s=x_s, x_t=x_t, x_e=x_e, u=u, w1=w1, b1=b1, w2=w2, b2=b2, w3=w3, b3=b3, w4=w4, b4=b4,
                      gamma=gamma, beta=beta, running_mean=rm, running_var=rv, act_sum=act_sum, y_pre=y_pre,
-                     bn_save=bn_save, act_save=act, g_out=g, table_s=tab_s)
+                     bn_save=bn_save, g_out=g, table_s=tab_s)
         add = ctx.bus.addend_for_target(x_e) if ctx.bus is not None else None
         named.update(gr, g_x_e_add=add)
         a = _abi.TargetArgs()

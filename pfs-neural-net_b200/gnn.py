@@ -161,8 +161,7 @@ class EdgeModel(MLP):
         topo = get_topology(edge_index, x_s.shape[1], x_t.shape[1])
         normed, gamma, beta, rm, rv, nbt = _norm_tensors(self)
         out = pf.EdgeFunction.apply(topo, self.training, normed, x_s, x_t, edge_attr, u, self[0].weight, self[0].bias,
-                                    self[2].weight, self[2].bias, gamma, beta, rm, rv, nbt, getattr(self, "_defer", None),
-                                    getattr(self, "_xe_bus", None))
+                                    self[2].weight, self[2].bias, gamma, beta, rm, rv, nbt, getattr(self, "_defer", None))
         return out[0] if single else out
 
 
@@ -277,22 +276,17 @@ class Block(torch.nn.Module):
         if (hasattr(self, "edge_model") and hasattr(self, "s_model") and x_e.is_cuda and x_e.dtype == torch.float32):
             defer = {}
         # fp32 path: the three gradients of x_e' (SModel, TModel, the output) are added up inside the backward
-        # kernels instead of by autograd (functional.XeGradBus); the values are the same sum.  The SModel backward, which
-        # stores that sum, also takes the statistics the EdgeModel's BatchNorm backward needs from it.
+        # kernels instead of by autograd (functional.XeGradBus); the values are the same sum
         bus = None
         if (torch.is_grad_enabled() and x_e.is_cuda and x_e.dtype == torch.float32
                 and hasattr(self, "s_model") and hasattr(self, "t_model")):
             bus = pf.XeGradBus()
-            if hasattr(self, "edge_model") and isinstance(self.edge_model.norm, torch.nn.Module) and self.edge_model.training:
-                bus.edge_beta = self.edge_model.norm.bias
         if hasattr(self, "edge_model"):
             self.edge_model._defer = defer
-            self.edge_model._xe_bus = bus
             try:
                 x_e = self.edge_model(x_s, x_t, edge_index, x_e, x_u)
             finally:
                 self.edge_model._defer = None
-                self.edge_model._xe_bus = None
         edge_affine = defer.pop("affine", None) if defer else None
         x_e_s = x_e_t = x_e
         if bus is not None and x_e.requires_grad:
