@@ -38,19 +38,20 @@
 extern "C" {
 #endif
 
-#define PFS_ABI_VERSION 6
+#define PFS_ABI_VERSION 7
 
 enum {
     PFS_OK = 0,
     PFS_ERR_ARG = -1,        /* bad argument (null pointer, unsupported F, ...) */
     PFS_ERR_CUDA = -2,       /* CUDA runtime error (message has the cudaGetErrorString) */
-    PFS_ERR_UNSUPPORTED = -3,/* valid request this build cannot serve (e.g. fibre degree > tile) */
+    PFS_ERR_UNSUPPORTED = -3,/* valid request this build cannot serve (e.g. an Fdim without kernels) */
     PFS_ERR_WORKSPACE = -4   /* workspace too small */
 };
 
 enum { PFS_LAYOUT_DENSE = 0, PFS_LAYOUT_CSR = 1 };
 
-/* edges processed by one CTA tile; a fibre's edges never straddle tiles (max fibre degree) */
+/* edges processed by one CTA tile.  A tile holds whole fibres; a fibre with more edges is split
+ * over consecutive tiles of its own (see the split fields of pfs_topology). */
 #define PFS_TILE_EDGES 256
 
 /*
@@ -69,10 +70,20 @@ typedef struct pfs_topology {
     const int32_t* csr_eid;    /* [E]    original edge id (row of x_e) at CSR position q      */
     const int32_t* csr_src;    /* [E]    fibre at CSR position q                              */
     const int32_t* csr_tgt;    /* [E]    class at CSR position q                              */
-    const int32_t* tile_fibre; /* [ntiles+1] first fibre of every tile (whole fibres, <= PFS_TILE_EDGES edges) */
+    const int32_t* tile_fibre; /* [ntiles+1] first fibre of every tile (<= PFS_TILE_EDGES edges)           */
     int32_t ntiles;            /* tiles per graph (CSR layout; dense layout derives it)       */
     const int32_t* csc_colptr; /* [T+1]  first CSC position of each class                     */
     const int32_t* csc_q;      /* [E]    CSR position of the k-th class-sorted edge           */
+    /* ABI 7: split tiles (from pfs_build_split_tiles, used when a fibre has more than PFS_TILE_EDGES
+     * edges).  A split tile holds one chunk [tile_q[i], tile_q[i+1]) of one fibre's edges; its per-fibre
+     * results go to a partial-record slot and are combined per fibre in slot order.  All NULL / 0: every
+     * tile holds whole fibres (the table of pfs_build_topology). */
+    const int32_t* tile_q;     /* [ntiles+1] first CSR position of every tile                 */
+    const int32_t* tile_slot;  /* [ntiles]   partial-record slot of a split tile, -1 for whole fibres */
+    const int32_t* split_fibre;/* [nsplit]   the split fibres, ascending                      */
+    const int32_t* split_ptr;  /* [nsplit+1] slots of split fibre i: [split_ptr[i], split_ptr[i+1]) */
+    int32_t nsplit;            /* split fibres                                                 */
+    int32_t nslots;            /* partial-record slots (= split tiles) per graph               */
 } pfs_topology;
 
 /* -------------------------------------------------------------------------------------------
@@ -119,6 +130,15 @@ int pfs_build_topology(const int64_t* edge_index, int64_t E, int32_t S, int32_t 
                        int32_t* csc_colptr, int32_t* csc_q, int32_t* tile_fibre,
                        int32_t* ntiles_dev, int32_t* max_degree_dev,
                        void* temp, size_t temp_bytes, void* stream);
+/* Tile table for a topology with fibres of more than PFS_TILE_EDGES edges, over the CSR order of
+ * pfs_build_topology.  Whole fibres are packed greedily as pfs_build_topology packs them; a fibre of
+ * d > PFS_TILE_EDGES edges gets ceil(d / PFS_TILE_EDGES) consecutive tiles of its own with balanced
+ * chunk sizes (sizes differ by at most one, the larger ones first).  Capacities (device int32):
+ * tile_fibre, tile_q [S + E/PFS_TILE_EDGES + 2], tile_slot [S + E/PFS_TILE_EDGES + 1], split_fibre [S],
+ * split_ptr [S+1]; counts_dev [3] receives ntiles, nsplit and nslots.  Sequential, once per topology. */
+int pfs_build_split_tiles(const int32_t* csr_rowptr, int32_t S, int32_t* tile_fibre, int32_t* tile_q,
+                          int32_t* tile_slot, int32_t* split_fibre, int32_t* split_ptr, int32_t* counts_dev,
+                          void* stream);
 
 /* -------------------------------------------------------------------------------------------
  * EdgeModel  (reference src/gnn.py:73-101: gather + cat + MLP(4F,4F,F) + BatchNorm1d applied twice)

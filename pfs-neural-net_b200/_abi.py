@@ -18,7 +18,7 @@ HEADER = os.path.join(os.path.dirname(_HERE), "include", "pfs_b200.h")
 PFS_LAYOUT_DENSE = 0
 PFS_LAYOUT_CSR = 1
 PFS_TILE_EDGES = 256
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 _P = ct.c_void_p
 
@@ -37,6 +37,8 @@ class TopologyStruct(ct.Structure):
         (_P, "csr_rowptr csr_eid csr_src csr_tgt tile_fibre"),
         (ct.c_int32, "ntiles"),
         (_P, "csc_colptr csc_q"),
+        (_P, "tile_q tile_slot split_fibre split_ptr"),     # ABI 7: split tiles
+        (ct.c_int32, "nsplit nslots"),
     ])
 
 
@@ -153,6 +155,7 @@ SYMBOLS = {
     "pfs_detect_dense": (ct.c_int, [_P, _I64, _I32, _I32, _P, _P]),
     "pfs_build_topology_temp_bytes": (ct.c_size_t, [_I64, _I32, _I32]),
     "pfs_build_topology": (ct.c_int, [_P, _I64, _I32, _I32] + [_P] * 9 + [_P, ct.c_size_t, _P]),
+    "pfs_build_split_tiles": (ct.c_int, [_P, _I32] + [_P] * 6 + [_P]),
     "pfs_edge_fwd": (ct.c_int, [ct.POINTER(EdgeArgs)]),
     "pfs_edge_bwd": (ct.c_int, [ct.POINTER(EdgeArgs)]),
     "pfs_source_fwd": (ct.c_int, [ct.POINTER(SourceArgs)]),

@@ -204,6 +204,12 @@ int make_topo(const pfs_topology& t, Topo& o) {
     o.layout = t.layout; o.G = t.G; o.F = t.F; o.S = t.S; o.T = t.T; o.E = t.E;
     o.rowptr = t.csr_rowptr; o.eid = t.csr_eid; o.csrc = t.csr_src; o.ctgt = t.csr_tgt;
     o.tile_fibre = t.tile_fibre; o.colptr = t.csc_colptr; o.cscq = t.csc_q;
+    o.tile_q = t.tile_q; o.tile_slot = t.tile_slot; o.split_fibre = t.split_fibre; o.split_ptr = t.split_ptr;
+    o.nsplit = t.nsplit; o.nslots = t.nslots;
+    if (t.nsplit != 0) {
+        PFS_REQUIRE(t.layout == PFS_LAYOUT_CSR && t.nsplit > 0 && t.nslots >= 2 * t.nsplit && t.tile_q && t.tile_slot &&
+                        t.split_fibre && t.split_ptr, "split tiles need the CSR layout and the arrays of pfs_build_split_tiles");
+    }
     if (t.layout == PFS_LAYOUT_DENSE) {
         if ((long long)t.S * t.T != t.E) return fail(PFS_ERR_ARG, "dense layout needs E == S*T");
         o.fpt = dense_fpt(t.T);
@@ -420,6 +426,13 @@ int class_sums(const Topo& tp, const float* part_or_rows, int J, float* out, flo
     }
     return PFS_OK;
 }
+// fibre sums of the split fibres from the partial rows of their tiles (W floats per row)
+int split_sums(const Topo& tp, int W, const float* part, float* out, cudaStream_t st) {
+    const long long n = (long long)tp.G * tp.nsplit * W;
+    k_split_sums<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(tp, W, part, out);
+    PFS_LAUNCH_CHECK("k_split_sums");
+    return PFS_OK;
+}
 size_t class_stage_floats(const Topo& tp, int J) {
     return tp.layout == PFS_LAYOUT_DENSE ? (size_t)tp.G * tp.ntiles * tp.T * J : (size_t)tp.G * tp.E * J;
 }
@@ -474,8 +487,9 @@ int edge_fwd_impl(const pfs_edge_args& a, const Topo& tp) {
     size_t smem = 0;
     const int nbuf = pick_nbuf([&](int nb) { return sizeof(float) * TileStage<F, 1, H, H>::floats(max_fib, tp.T, sc, nb); }, smem);
     if (!nbuf) return fail(PFS_ERR_UNSUPPORTED, "edge_fwd: tile staging does not fit shared memory");
-    PFS_TRY(allow_smem(k_edge_fwd<F>, smem));
-    const int grid = persistent_grid(k_edge_fwd<F>, smem, total);
+    auto kern = tp.nsplit > 0 ? k_edge_fwd<F, true> : k_edge_fwd<F>;
+    PFS_TRY(allow_smem(kern, smem));
+    const int grid = persistent_grid(kern, smem, total);
     const int nrec = chunk_records(grid, total, tp.ntiles);
     Bump ws(a.workspace, a.workspace_bytes);
     float* uvec = ws.f((size_t)tp.G * H);
@@ -496,7 +510,7 @@ int edge_fwd_impl(const pfs_edge_args& a, const Topo& tp) {
     PFS_TRY((run_prep<F, H>(tp.G, jobs, 2, a.w1, H, a.u, pl, 2 * F * H + F, wstage, st)));
     const bool stats = a.normed && a.training;
     EdgeFwdParams p{tp, a.x_e, Ps, Pt, a.w1, a.w2, a.b2, a.x_e_out, stats ? part : nullptr, max_fib, sc ? 1 : 0, nrec, nbuf};
-    k_edge_fwd<F><<<grid, kThreads, smem, st>>>(p);
+    kern<<<grid, kThreads, smem, st>>>(p);
     PFS_LAUNCH_CHECK("k_edge_fwd");
     if (a.normed) {
         PFS_REQUIRE(a.gamma && a.beta && a.bn_save, "normed edge model needs gamma, beta, bn_save");
@@ -520,7 +534,8 @@ int edge_bwd_impl(const pfs_edge_args& a, const Topo& tp) {
     // its tiles fit 113 KB, else the double-buffered one-CTA-per-SM k_edge_bwd (Fdim 16).
     // Measured at C3: 1.21 ms against 1.60 ms.
     constexpr bool lean = SM::lean_fits;
-    auto kern = lean ? k_edge_bwd2<F> : k_edge_bwd<F>;
+    const bool split = tp.nsplit > 0;
+    auto kern = lean ? (split ? k_edge_bwd2<F, true> : k_edge_bwd2<F>) : (split ? k_edge_bwd<F, true> : k_edge_bwd<F>);
     const int max_fib = max_fibres_per_tile(tp);
     const bool sc = stage_class_table(tp, H);
     size_t smem_bwd = SM::bytes_lean;
@@ -551,6 +566,7 @@ int edge_bwd_impl(const pfs_edge_args& a, const Topo& tp) {
     float* opart = ws.f((size_t)kMaxCtas * (H * F + H));
     float* opart2 = ws.f((size_t)((tp.G * tp.T + kTile - 1) / kTile + 1) * (H * F + H));     // class table: few row tiles
     float* wstage = ws.f(kConstFloats);
+    float* dPs_split = split ? ws.f((size_t)tp.G * tp.nslots * H) : nullptr;
     if (!ws.ok) return fail(PFS_ERR_WORKSPACE, "edge_bwd: workspace too small (%zu B)", a.workspace_bytes);
     {
         (void)uvec;
@@ -570,8 +586,9 @@ int edge_bwd_impl(const pfs_edge_args& a, const Topo& tp) {
     PFS_LAUNCH_CHECK("k_edge_bn_bwd_coef/0");
     if (mode != 0) {
         EdgeBnStatParams sp{tp, a.x_e_out, a.g_out, coef, statp};
-        const int g2 = persistent_grid(k_edge_bn_bwd_stats<F>, 0, total);
-        k_edge_bn_bwd_stats<F><<<g2, kThreads, 0, st>>>(sp);
+        auto ks = split ? k_edge_bn_bwd_stats<F, true> : k_edge_bn_bwd_stats<F>;
+        const int g2 = persistent_grid(ks, 0, total);
+        ks<<<g2, kThreads, 0, st>>>(sp);
         PFS_LAUNCH_CHECK("k_edge_bn_bwd_stats");
         k_tile_partial_sums<<<tp.G, 256, 0, st>>>(statp, tp.ntiles, 2 * F, statsum);
         PFS_LAUNCH_CHECK("k_tile_partial_sums");
@@ -583,7 +600,7 @@ int edge_bwd_impl(const pfs_edge_args& a, const Topo& tp) {
     }
     const bool dense = tp.layout == PFS_LAYOUT_DENSE;
     EdgeBwdParams p{tp, a.x_e, a.x_e_out, a.g_out, Ps, Pt, coef, a.g_x_e, dPs,
-                    dense ? stage : nullptr, dense ? nullptr : stage, wpart, pstride, max_fib, sc ? 1 : 0, nbuf};
+                    dense ? stage : nullptr, dense ? nullptr : stage, wpart, pstride, max_fib, sc ? 1 : 0, nbuf, dPs_split};
     kern<<<grid, kThreads, smem_bwd, st>>>(p);
     if (lean) {
         PFS_LAUNCH_CHECK("k_edge_bwd2");
@@ -596,6 +613,7 @@ int edge_bwd_impl(const pfs_edge_args& a, const Topo& tp) {
     rd.add(H * F, F * H, H, a.g_w2, H, 0);
     rd.add(2 * H * F, F, F, a.g_b2, F, 0);
     PFS_TRY(class_sums(tp, stage, H, dPt, cscs, st));
+    if (split) PFS_TRY(split_sums(tp, H, dPs_split, dPs, st));
     // node-table backward, one pass per table: g_x_s = dPs . W1_s, dW1_s += dPs^T x_s (the same for the class table)
     PFS_TRY((outer_rows<H, F, 8, F / 2>(rd, dPs, a.x_s, (long long)tp.G * tp.S, opart, a.g_w1, H, 0, nullptr, st, a.w1, a.g_x_s)));
     PFS_TRY((outer_rows<H, F, 8, F / 2>(rd, dPt, a.x_t, (long long)tp.G * tp.T, opart2, a.g_w1, H, F, nullptr, st, a.w1, a.g_x_t)));
@@ -621,6 +639,8 @@ int source_fwd_impl(const pfs_source_args& a, const Topo& tp) {
     float* Qt = ws.f((size_t)tp.G * tp.T * M);
     float* partn = ws.f((size_t)tp.G * ntn * bn_partial_stride(F));
     float* wstage = ws.f(kConstFloats);
+    const bool split = tp.nsplit > 0;
+    float* srec = split ? ws.f((size_t)tp.G * tp.nslots * moment_record_floats(M)) : nullptr;
     if (!ws.ok) return fail(PFS_ERR_WORKSPACE, "source_fwd: workspace too small (%zu B)", a.workspace_bytes);
     {
         // one prologue: the class table Q_t, the message-MLP weights and the node-MLP weights (disjoint regions of the
@@ -640,10 +660,16 @@ int source_fwd_impl(const pfs_source_args& a, const Topo& tp) {
     }
     {
         if (a.x_e_affine) PFS_REQUIRE(a.x_e_norm_out, "x_e_affine needs x_e_norm_out");
-        SourceEdgeFwdParams p{tp, a.x_e, Qt, a.w1, a.w2, a.b2, a.moments, a.x_e_affine, a.x_e_norm_out};
-        const int grid = persistent_grid(k_source_edge_fwd<F>, 0, total);
-        k_source_edge_fwd<F><<<grid, kThreads, 0, st>>>(p);
+        SourceEdgeFwdParams p{tp, a.x_e, Qt, a.w1, a.w2, a.b2, a.moments, a.x_e_affine, a.x_e_norm_out, srec};
+        auto kern = split ? k_source_edge_fwd<F, true> : k_source_edge_fwd<F>;
+        const int grid = persistent_grid(kern, 0, total);
+        kern<<<grid, kThreads, 0, st>>>(p);
         PFS_LAUNCH_CHECK("k_source_edge_fwd");
+        if (split) {
+            const long long n = (long long)tp.G * tp.nsplit * M;
+            k_split_moments<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(tp, M, srec, a.moments);
+            PFS_LAUNCH_CHECK("k_split_moments");
+        }
     }
     {
         const bool stats = a.normed && a.training;
@@ -687,7 +713,7 @@ int source_bwd_impl(const pfs_source_args& a, const Topo& tp) {
     const int mode = !a.normed ? 0 : (a.training ? 1 : 2);
     constexpr size_t smem_e = SourceEdgeBwdSmem<F>::bytes;
     constexpr bool kNodeMma = SourceNodeBwdMma<F>::fits;
-    auto ke = k_source_edge_bwd<F>;
+    auto ke = tp.nsplit > 0 ? k_source_edge_bwd<F, true> : k_source_edge_bwd<F>;
     PFS_TRY(allow_smem(ke, smem_e));
     int gridn = 0;
     if constexpr (kNodeMma) {
@@ -825,8 +851,9 @@ int target_fwd_impl(const pfs_target_args& a, const Topo& tp) {
     {
         const bool dense = tp.layout == PFS_LAYOUT_DENSE;
         TargetEdgeFwdParams p{tp, a.x_e, Rs, a.w1, dense ? stage : nullptr, dense ? nullptr : stage};
-        const int grid = persistent_grid(k_target_edge_fwd<F>, 0, total);
-        k_target_edge_fwd<F><<<grid, kThreads, 0, st>>>(p);
+        auto kern = tp.nsplit > 0 ? k_target_edge_fwd<F, true> : k_target_edge_fwd<F>;
+        const int grid = persistent_grid(kern, 0, total);
+        kern<<<grid, kThreads, 0, st>>>(p);
         PFS_LAUNCH_CHECK("k_target_edge_fwd");
     }
     PFS_TRY(class_sums(tp, stage, M, a.act_sum, cscs, st));
@@ -853,7 +880,8 @@ int target_bwd_impl(const pfs_target_args& a, const Topo& tp) {
     prof_mark(nullptr, st);
     const int total = tp.ntiles * tp.G;
     using SM = TargetEdgeBwdSmem<F>;
-    auto ke = k_target_edge_bwd<F>;
+    const bool split = tp.nsplit > 0;
+    auto ke = split ? k_target_edge_bwd<F, true> : k_target_edge_bwd<F>;
     PFS_TRY(allow_smem(ke, SM::bytes));
     const int gride = persistent_grid(ke, SM::bytes, total);
     constexpr int pstride_e = M * F;
@@ -867,6 +895,7 @@ int target_bwd_impl(const pfs_target_args& a, const Topo& tp) {
     float* wpe = ws.f((size_t)gride * pstride_e);
     float* opart = ws.f((size_t)kMaxCtas * (M * F + M));
     float* wstage = ws.f(kConstFloats);
+    float* dRs_split = split ? ws.f((size_t)tp.G * tp.nslots * M) : nullptr;
     if (!ws.ok) return fail(PFS_ERR_WORKSPACE, "target_bwd: workspace too small (%zu B)", a.workspace_bytes);
     {
         TargetTailParams p = make_tail(a, tp);
@@ -899,10 +928,11 @@ int target_bwd_impl(const pfs_target_args& a, const Topo& tp) {
         PFS_TRY((run_prep<F, M>(tp.G, jobs, cached ? 0 : 1, a.w1, M, a.u, pl, MsgEdgeConst<F>::kFloats, wstage, st)));
     }
     {
-        TargetEdgeBwdParams p{tp, a.x_e, Rs, a.w1, dasum, a.g_x_e, a.g_x_e_add, dRs, wpe, pstride_e};
+        TargetEdgeBwdParams p{tp, a.x_e, Rs, a.w1, dasum, a.g_x_e, a.g_x_e_add, dRs, wpe, pstride_e, dRs_split};
         ke<<<gride, kThreads, SM::bytes, st>>>(p);
         PFS_LAUNCH_CHECK("k_target_edge_bwd");
     }
+    if (split) PFS_TRY(split_sums(tp, M, dRs_split, dRs, st));
     rd.source(wpe, gride, pstride_e);
     rd.add(0, M * F, F, a.g_w1, M, F);
     PFS_TRY((outer_rows<M, F, 4, F / 2>(rd, dRs, a.x_s, (long long)tp.G * tp.S, opart, a.g_w1, M, 0, a.g_b1, st, a.w1, a.g_x_s)));
@@ -1002,6 +1032,48 @@ __global__ void k_pack_tiles(const int* rowptr, int S, int* tile_fibre, int* nti
     *max_degree = maxd;
 }
 
+// Tile table with split fibres (sequential, one-time per topology): whole fibres packed as k_pack_tiles packs them, a
+// fibre of d > kTile edges cut into ceil(d / kTile) consecutive tiles of its own whose sizes differ by at most one
+// (257 -> 129 + 128: no chunk of a handful of edges)
+__global__ void k_pack_split_tiles(const int* rowptr, int S, int* tile_fibre, int* tile_q, int* tile_slot, int* split_fibre,
+                                   int* split_ptr, int* counts) {
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    int nt = 0, cur = 0, nf = 0, ns = 0, nslot = 0;
+    bool open = false;                      // the last tile holds whole fibres and may take more
+    for (int f = 0; f < S; ++f) {
+        const int q = rowptr[f], d = rowptr[f + 1] - q;
+        if (d > kTile) {
+            const int k = (d + kTile - 1) / kTile, base = d / k, rem = d - base * k;
+            split_fibre[ns] = f;
+            split_ptr[ns++] = nslot;
+            for (int c = 0, qc = q; c < k; ++c) {
+                tile_fibre[nt] = f;
+                tile_q[nt] = qc;
+                tile_slot[nt++] = nslot++;
+                qc += base + (c < rem ? 1 : 0);
+            }
+            open = false;
+            continue;
+        }
+        if (!open || (cur + d > kTile && cur > 0) || nf >= kTile) {
+            tile_fibre[nt] = f;
+            tile_q[nt] = q;
+            tile_slot[nt++] = -1;
+            cur = 0;
+            nf = 0;
+            open = true;
+        }
+        cur += d;
+        ++nf;
+    }
+    tile_fibre[nt] = S;
+    tile_q[nt] = rowptr[S];
+    split_ptr[ns] = nslot;
+    counts[0] = nt;
+    counts[1] = ns;
+    counts[2] = nslot;
+}
+
 size_t sort_temp_bytes(long long E) {
     size_t bytes = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, bytes, (const int*)nullptr, (int*)nullptr, (const int*)nullptr,
@@ -1083,6 +1155,7 @@ size_t pfs_workspace_bytes(const pfs_topology* t) {
     fl += 2 * kConstFloats;                                       // weight staging for the constant bank
     fl += G * (36 * F * F + 128 * F);
     fl += G * 64 * 2 * F + 64;                                   // chunk partials of the node BatchNorm backward sums
+    if (t->nsplit > 0) fl += G * (size_t)t->nslots * (10 * F + 1) + 64;   // split tiles: chunk records / partial fibre sums
     fl += 4096;
     return fl * sizeof(float) + 64 * 256;
 }
@@ -1139,6 +1212,16 @@ int pfs_build_topology(const int64_t* edge_index, int64_t E, int32_t S, int32_t 
     PFS_LAUNCH_CHECK("k_lower_bounds(tgt)");
     k_pack_tiles<<<1, 1, 0, st>>>(csr_rowptr, S, tile_fibre, ntiles_dev, max_degree_dev);
     PFS_LAUNCH_CHECK("k_pack_tiles");
+    return PFS_OK;
+}
+
+int pfs_build_split_tiles(const int32_t* csr_rowptr, int32_t S, int32_t* tile_fibre, int32_t* tile_q, int32_t* tile_slot,
+                          int32_t* split_fibre, int32_t* split_ptr, int32_t* counts_dev, void* stream) {
+    PFS_REQUIRE(csr_rowptr && tile_fibre && tile_q && tile_slot && split_fibre && split_ptr && counts_dev, "null pointer");
+    PFS_REQUIRE(S >= 1, "bad sizes");
+    cudaStream_t st = (cudaStream_t)stream;
+    k_pack_split_tiles<<<1, 1, 0, st>>>(csr_rowptr, S, tile_fibre, tile_q, tile_slot, split_fibre, split_ptr, counts_dev);
+    PFS_LAUNCH_CHECK("k_pack_split_tiles");
     return PFS_OK;
 }
 

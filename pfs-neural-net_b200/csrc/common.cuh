@@ -34,21 +34,35 @@ struct Topo {
     int ntiles;  // tiles per graph
     const int *colptr, *cscq;
     int fpt;     // fibres per tile (dense layout)
+    // split tiles (CSR layout, a fibre of more than kTile edges): see pfs_topology in include/pfs_b200.h
+    const int *tile_q, *tile_slot, *split_fibre, *split_ptr;
+    int nsplit, nslots;
 };
 
 struct Tile {
     int g, lt, fibre0, nfib, q0, ne;
+    int slot;    // partial-record slot of a split tile (one chunk of one fibre), else -1
 };
 
+// SPLIT: the topology has split tiles (Topo::nsplit > 0).  The kernels that run on such a topology are separate
+// instantiations, so the ones for whole-fibre tables compile exactly as without the split handling.
+template <bool SPLIT = false>
 __device__ __forceinline__ Tile get_tile(const Topo& tp, int tile) {
     Tile t;
     t.g = tile / tp.ntiles;
     t.lt = tile - t.g * tp.ntiles;
+    t.slot = -1;
     if (tp.layout == PFS_LAYOUT_DENSE) {
         t.fibre0 = t.lt * tp.fpt;
         t.nfib = min(tp.fpt, tp.S - t.fibre0);
         t.q0 = t.fibre0 * tp.T;
         t.ne = t.nfib * tp.T;
+    } else if constexpr (SPLIT) {
+        t.fibre0 = tp.tile_fibre[t.lt];
+        t.q0 = tp.tile_q[t.lt];
+        t.ne = tp.tile_q[t.lt + 1] - t.q0;
+        t.slot = tp.tile_slot[t.lt];
+        t.nfib = t.slot >= 0 ? 1 : tp.tile_fibre[t.lt + 1] - t.fibre0;
     } else {
         t.fibre0 = tp.tile_fibre[t.lt];
         const int f1 = tp.tile_fibre[t.lt + 1];
@@ -79,11 +93,17 @@ __device__ __forceinline__ EdgeRef get_edge(const Topo& tp, const Tile& t, int t
     return r;
 }
 
-// edges of local fibre lf inside the tile: [e0, e0 + n)
+// edges of local fibre lf inside the tile: [e0, e0 + n) (SPLIT: clipped to the tile, a split tile holds a chunk)
+template <bool SPLIT = false>
 __device__ __forceinline__ void fibre_range(const Topo& tp, const Tile& t, int lf, int& e0, int& n) {
     if (tp.layout == PFS_LAYOUT_DENSE) {
         e0 = lf * tp.T;
         n = tp.T;
+    } else if constexpr (SPLIT) {
+        const int a = max(tp.rowptr[t.fibre0 + lf], t.q0);
+        const int b = min(tp.rowptr[t.fibre0 + lf + 1], t.q0 + t.ne);
+        e0 = a - t.q0;
+        n = b - a;
     } else {
         const int a = tp.rowptr[t.fibre0 + lf];
         e0 = a - t.q0;
@@ -654,7 +674,7 @@ struct RunningStats {
 // Threads [T0, T0 + NT) of the CTA take part (whole warps).  Two running sums per thread (even / odd edges, added at
 // the end) halve the dependent FADD chain and keep 8 loads in flight: these sums are latency-bound, not
 // bandwidth-bound (ncu source view of k_edge_bwd2: 16 % of the stall samples sat on their FADDs).
-template <int W, int LD, int T0 = 0, int NT = kThreads>
+template <int W, int LD, int T0 = 0, int NT = kThreads, bool SPLIT = false>
 __device__ __forceinline__ void tile_fibre_sums(const Topo& tp, const Tile& t, const float* X, float* __restrict__ out) {
     static_assert(W % 4 == 0 && LD % 4 == 0 && T0 % 32 == 0 && NT % 32 == 0, "16-byte rows, whole warps");
     constexpr int W4 = W / 4;
@@ -663,7 +683,7 @@ __device__ __forceinline__ void tile_fibre_sums(const Topo& tp, const Tile& t, c
     for (int i = tt; i < t.nfib * W4; i += NT) {
         const int lf = i / W4, k = (i - lf * W4) * 4;
         int e0, n;
-        fibre_range(tp, t, lf, e0, n);
+        fibre_range<SPLIT>(tp, t, lf, e0, n);
         const float4* x = reinterpret_cast<const float4*>(X + e0 * LD + k);
         float4 s = make_float4(0.f, 0.f, 0.f, 0.f), s1 = s;
         int e = 0;
@@ -712,6 +732,28 @@ __device__ __forceinline__ void tile_class_sums(const Topo& tp, const Tile& t, c
         s.w += __shfl_xor_sync(0xffffffffu, s.w, 1);
         if (on && half == 0) *reinterpret_cast<float4*>(cp + c * W + k) = s;
     }
+}
+
+// Row of the fibre sums of tile t: the fibre table's row of its first fibre, or the tile's partial-record row when the
+// tile is one chunk of a split fibre (W floats per row, nslots rows per graph; combined by k_split_sums)
+template <bool SPLIT>
+__device__ __forceinline__ float* fibre_sum_row(const Topo& tp, const Tile& t, float* table, float* split_part, int W) {
+    if constexpr (SPLIT) {
+        if (t.slot >= 0) return split_part + ((size_t)t.g * tp.nslots + t.slot) * W;
+    }
+    return table + ((size_t)t.g * tp.S + t.fibre0) * W;
+}
+
+// out[(g, split_fibre[i])][k] = sum of the partial rows of split fibre i, in slot order (W floats per row)
+__global__ void k_split_sums(const Topo tp, int W, const float* __restrict__ part, float* __restrict__ out) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)tp.G * tp.nsplit * W) return;
+    const int k = (int)(i % W);
+    const long long gs = i / W;
+    const int g = (int)(gs / tp.nsplit), sf = (int)(gs - (long long)g * tp.nsplit);
+    float s = 0.f;
+    for (int q = tp.split_ptr[sf]; q < tp.split_ptr[sf + 1]; ++q) s += part[((size_t)g * tp.nslots + q) * W + k];
+    out[((size_t)g * tp.S + tp.split_fibre[sf]) * W + k] = s;
 }
 
 // ------------------------------------------------------------------------------------------

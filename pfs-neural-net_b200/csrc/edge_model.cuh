@@ -28,7 +28,7 @@ struct EdgeFwdParams {
     int nbuf;           // staging buffers (2 = prefetch the next tile)
 };
 
-template <int F>
+template <int F, bool SPLIT = false>
 __global__ void __launch_bounds__(kThreads, 2) k_edge_fwd(const EdgeFwdParams p) {
     constexpr int H = 4 * F;
     using Stage = TileStage<F, 1, H, H>;
@@ -40,7 +40,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_edge_fwd(const EdgeFwdParams p)
     Stage stg;
     stg.init(dyn, p.max_fib, tp.T, p.stage_class != 0, p.nbuf);
     const float* esrc[1] = {p.x_e};
-    auto tile_of = [&](int i) { return get_tile(tp, i); };
+    auto tile_of = [&](int i) { return get_tile<SPLIT>(tp, i); };
     const int total = tp.ntiles * tp.G;
     const int t_begin = chunk_begin(blockIdx.x, gridDim.x, total), t_end = chunk_begin(blockIdx.x + 1, gridDim.x, total);
     RunningStats<F> rs;
@@ -49,7 +49,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_edge_fwd(const EdgeFwdParams p)
     int slot = 0, cur_graph = -1, par = 0;
     stg.prologue(tp, t_begin, t_end, esrc, p.Ps, p.Pt, tile_of);
     for (int tile = t_begin; tile < t_end; ++tile, par ^= 1) {
-        const Tile t = get_tile(tp, tile);
+        const Tile t = get_tile<SPLIT>(tp, tile);
         const int b = stg.step(tp, tile, t_end, par, esrc, p.Ps, p.Pt, tile_of);   // this tile's copies have landed
         if (rec && t.g != cur_graph) {   // graph boundary: emit the finished graph's statistics
             if (cur_graph >= 0) rs.flush(red, rec + (size_t)(slot++) * bn_partial_stride(F), cur_graph);
@@ -97,7 +97,7 @@ struct EdgeBnStatParams {
 // of that range and reduced over the CTA ONCE per segment (not once per tile: the 2F warp-shuffle trees per tile
 // made this streaming kernel instruction-bound at half the HBM rate).  The segment's sums go to the slot of its
 // first tile, the other tiles of the segment get zeros, so the per-graph consumer (k_tile_partial_sums) is unchanged.
-template <int F>
+template <int F, bool SPLIT = false>
 __global__ void __launch_bounds__(kThreads) k_edge_bn_bwd_stats(const EdgeBnStatParams p) {
     __shared__ float red[kWarps * 2 * F];
     const Topo& tp = p.tp;
@@ -109,7 +109,7 @@ __global__ void __launch_bounds__(kThreads) k_edge_bn_bwd_stats(const EdgeBnStat
     for (int j = 0; j < F; ++j) sg[j] = sx[j] = 0.f;
     int seg_first = t_begin;
     for (int tile = t_begin; tile < t_end; ++tile) {
-        const Tile t = get_tile(tp, tile);
+        const Tile t = get_tile<SPLIT>(tp, tile);
         if (threadIdx.x < t.ne) {
             const EdgeRef er = get_edge(tp, t, threadIdx.x);
             const size_t row = ((size_t)t.g * tp.E + er.e) * F;
@@ -223,6 +223,7 @@ struct EdgeBwdParams {
     float* wpartial;                 // [ncta][pstride]: dW1_e [4F*F], dW2 [F*4F], db2 [F]
     int pstride;
     int max_fib, stage_class, nbuf;
+    float* dPs_split;                // split tiles: [G,nslots,4F] partial fibre sums of dh (k_split_sums -> dPs)
 };
 
 // constant-bank layout of the edge backward (floats): W1_e input-major [F][H] (recompute h),
@@ -253,7 +254,7 @@ struct EdgeBwdSmem {
     static constexpr bool lean_fits = bytes_lean <= 113 * 1024;
 };
 
-template <int F>
+template <int F, bool SPLIT = false>
 __global__ void __launch_bounds__(kThreads) k_edge_bwd(const EdgeBwdParams p) {
     constexpr int H = 4 * F;
     using SM = EdgeBwdSmem<F>;
@@ -267,7 +268,7 @@ __global__ void __launch_bounds__(kThreads) k_edge_bwd(const EdgeBwdParams p) {
     const Topo& tp = p.tp;
     Stage stg;
     stg.init(DZ + kTile * LDF, p.max_fib, tp.T, p.stage_class != 0, p.nbuf);
-    auto tile_of = [&](int i) { return get_tile(tp, i); };
+    auto tile_of = [&](int i) { return get_tile<SPLIT>(tp, i); };
     // the two weight-gradient accumulations run side by side on the two halves of the CTA
     typename SM::AccW1 accw1;
     typename SM::AccW2 accw2;
@@ -282,7 +283,7 @@ __global__ void __launch_bounds__(kThreads) k_edge_bwd(const EdgeBwdParams p) {
     int par = 0;
     stg.prologue(tp, t_begin, t_end, esrc, p.Ps, p.Pt, tile_of);
     for (int tile = t_begin; tile < t_end; ++tile, par ^= 1) {
-        const Tile t = get_tile(tp, tile);
+        const Tile t = get_tile<SPLIT>(tp, tile);
         const int b = stg.step(tp, tile, t_end, par, esrc, p.Ps, p.Pt, tile_of);
         __syncthreads();
         const float* XE = stg.edge(b, 0);
@@ -329,7 +330,7 @@ __global__ void __launch_bounds__(kThreads) k_edge_bwd(const EdgeBwdParams p) {
         accw1.accumulate(DH, LDH, XE, F, t.ne);
         accw2.accumulate(DZ, LDF, A1, LDH, t.ne);
         // fibre sums of dh -> dPs, class sums of dh (dense layout: edge lf*T + c belongs to class c)
-        tile_fibre_sums<H, LDH>(tp, t, DH, p.dPs + ((size_t)t.g * tp.S + t.fibre0) * H);
+        tile_fibre_sums<H, LDH, 0, kThreads, SPLIT>(tp, t, DH, fibre_sum_row<SPLIT>(tp, t, p.dPs, p.dPs_split, H));
         if (p.class_part) tile_class_sums<H, LDH>(tp, t, DH, p.class_part + (size_t)tile * tp.T * H);
         __syncthreads();
     }
@@ -388,7 +389,7 @@ __device__ __forceinline__ void edge_bwd_half(const EdgeBwdParams& p, const floa
     if (dh_row_out) store_row<HH>(dh_row_out + HALF * HH, da);
 }
 
-template <int F>
+template <int F, bool SPLIT = false>
 __global__ void __launch_bounds__(kThreads, 2) k_edge_bwd2(const EdgeBwdParams p) {
     constexpr int H = 4 * F;
     using SM = EdgeBwdSmem<F>;
@@ -401,7 +402,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_edge_bwd2(const EdgeBwdParams p
     const Topo& tp = p.tp;
     Stage stg;
     stg.init(DZ + kTile * LDF, 0, tp.T, false, 1);
-    auto tile_of = [&](int i) { return get_tile(tp, i); };
+    auto tile_of = [&](int i) { return get_tile<SPLIT>(tp, i); };
     using AccW1 = OuterAccX<H, F, 8, F / 2, 0, kThreads / 2>;              // dW1_e[j][k] = sum dh_j x_k
     using AccW2 = OuterAccX<F, H, 2, 2 * F, kThreads / 2, kThreads / 2>;   // dW2[j][k]   = sum dz_j a1_k
     constexpr int kAcc = AccW1::kAcc > AccW2::kAcc ? AccW1::kAcc : AccW2::kAcc;
@@ -419,10 +420,10 @@ __global__ void __launch_bounds__(kThreads, 2) k_edge_bwd2(const EdgeBwdParams p
     const int total = tp.ntiles * tp.G;
     const int t_begin = chunk_begin(blockIdx.x, gridDim.x, total), t_end = chunk_begin(blockIdx.x + 1, gridDim.x, total);
     for (int tile = t_begin; tile < t_end; ++tile) {
-        const Tile t = get_tile(tp, tile);
+        const Tile t = get_tile<SPLIT>(tp, tile);
         const int b = stg.step(tp, tile, t_end, 0, esrc, nullptr, nullptr, tile_of);
         if (threadIdx.x == 0 && tile + 1 < t_end && tp.layout == PFS_LAYOUT_DENSE) {   // next tile's slabs -> L2
-            const Tile tn = get_tile(tp, tile + 1);
+            const Tile tn = get_tile<SPLIT>(tp, tile + 1);
             const size_t off = ((size_t)tn.g * tp.E + tn.q0) * F, bytes = (size_t)tn.ne * F * sizeof(float);
             bulk_prefetch_l2(p.x_e + off, bytes);
             bulk_prefetch_l2(p.xe2 + off, bytes);
@@ -461,7 +462,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_edge_bwd2(const EdgeBwdParams p
         // order, so every scheduler always holds a warp of each kind (warp w and warp w + 4 share a scheduler).
         if (threadIdx.x < kThreads / 2) {
             accw1.template accumulate<4, 1>(acc, DH, LDH, XE, F, t.ne);       // DH rows, j0: 16-byte aligned; x_e rows: 40 B
-            tile_fibre_sums<H, LDH, 0, kThreads / 2>(tp, t, DH, p.dPs + ((size_t)t.g * tp.S + t.fibre0) * H);
+            tile_fibre_sums<H, LDH, 0, kThreads / 2, SPLIT>(tp, t, DH, fibre_sum_row<SPLIT>(tp, t, p.dPs, p.dPs_split, H));
         } else {
             if (p.class_part) tile_class_sums<H, LDH, kThreads / 2, kThreads / 2>(tp, t, DH, p.class_part + (size_t)tile * tp.T * H);
             accw2.template accumulate<2, 4>(acc, DZ, LDF, A1, LDH, t.ne);      // dz pairs: 8 bytes; a1 rows, k0: 16 bytes

@@ -30,9 +30,14 @@ struct SourceEdgeFwdParams {
     float* moments;        // [G,S,5,2F]: mean, E[m^2], c2, c3, c4
     const float* xaff;     // [G,4,F] (rows 2, 3: scale, shift) of a deferred EdgeModel norm, or null: xe2 then holds z
     float* xe_norm_out;    // [G,E,F] where x_e' = scale z + shift is stored (may alias xe2)
+    float* split_rec;      // split tiles: [G,nslots,moment_record_floats(2F)] chunk records (k_split_moments -> moments)
 };
 
-template <int F>
+// Chunk record of a split tile, per message feature j (rows of M floats): the sums of m and m^2, the sums of the
+// 2nd, 3rd and 4th powers of m - (chunk mean), then the chunk's edge count.
+__host__ __device__ constexpr int moment_record_floats(int M) { return 5 * M + 1; }
+
+template <int F, bool SPLIT = false>
 __global__ void __launch_bounds__(kThreads) k_source_edge_fwd(const SourceEdgeFwdParams p) {
     constexpr int M = 2 * F;
     constexpr int LDT = kTile + 1;
@@ -41,7 +46,7 @@ __global__ void __launch_bounds__(kThreads) k_source_edge_fwd(const SourceEdgeFw
     const Topo& tp = p.tp;
     const int total = tp.ntiles * tp.G;
     for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
-        const Tile t = get_tile(tp, tile);
+        const Tile t = get_tile<SPLIT>(tp, tile);
         if (threadIdx.x < t.ne) {
             const EdgeRef er = get_edge(tp, t, threadIdx.x);
             float x[F], h[M], m[M];
@@ -67,7 +72,7 @@ __global__ void __launch_bounds__(kThreads) k_source_edge_fwd(const SourceEdgeFw
         for (int i = threadIdx.x; i < t.nfib * M; i += kThreads) {
             const int lf = i / M, j = i - lf * M;
             int e0, n;
-            fibre_range(tp, t, lf, e0, n);
+            fibre_range<SPLIT>(tp, t, lf, e0, n);
             const float* col = MT + j * LDT + e0;
             float s1 = 0.f, s2 = 0.f;
             for (int e = 0; e < n; ++e) {
@@ -85,6 +90,18 @@ __global__ void __launch_bounds__(kThreads) k_source_edge_fwd(const SourceEdgeFw
                 c3 += d2 * d;
                 c4 += d2 * d2;
             }
+            if constexpr (SPLIT) {
+                if (t.slot >= 0) {
+                    float* r = p.split_rec + ((size_t)t.g * tp.nslots + t.slot) * moment_record_floats(M) + j;
+                    r[0] = s1;
+                    r[M] = s2;
+                    r[2 * M] = c2;
+                    r[3 * M] = c3;
+                    r[4 * M] = c4;
+                    if (j == 0) r[5 * M] = (float)n;
+                    continue;
+                }
+            }
             float* o = p.moments + ((size_t)t.g * tp.S + t.fibre0 + lf) * 5 * M + j;
             o[0] = mean;
             o[M] = s2 / cnt;
@@ -94,6 +111,42 @@ __global__ void __launch_bounds__(kThreads) k_source_edge_fwd(const SourceEdgeFw
         }
         __syncthreads();
     }
+}
+
+// Moment rows [mean, E[m^2], c2, c3, c4] of the split fibres from their chunk records: one thread per (graph, split
+// fibre, feature) combines the records in slot order in fp64 with the pairwise update of the central moments
+// (Chan, Golub and LeVeque; Pebay 2008), so the result does not depend on how the fibre was cut.
+__global__ void k_split_moments(const Topo tp, int M, const float* __restrict__ rec, float* __restrict__ moments) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)tp.G * tp.nsplit * M) return;
+    const int j = (int)(i % M);
+    const long long gs = i / M;
+    const int g = (int)(gs / tp.nsplit), sf = (int)(gs - (long long)g * tp.nsplit);
+    const int R = 5 * M + 1;
+    double n = 0.0, mean = 0.0, sq = 0.0, m2 = 0.0, m3 = 0.0, m4 = 0.0;
+    for (int s = tp.split_ptr[sf]; s < tp.split_ptr[sf + 1]; ++s) {
+        const float* r = rec + ((size_t)g * tp.nslots + s) * R;
+        const double nb = r[5 * M];
+        const double mb = (double)r[j] / nb, b2 = r[2 * M + j], b3 = r[3 * M + j], b4 = r[4 * M + j];
+        sq += (double)r[M + j];
+        if (n == 0.0) {
+            n = nb; mean = mb; m2 = b2; m3 = b3; m4 = b4;
+            continue;
+        }
+        const double na = n, nn = na + nb, d = mb - mean, dn = d / nn, dn2 = dn * dn;
+        m4 += b4 + d * dn2 * dn * na * nb * (na * na - na * nb + nb * nb) + 6.0 * dn2 * (na * na * b2 + nb * nb * m2) +
+              4.0 * dn * (na * b3 - nb * m3);
+        m3 += b3 + d * dn2 * na * nb * (na - nb) + 3.0 * dn * (na * b2 - nb * m2);
+        m2 += b2 + d * dn * na * nb;
+        mean += dn * nb;
+        n = nn;
+    }
+    float* o = moments + ((size_t)g * tp.S + tp.split_fibre[sf]) * 5 * M + j;
+    o[0] = (float)mean;
+    o[M] = (float)(sq / n);
+    o[2 * M] = (float)(m2 / n);
+    o[3 * M] = (float)(m3 / n);
+    o[4 * M] = (float)(m4 / n);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -484,7 +537,7 @@ struct SourceEdgeBwdSmem {
     static constexpr size_t bytes = sizeof(float) * (kWeights + kTiles);
 };
 
-template <int F>
+template <int F, bool SPLIT = false>
 __global__ void __launch_bounds__(kThreads, (F <= 10 ? 2 : 1)) k_source_edge_bwd(const SourceEdgeBwdParams p) {
     using SM = SourceEdgeBwdSmem<F>;
     constexpr int M = 2 * F, LDM = SM::LDM, LDF = SM::LDF;
@@ -506,9 +559,9 @@ __global__ void __launch_bounds__(kThreads, (F <= 10 ? 2 : 1)) k_source_edge_bwd
     const Topo& tp = p.tp;
     const int total = tp.ntiles * tp.G;
     for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
-        const Tile t = get_tile(tp, tile);
+        const Tile t = get_tile<SPLIT>(tp, tile);
         if (threadIdx.x == 0 && tile + (int)gridDim.x < total && tp.layout == PFS_LAYOUT_DENSE) {   // next tile -> L2
-            const Tile tn = get_tile(tp, tile + gridDim.x);
+            const Tile tn = get_tile<SPLIT>(tp, tile + gridDim.x);
             const size_t off = ((size_t)tn.g * tp.E + tn.q0) * F, bytes = (size_t)tn.ne * F * sizeof(float);
             const size_t frow = (size_t)tn.g * tp.S + tn.fibre0;
             bulk_prefetch_l2(p.xe2 + off, bytes);
@@ -529,9 +582,14 @@ __global__ void __launch_bounds__(kThreads, (F <= 10 ? 2 : 1)) k_source_edge_bwd
                 m[j] = c_w[CW::kB2 + j];
             }
             dense_acc_c<M, M, CW::kW2t>(a, m);
-            // dm = (A0 + A1 m + A2 d^2 + A3 d^3) / count
-            int e0, n;
-            fibre_range(tp, t, er.src - t.fibre0, e0, n);
+            // dm = (A0 + A1 m + A2 d^2 + A3 d^3) / count, count = the fibre's degree (a split tile holds a chunk of it)
+            int n;
+            if constexpr (SPLIT) {
+                n = tp.rowptr[er.src + 1] - tp.rowptr[er.src];
+            } else {
+                int e0;
+                fibre_range(tp, t, er.src - t.fibre0, e0, n);
+            }
             const float inv = 1.f / (float)max(n, 1);
             const size_t frow = (size_t)t.g * tp.S + er.src;
             const float* cA = p.coefA + frow * 4 * M;

@@ -20,7 +20,7 @@ struct TargetEdgeFwdParams {
     float* act_rows;        // general: [G,E(q),2F]
 };
 
-template <int F>
+template <int F, bool SPLIT = false>
 __global__ void __launch_bounds__(kThreads) k_target_edge_fwd(const TargetEdgeFwdParams p) {
     constexpr int M = 2 * F, LDM = M + 1;
     using CW = MsgEdgeConst<F>;      // only W1t / W1o of the layout are used by the TModel kernels
@@ -28,7 +28,7 @@ __global__ void __launch_bounds__(kThreads) k_target_edge_fwd(const TargetEdgeFw
     const Topo& tp = p.tp;
     const int total = tp.ntiles * tp.G;
     for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
-        const Tile t = get_tile(tp, tile);
+        const Tile t = get_tile<SPLIT>(tp, tile);
         if (threadIdx.x < t.ne) {
             const EdgeRef er = get_edge(tp, t, threadIdx.x);
             float x[F], h[M];
@@ -333,6 +333,7 @@ struct TargetEdgeBwdParams {
     float* dRs;             // [G,S,2F]
     float* wpartial;        // [ncta][pstride]: dW1_e [2F*F]
     int pstride;
+    float* dRs_split;       // split tiles: [G,nslots,2F] partial fibre sums (k_split_sums -> dRs)
 };
 
 template <int F>
@@ -346,7 +347,7 @@ struct TargetEdgeBwdSmem {
     static constexpr size_t bytes = sizeof(float) * kFloats;
 };
 
-template <int F>
+template <int F, bool SPLIT = false>
 __global__ void __launch_bounds__(kThreads) k_target_edge_bwd(const TargetEdgeBwdParams p) {
     using SM = TargetEdgeBwdSmem<F>;
     constexpr int M = 2 * F, LDM = SM::LDM, LDF = SM::LDF;
@@ -360,9 +361,9 @@ __global__ void __launch_bounds__(kThreads) k_target_edge_bwd(const TargetEdgeBw
     const Topo& tp = p.tp;
     const int total = tp.ntiles * tp.G;
     for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
-        const Tile t = get_tile(tp, tile);
+        const Tile t = get_tile<SPLIT>(tp, tile);
         if (threadIdx.x == 0 && tile + (int)gridDim.x < total && tp.layout == PFS_LAYOUT_DENSE) {   // next tile -> L2
-            const Tile tn = get_tile(tp, tile + gridDim.x);
+            const Tile tn = get_tile<SPLIT>(tp, tile + gridDim.x);
             const size_t off = ((size_t)tn.g * tp.E + tn.q0) * F, bytes = (size_t)tn.ne * F * sizeof(float);
             bulk_prefetch_l2(p.xe2 + off, bytes);
             if (p.g_add) bulk_prefetch_l2(p.g_add + off, bytes);
@@ -389,7 +390,7 @@ __global__ void __launch_bounds__(kThreads) k_target_edge_bwd(const TargetEdgeBw
         }
         __syncthreads();
         accw1.accumulate(DHT, LDM, XE, LDF, t.ne);
-        tile_fibre_sums<M, LDM>(tp, t, DHT, p.dRs + ((size_t)t.g * tp.S + t.fibre0) * M);
+        tile_fibre_sums<M, LDM, 0, kThreads, SPLIT>(tp, t, DHT, fibre_sum_row<SPLIT>(tp, t, p.dRs, p.dRs_split, M));
         __syncthreads();
     }
     accw1.flush(DHT, p.wpartial + (size_t)blockIdx.x * p.pstride, F, 0);

@@ -4,7 +4,9 @@ the kernels consume.
   * canonical dense order (reference src/train.py:94, e = k*T + i) is DETECTED on the device, never
     assumed -- `graphs/graph-0.pt` is fibre-major but class-permuted (SURVEY.md section 0.10);
   * anything else gets int32 CSR (fibre-sorted) and CSC (class-sorted) arrays plus a tile table
-    from `pfs_build_topology`, built once per `edge_index` and cached here.
+    from `pfs_build_topology`, built once per `edge_index` and cached here;
+  * when a fibre has more than PFS_TILE_EDGES edges, the fp32 kernels take the split tile table of
+    `pfs_build_split_tiles` instead (built on first use by `struct()`; the bf16 wide path never asks).
 """
 import collections
 import ctypes as ct
@@ -36,6 +38,7 @@ class Topology:
         self.ntiles = 0
         self.max_degree = self.T if self.canonical else None
         self._wide = None
+        self._split = None
         self._workspaces = {}
 
     def csr(self):
@@ -76,19 +79,47 @@ class Topology:
         self.ntiles, self.max_degree = (int(v) for v in scalars.tolist())
         self.arrays = a
 
+    def split_tiles(self):
+        """Tile table of pfs_build_split_tiles (fibres of more than PFS_TILE_EDGES edges cut into chunks), built
+        on first use and cached: {"tile_fibre", "tile_q", "tile_slot", "split_fibre", "split_ptr"} (int32,
+        trimmed to their lengths) and the counts "ntiles", "nsplit", "nslots"."""
+        if self._split is None:
+            a = self.csr()
+            lib = _abi.load_library()
+            cap = self.S + self.E // _abi.PFS_TILE_EDGES + 2
+            i32 = dict(dtype=torch.int32, device=self.device)
+            b = {"tile_fibre": torch.empty(cap, **i32), "tile_q": torch.empty(cap, **i32),
+                 "tile_slot": torch.empty(cap, **i32), "split_fibre": torch.empty(self.S, **i32),
+                 "split_ptr": torch.empty(self.S + 1, **i32)}
+            counts = torch.zeros(3, **i32)
+            _abi.check(lib.pfs_build_split_tiles(
+                a["csr_rowptr"].data_ptr(), self.S, b["tile_fibre"].data_ptr(), b["tile_q"].data_ptr(),
+                b["tile_slot"].data_ptr(), b["split_fibre"].data_ptr(), b["split_ptr"].data_ptr(), counts.data_ptr(),
+                torch.cuda.current_stream(self.device).cuda_stream), "pfs_build_split_tiles")
+            nt, ns, nslots = (int(v) for v in counts.tolist())
+            for k, n in (("tile_fibre", nt + 1), ("tile_q", nt + 1), ("tile_slot", nt), ("split_fibre", ns),
+                         ("split_ptr", ns + 1)):
+                b[k] = b[k][:n]
+            b.update(ntiles=nt, nsplit=ns, nslots=nslots)
+            self._split = b
+        return self._split
+
     def struct(self, G, F):
         t = _abi.TopologyStruct()
         t.layout = _abi.PFS_LAYOUT_DENSE if self.dense else _abi.PFS_LAYOUT_CSR
         t.G, t.F, t.S, t.T, t.E = int(G), int(F), self.S, self.T, self.E
         if not self.dense:
             a = self.csr()
-            if self.max_degree > _abi.PFS_TILE_EDGES:
-                raise _abi.PfsError("a fibre has %d edges; the fp32 kernels handle at most %d per fibre (the bf16 wide "
-                                    "path has no such limit)" % (self.max_degree, _abi.PFS_TILE_EDGES))
             t.csr_rowptr, t.csr_eid = a["csr_rowptr"].data_ptr(), a["csr_eid"].data_ptr()
             t.csr_src, t.csr_tgt = a["csr_src"].data_ptr(), a["csr_tgt"].data_ptr()
             t.tile_fibre, t.ntiles = a["tile_fibre"].data_ptr(), self.ntiles
             t.csc_colptr, t.csc_q = a["csc_colptr"].data_ptr(), a["csc_q"].data_ptr()
+            if self.max_degree > _abi.PFS_TILE_EDGES:
+                b = self.split_tiles()
+                t.tile_fibre, t.ntiles = b["tile_fibre"].data_ptr(), b["ntiles"]
+                t.tile_q, t.tile_slot = b["tile_q"].data_ptr(), b["tile_slot"].data_ptr()
+                t.split_fibre, t.split_ptr = b["split_fibre"].data_ptr(), b["split_ptr"].data_ptr()
+                t.nsplit, t.nslots = b["nsplit"], b["nslots"]
         return t
 
     def workspace(self, G, F):
