@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define PFS_ABI_VERSION 7
+#define PFS_ABI_VERSION 8
 
 enum {
     PFS_OK = 0,
@@ -394,34 +394,43 @@ int pfs_wide_transpose(const void* in_bf16, int32_t R, int32_t C, int64_t ld, vo
 
 /* -------------------------------------------------------------------------------------------
  * Training loss that consumes the edge times (reference src/train.py:21-80: softfloor + loss_function
- * from `time = gnn.edge_prediction(...)` on; SURVEY.md section 8f row N1).  fp32, one graph, dense
- * canonical edge order e = k*T + i (the reference reshapes the times to [NFIBERS, NCLASSES],
- * src/train.py:67).  `noise` is the uniform [0,1) draw of softfloor (torch.rand_like, src/train.py:22),
- * supplied by the caller so the result is reproducible.
+ * from `time = gnn.edge_prediction(...)` on; SURVEY.md section 8f row N1).  fp32, dense canonical edge
+ * order e = k*T + i (the reference reshapes the times to [NFIBERS, NCLASSES], src/train.py:67).  `noise`
+ * is the uniform [0,1) draw of softfloor (torch.rand_like, src/train.py:22), supplied by the caller so the
+ * result is reproducible.
  *   forward : galaxies = max(0, softfloor(time / T_i)), time2 = galaxies T_i, n'_i, fibre times, and
  *             scalars = {loss, totutils (min completeness), class_penalty, fibre_penalty, variance, #minima}
- *   backward: g_time = dloss/dtime * g_loss (g_loss: device scalar, NULL = 1)
+ *   backward: g_time = dloss/dtime * g_loss (g_loss: device vector [G], NULL = 1)
+ * Graph dimension (ABI 8): G independent graphs of the same S x T in one call; every per-graph array below
+ * gains a leading [G] (G = 0 or 1: one graph, the shapes without it).  S*T < 2^31 per graph; G*S*T may
+ * exceed it.  A forward + backward is 5 launches whatever G is.  Graph g's results depend on graph g's
+ * inputs alone (not on G or on g's position): a batched call is bitwise equal to G single-graph calls.
+ * The batched forward needs G * pfs_loss_workspace_bytes(S, T) bytes of workspace.
  * ---------------------------------------------------------------------------------------- */
 typedef struct pfs_loss_args {
-    int32_t S, T;                                /* fibres, classes */
-    const float* time;                           /* [S*T] */
-    const float* noise;                          /* [S*T] uniform [0,1) */
-    const float* hours;                          /* [T] T_i = class_info[:,0] */
-    const float* counts;                         /* [T] N_i = class_info[:,1] / NFIELDS */
+    int32_t S, T;                                /* fibres, classes (per graph) */
+    const float* time;                           /* [G, S*T] */
+    const float* noise;                          /* [G, S*T] uniform [0,1) */
+    const float* hours;                          /* [T] or [G, T] (class_tables): T_i = class_info[:,0] */
+    const float* counts;                         /* [T] or [G, T] (class_tables): N_i = class_info[:,1] / NFIELDS */
     float total_time, wutils, wvar, pclass, pfiber, sharpness, noiselevel;   /* src/config.py:19,27-28; train.py:21,29 */
-    float* galaxies;                             /* [S*T] */
-    float* time2;                                /* [S*T] galaxies * T_i (the `time` of finaloutput) */
-    float* fibre_time;                           /* [S] */
-    float* n_prime;                              /* [T] */
-    float* class_mean;                           /* [T] mean over fibres of time2 */
-    float* class_coef;                           /* [T] dloss/dn'_i */
-    float* scalars;                              /* [8] */
-    const float* g_loss;                         /* backward: device scalar or NULL */
-    float* g_time;                               /* backward: [S*T] */
-    void* workspace; size_t workspace_bytes;     /* pfs_loss_workspace_bytes(S, T) */
+    float* galaxies;                             /* [G, S*T] */
+    float* time2;                                /* [G, S*T] galaxies * T_i (the `time` of finaloutput) */
+    float* fibre_time;                           /* [G, S] */
+    float* n_prime;                              /* [G, T] */
+    float* class_mean;                           /* [G, T] mean over fibres of time2 */
+    float* class_coef;                           /* [G, T] dloss/dn'_i */
+    float* scalars;                              /* [G, 8] */
+    const float* g_loss;                         /* backward: device vector [G] (upstream gradient of each graph's loss)
+                                                    or NULL (1 for every graph) */
+    float* g_time;                               /* backward: [G, S*T] */
+    void* workspace; size_t workspace_bytes;     /* forward: G * pfs_loss_workspace_bytes(S, T) */
     void* stream;
     const float* sharpness_dev;                  /* optional device scalar overriding `sharpness` (a sharpness schedule
                                                     under CUDA-graph replay, src/train.py:139) */
+    int32_t G;                                   /* ABI 8: graphs in the batch; 0 or 1 = one graph */
+    int32_t class_tables;                        /* ABI 8: 0 = hours / counts are one [T] table shared by every graph,
+                                                    1 = one [G, T] table per graph */
 } pfs_loss_args;
 size_t pfs_sizeof_loss_args(void);
 size_t pfs_loss_workspace_bytes(int32_t S, int32_t T);

@@ -18,7 +18,7 @@ HEADER = os.path.join(os.path.dirname(_HERE), "include", "pfs_b200.h")
 PFS_LAYOUT_DENSE = 0
 PFS_LAYOUT_CSR = 1
 PFS_TILE_EDGES = 256
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 _P = ct.c_void_p
 
@@ -128,7 +128,8 @@ class LossArgs(ct.Structure):
     _fields_ = [("S", ct.c_int32), ("T", ct.c_int32), ("time", _P), ("noise", _P), ("hours", _P), ("counts", _P)] + \
         [(n, ct.c_float) for n in "total_time wutils wvar pclass pfiber sharpness noiselevel".split()] + \
         [(n, _P) for n in "galaxies time2 fibre_time n_prime class_mean class_coef scalars g_loss g_time workspace".split()] + \
-        [("workspace_bytes", ct.c_size_t), ("stream", _P), ("sharpness_dev", _P)]
+        [("workspace_bytes", ct.c_size_t), ("stream", _P), ("sharpness_dev", _P)] + \
+        [("G", ct.c_int32), ("class_tables", ct.c_int32)]          # ABI 8: graph dimension
 
 
 class WideSegments(ct.Structure):

@@ -3,6 +3,11 @@
 // gradient w.r.t. the edge times, as five small kernels instead of ~45 ATen ops and two torch_scatter
 // calls.  fp32, dense canonical edge order (the reference reshapes the times to [NFIBERS, NCLASSES],
 // src/train.py:67), deterministic: every reduction has a fixed order.
+//
+// A leading graph dimension G batches independent graphs of the same S x T: graph g's rows start at g*S*T (edges),
+// g*S (fibres), g*T (classes).  Every graph is reduced by the same code in the same order as a single-graph call
+// (the row-block count depends on S alone), so graph g's results are bitwise those of a call on graph g by itself,
+// and the launch count does not depend on G.
 #include <cstdarg>
 #include <cstdio>
 #include <math_constants.h>
@@ -39,7 +44,8 @@ int lfail(int code, const char* fmt, ...) {
     } while (0)
 
 struct LossConst {
-    int S, T;
+    int S, T, G;
+    int class_stride;     // T: hours / counts are [G, T] tables; 0: one [T] table shared by every graph
     float total_time, wutils, wvar, pclass, pfiber, noiselevel;
     float r, atan_r;      // r = exp(-1 / sharpness) (0 when sharpness == 0), atan(r / (1 - r))
     const float* sharp_dev;   // optional device scalar overriding the sharpness (CUDA-graph replays with a schedule)
@@ -62,14 +68,29 @@ __device__ __forceinline__ void softfloor_eval(float visited, float u, const Los
     dsf = 1.f + 2.f * c.r * (cs - c.r) / (1.f - 2.f * c.r * cs + c.r * c.r);
 }
 
+// edge e of the batch = row `row` (= g*S + k, the fibre over all graphs) and class i; g is only divided out when
+// there is more than one graph
+struct EdgeAt {
+    long long row;
+    int i, g;
+};
+__device__ __forceinline__ EdgeAt edge_at(long long e, const LossConst& c) {
+    EdgeAt a;
+    a.row = e / c.T;
+    a.i = (int)(e - a.row * c.T);
+    a.g = c.G > 1 ? (int)(a.row / c.S) : 0;
+    return a;
+}
+
 // per edge: galaxies = max(0, softfloor(time / T_i)), time2 = galaxies * T_i      (src/train.py:43-49)
 __global__ void __launch_bounds__(256) k_loss_edge_fwd(LossConst c, const float* __restrict__ time,
                                                        const float* __restrict__ noise, const float* __restrict__ hours,
                                                        float* __restrict__ galaxies, float* __restrict__ time2) {
     resolve_sharpness(c);
-    const long long E = (long long)c.S * c.T;
+    const long long E = (long long)c.G * c.S * c.T;
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < E; e += (long long)gridDim.x * blockDim.x) {
-        const float h = hours[e % c.T];
+        const EdgeAt a = edge_at(e, c);
+        const float h = hours[(size_t)a.g * c.class_stride + a.i];
         float sf, dsf;
         softfloor_eval(time[e] / h, noise[e], c, sf, dsf);
         const float g = fmaxf(sf, 0.f);
@@ -78,10 +99,12 @@ __global__ void __launch_bounds__(256) k_loss_edge_fwd(LossConst c, const float*
     }
 }
 
-// fibre sums of time2 (src/train.py:61): one warp per fibre
-__global__ void __launch_bounds__(256) k_loss_fibre_sums(int S, int T, const float* __restrict__ time2, float* __restrict__ fibre_time) {
-    const int k = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (k >= S) return;
+// fibre sums of time2 (src/train.py:61): one warp per fibre, GS = G*S fibres over all graphs
+__global__ void __launch_bounds__(256) k_loss_fibre_sums(long long GS, int T, const float* __restrict__ time2,
+                                                         float* __restrict__ fibre_time) {
+    const long long k = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (k >= GS) return;
     float s = 0.f;
     for (int i = lane; i < T; i += 32) s += time2[(size_t)k * T + i];
 #pragma unroll
@@ -90,15 +113,20 @@ __global__ void __launch_bounds__(256) k_loss_fibre_sums(int S, int T, const flo
 }
 
 // class statistics over the fibres: partial[rb][0][i] = sum galaxies, [1] = sum (time2 - shift_i), [2] = sum (time2 - shift_i)^2,
-// shift_i = time2 of fibre 0 (shifted sums do not cancel).  grid = row blocks, 256 threads = (row lane, class)
-__global__ void __launch_bounds__(256) k_loss_class_partial(int S, int T, const float* __restrict__ galaxies,
+// shift_i = time2 of fibre 0 (shifted sums do not cancel).  grid = nrb row blocks x G graphs, flattened into x
+// (block = g * nrb + row block, so any G fits the grid), 256 threads = (row lane, class); partial is [G][nrb][3][T]
+__global__ void __launch_bounds__(256) k_loss_class_partial(int S, int T, int nrb, const float* __restrict__ galaxies,
                                                             const float* __restrict__ time2, int rows_per_block,
                                                             float* __restrict__ partial) {
     __shared__ float red[3][256];
+    const int g = blockIdx.x / nrb, rb = blockIdx.x - g * nrb;
+    galaxies += (size_t)g * S * T;
+    time2 += (size_t)g * S * T;
+    partial += (size_t)g * nrb * 3 * T;
     const int tc = T < 256 ? T : 256;
     const int lanes = 256 / tc;
     const int lr = threadIdx.x / tc, lc = threadIdx.x - lr * tc;
-    const int r0 = blockIdx.x * rows_per_block, r1 = min(S, r0 + rows_per_block);
+    const int r0 = rb * rows_per_block, r1 = min(S, r0 + rows_per_block);
     for (int c0 = 0; c0 < T; c0 += tc) {
         const int i = c0 + lc;
         float a = 0.f, b = 0.f, q = 0.f;
@@ -120,7 +148,7 @@ __global__ void __launch_bounds__(256) k_loss_class_partial(int S, int T, const 
             for (int r = 0; r < lanes; ++r) {
                 s0 += red[0][r * tc + lc]; s1 += red[1][r * tc + lc]; s2 += red[2][r * tc + lc];
             }
-            float* o = partial + (size_t)blockIdx.x * 3 * T;
+            float* o = partial + (size_t)rb * 3 * T;
             o[i] = s0; o[T + i] = s1; o[2 * T + i] = s2;
         }
     }
@@ -138,8 +166,8 @@ __device__ __forceinline__ double block_sum(double v, double* red) {     // fixe
     return r;
 }
 
-// one CTA: class totals, completeness and its minimum, penalties, variance, loss (src/train.py:51-71) and the per-class
-// gradient coefficient dL/dn'_i.  scalars = {loss, totutils, class_penalty, fibre_penalty, variance, #minima}
+// one CTA per graph: class totals, completeness and its minimum, penalties, variance, loss (src/train.py:51-71) and the
+// per-class gradient coefficient dL/dn'_i.  scalars = {loss, totutils, class_penalty, fibre_penalty, variance, #minima}
 __global__ void __launch_bounds__(1024) k_loss_scalars(const LossConst c, const float* __restrict__ partial, int nrb,
                                                        const float* __restrict__ counts, const float* __restrict__ time2,
                                                        const float* __restrict__ fibre_time, float* __restrict__ n_prime,
@@ -148,11 +176,21 @@ __global__ void __launch_bounds__(1024) k_loss_scalars(const LossConst c, const 
     __shared__ double red[1024];
     __shared__ float s_min;
     const int S = c.S, T = c.T;
+    // graph blockIdx.x's rows (its row blocks of `partial` are indexed from the global row-block number: a pointer
+    // offset there makes the unrolled loop spill at the 64 registers of a 1024-thread CTA)
+    const size_t g = blockIdx.x;
+    counts += g * c.class_stride;
+    time2 += g * S * T;
+    fibre_time += g * S;
+    n_prime += g * T;
+    class_mean += g * T;
+    class_coef += g * T;
+    scalars += g * 8;
     double var_sum = 0.0, cpen = 0.0;
     float my_min = CUDART_INF_F;
     for (int i = threadIdx.x; i < T; i += blockDim.x) {
         double s0 = 0.0, s1 = 0.0, s2 = 0.0;
-        for (int b = 0; b < nrb; ++b) {
+        for (int b = blockIdx.x * nrb; b < (blockIdx.x + 1) * nrb; ++b) {
             s0 += partial[(size_t)b * 3 * T + i];
             s1 += partial[(size_t)b * 3 * T + T + i];
             s2 += partial[(size_t)b * 3 * T + 2 * T + i];
@@ -206,28 +244,28 @@ __global__ void __launch_bounds__(1024) k_loss_scalars(const LossConst c, const 
     }
 }
 
-// g_time[e] = gL * [softfloor > 0] * softfloor' / T_i * (dL/dn'_i + T_i * (dL/dfibre_time_k - 2 wvar (time2 - mean_i) / (S - 1)))
+// g_time[e] = gL_g * [softfloor > 0] * softfloor' / T_i * (dL/dn'_i + T_i * (dL/dfibre_time_k - 2 wvar (time2 - mean_i) / (S - 1)))
 __global__ void __launch_bounds__(256) k_loss_edge_bwd(LossConst c, const float* __restrict__ time,
                                                        const float* __restrict__ noise, const float* __restrict__ hours,
                                                        const float* __restrict__ time2, const float* __restrict__ fibre_time,
                                                        const float* __restrict__ class_mean, const float* __restrict__ class_coef,
                                                        const float* __restrict__ g_loss, float* __restrict__ g_time) {
     resolve_sharpness(c);
-    const long long E = (long long)c.S * c.T;
-    const float gl = g_loss ? g_loss[0] : 1.f;
+    const long long E = (long long)c.G * c.S * c.T;
     const float vscale = 2.f * c.wvar / (float)(c.S - 1);
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < E; e += (long long)gridDim.x * blockDim.x) {
-        const int i = (int)(e % c.T);
-        const long long k = e / c.T;
-        const float h = hours[i];
+        const EdgeAt a = edge_at(e, c);
+        const size_t ci = (size_t)a.g * c.T + a.i;
+        const float h = hours[(size_t)a.g * c.class_stride + a.i];
         float sf, dsf;
         softfloor_eval(time[e] / h, noise[e], c, sf, dsf);
         float g = 0.f;
         if (sf > 0.f) {
-            const float ot = fibre_time[k] - c.total_time;
+            const float gl = g_loss ? g_loss[a.g] : 1.f;
+            const float ot = fibre_time[a.row] - c.total_time;
             const float dft = 2.f * c.pfiber * (ot > 0.f ? ot : 0.01f * ot);      // d/d ot of lrelu_0.1(ot)^2
-            const float d_t2 = dft - vscale * (time2[e] - class_mean[i]);
-            g = gl * (class_coef[i] + h * d_t2) * dsf / h;
+            const float d_t2 = dft - vscale * (time2[e] - class_mean[ci]);
+            g = gl * (class_coef[ci] + h * d_t2) * dsf / h;
         }
         g_time[e] = g;
     }
@@ -235,7 +273,11 @@ __global__ void __launch_bounds__(256) k_loss_edge_bwd(LossConst c, const float*
 
 int make_const(const pfs_loss_args& a, LossConst& c) {
     L_REQUIRE(a.S >= 2 && a.T >= 1 && (long long)a.S * a.T < (1ll << 31), "loss: bad graph sizes (at least 2 fibres)");
+    L_REQUIRE(a.G >= 0, "loss: negative graph count");
+    L_REQUIRE(a.class_tables == 0 || a.class_tables == 1, "loss: class_tables is 0 (one [T] table) or 1 ([G, T])");
     c.S = a.S; c.T = a.T;
+    c.G = a.G > 1 ? a.G : 1;
+    c.class_stride = a.class_tables ? a.T : 0;
     c.total_time = a.total_time; c.wutils = a.wutils; c.wvar = a.wvar; c.pclass = a.pclass; c.pfiber = a.pfiber;
     c.noiselevel = a.noiselevel;
     c.r = a.sharpness == 0.f ? 0.f : expf(-1.f / a.sharpness);
@@ -269,18 +311,20 @@ int pfs_loss_fwd(const pfs_loss_args* a) {
     cudaStream_t st = (cudaStream_t)a->stream;
     pfs_host::mark_launch(nullptr, st);
     const int nrb = class_row_blocks(c.S);
-    if (a->workspace_bytes < (size_t)nrb * 3 * c.T * sizeof(float)) return lfail(PFS_ERR_WORKSPACE, "loss: workspace too small");
+    L_REQUIRE((long long)nrb * c.G < (1ll << 31), "loss: too many graphs for one launch");
+    if (a->workspace_bytes < (size_t)c.G * nrb * 3 * c.T * sizeof(float))
+        return lfail(PFS_ERR_WORKSPACE, "loss: workspace too small (%zu bytes for %d graph(s))", a->workspace_bytes, c.G);
     float* partial = (float*)(((uintptr_t)a->workspace + 255) & ~(uintptr_t)255);
-    const long long E = (long long)c.S * c.T;
-    k_loss_edge_fwd<<<edge_grid(E), 256, 0, st>>>(c, a->time, a->noise, a->hours, a->galaxies, a->time2);
+    const long long GS = (long long)c.G * c.S;
+    k_loss_edge_fwd<<<edge_grid(GS * c.T), 256, 0, st>>>(c, a->time, a->noise, a->hours, a->galaxies, a->time2);
     L_LAUNCH_CHECK("k_loss_edge_fwd");
-    k_loss_fibre_sums<<<(c.S * 32 + 255) / 256, 256, 0, st>>>(c.S, c.T, a->time2, a->fibre_time);
+    k_loss_fibre_sums<<<(unsigned)((GS * 32 + 255) / 256), 256, 0, st>>>(GS, c.T, a->time2, a->fibre_time);
     L_LAUNCH_CHECK("k_loss_fibre_sums");
     const int rpb = (c.S + nrb - 1) / nrb;
-    k_loss_class_partial<<<nrb, 256, 0, st>>>(c.S, c.T, a->galaxies, a->time2, rpb, partial);
+    k_loss_class_partial<<<nrb * c.G, 256, 0, st>>>(c.S, c.T, nrb, a->galaxies, a->time2, rpb, partial);
     L_LAUNCH_CHECK("k_loss_class_partial");
-    k_loss_scalars<<<1, 1024, 0, st>>>(c, partial, nrb, a->counts, a->time2, a->fibre_time, a->n_prime, a->class_mean,
-                                       a->class_coef, a->scalars);
+    k_loss_scalars<<<c.G, 1024, 0, st>>>(c, partial, nrb, a->counts, a->time2, a->fibre_time, a->n_prime, a->class_mean,
+                                         a->class_coef, a->scalars);
     L_LAUNCH_CHECK("k_loss_scalars");
     return PFS_OK;
 }
@@ -292,7 +336,7 @@ int pfs_loss_bwd(const pfs_loss_args* a) {
     if (int rc = make_const(*a, c)) return rc;
     cudaStream_t st = (cudaStream_t)a->stream;
     pfs_host::mark_launch(nullptr, st);
-    k_loss_edge_bwd<<<edge_grid((long long)c.S * c.T), 256, 0, st>>>(c, a->time, a->noise, a->hours, a->time2, a->fibre_time,
+    k_loss_edge_bwd<<<edge_grid((long long)c.G * c.S * c.T), 256, 0, st>>>(c, a->time, a->noise, a->hours, a->time2, a->fibre_time,
                                                                     a->class_mean, a->class_coef, a->g_loss, a->g_time);
     L_LAUNCH_CHECK("k_loss_edge_bwd");
     return PFS_OK;

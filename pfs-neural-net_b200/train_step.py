@@ -12,6 +12,12 @@ The warm-up and capture passes execute real steps; everything they touch -- para
 statistics AND num_batches_tracked), Adam moments and step counters, the CUDA generator -- is snapshotted before and
 restored afterwards IN PLACE (the captured graph keeps the addresses), so the first user-visible step starts from the
 state the caller handed in, like reference src/train.py:133 or a resumed checkpoint (:126-132).
+
+The graph may be a collated batch of G graphs that share one `edge_index` (`Loader.collate`, x_e [G, E, F]) with a
+class table [T, 2] for all of them or [G, T, 2]: the step then trains on the sum of the G per-graph losses (the
+parameter gradients of the G graphs stepped one after the other, summed) and returns the G utilities.  `load()`
+copies the next batch of the same shapes and topology into the step's input tensors, so an epoch over
+`Loader.batches(G)` replays the one captured graph.
 """
 import torch
 
@@ -21,8 +27,10 @@ from . import loss as _loss
 class TrainStep:
     def __init__(self, model, graph, class_info, optimizer, *, pclass=0.1, pfiber=1.0, nfields=10, total_time=42,
                  wutils=2000.0, wvar=1.0, use_graph=True, warmup=3, noise=None):
-        """`noise`: optional static device tensor [E] of softfloor draws in [0, 1) (reference src/train.py:22); the caller
-        refills it (copy_) before a step to control the draw.  None: torch.rand_like per step, as the reference."""
+        """`noise`: optional static device tensor [E] (a batch: [G, E]) of softfloor draws in [0, 1) (reference
+        src/train.py:22); the caller refills it (copy_) before a step to control the draw.  None: torch.rand_like per
+        step, as the reference.  The tensors of `graph` and `class_info` are the step's static inputs: `load()`
+        overwrites them in place."""
         self.model, self.graph, self.class_info, self.opt = model, graph, class_info, optimizer
         self.kw = dict(pclass=pclass, pfiber=pfiber, nfields=nfields, total_time=total_time, wutils=wutils, wvar=wvar)
         dev = class_info.device
@@ -77,8 +85,29 @@ class TrainStep:
         self.loss.backward()
         self.opt.step()
 
+    def load(self, batch, class_info=None):
+        """Copies the node, edge and global features of `batch` (and `class_info`, if given) into the step's input
+        tensors in place, for the next call.  The batch must have the shapes of the step's graph and its `edge_index`:
+        the captured kernels hold that topology.  A batch of another size (the short last batch of `Loader.batches`)
+        needs a step of its own."""
+        mine = self.graph
+        ei = batch.edge_index
+        if ei is not mine.edge_index and (ei.shape != mine.edge_index.shape or not torch.equal(ei, mine.edge_index.to(ei.device))):
+            raise ValueError("TrainStep.load: the batch's edge_index differs from the one the step was built on")
+        pairs = [(getattr(mine, k), getattr(batch, k), k) for k in ("x_s", "x_t", "x_e", "x_u")]
+        if class_info is not None:
+            pairs.append((self.class_info, class_info, "class_info"))
+        for dst, src, k in pairs:
+            if src.shape != dst.shape:
+                raise ValueError("TrainStep.load: %s is %s, the step was built for %s" % (k, tuple(src.shape), tuple(dst.shape)))
+        with torch.no_grad():
+            for dst, src, _ in pairs:
+                if src is not dst:
+                    dst.copy_(src)
+
     def __call__(self, sharpness):
-        """Runs one step at this sharpness; returns (loss, utility) as device scalars (no host synchronisation)."""
+        """Runs one step at this sharpness; returns (loss, utility) as device tensors (no host synchronisation): scalars,
+        or for a batch the summed loss and the utilities [G]."""
         self.sharp.fill_(float(sharpness))
         if self._graph is not None:
             self._graph.replay()
