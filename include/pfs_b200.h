@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define PFS_ABI_VERSION 8
+#define PFS_ABI_VERSION 9
 
 enum {
     PFS_OK = 0,
@@ -406,6 +406,17 @@ int pfs_wide_transpose(const void* in_bf16, int32_t R, int32_t C, int64_t ld, vo
  * exceed it.  A forward + backward is 5 launches whatever G is.  Graph g's results depend on graph g's
  * inputs alone (not on G or on g's position): a batched call is bitwise equal to G single-graph calls.
  * The batched forward needs G * pfs_loss_workspace_bytes(S, T) bytes of workspace.
+ * Fibre-sharded graph (ABI 9): one graph whose fibres are split over `world` ranks, each calling with its own
+ * contiguous fibre range (S local fibres, S_total over all ranks, one graph per call).  The forward is
+ *   1. pfs_loss_shard_fwd: the per-edge and per-fibre outputs of the local fibres and this rank's record
+ *      shard_record [2 + 3T] doubles = {n_r, local fibre-penalty sum, per class: sum galaxies [T], mean [T] and
+ *      M2 [T] of time2 over the local fibres} (4 launches);
+ *   2. the caller makes every rank's record visible to every rank as shard_records [world][2 + 3T], rank order;
+ *   3. pfs_loss_shard_merge: n_prime, class_mean, class_coef and scalars of the whole graph (1 launch).  The records
+ *      are combined in rank order, so every rank gets bitwise the same results; with world = 1 they are bitwise those
+ *      of pfs_loss_fwd.
+ * pfs_loss_bwd with S_total set takes the variance over S_total fibres; time, noise, time2, fibre_time and g_time are
+ * the local rows, class_mean and class_coef the merged ones.
  * ---------------------------------------------------------------------------------------- */
 typedef struct pfs_loss_args {
     int32_t S, T;                                /* fibres, classes (per graph) */
@@ -431,11 +442,18 @@ typedef struct pfs_loss_args {
     int32_t G;                                   /* ABI 8: graphs in the batch; 0 or 1 = one graph */
     int32_t class_tables;                        /* ABI 8: 0 = hours / counts are one [T] table shared by every graph,
                                                     1 = one [G, T] table per graph */
+    int32_t S_total;                             /* ABI 9: fibres over all shards; 0 = not sharded (the ABI 8 behaviour).
+                                                    With S_total set, S >= 1, S_total >= 2 and G is 0 or 1 */
+    int32_t world;                               /* ABI 9: ranks of the sharded graph (pfs_loss_shard_merge) */
+    double* shard_record;                        /* ABI 9: pfs_loss_shard_fwd output, [2 + 3T] */
+    const double* shard_records;                 /* ABI 9: pfs_loss_shard_merge input, [world][2 + 3T] in rank order */
 } pfs_loss_args;
 size_t pfs_sizeof_loss_args(void);
 size_t pfs_loss_workspace_bytes(int32_t S, int32_t T);
 int pfs_loss_fwd(const pfs_loss_args* a);
 int pfs_loss_bwd(const pfs_loss_args* a);
+int pfs_loss_shard_fwd(const pfs_loss_args* a);
+int pfs_loss_shard_merge(const pfs_loss_args* a);
 
 #ifdef __cplusplus
 }

@@ -18,7 +18,7 @@ HEADER = os.path.join(os.path.dirname(_HERE), "include", "pfs_b200.h")
 PFS_LAYOUT_DENSE = 0
 PFS_LAYOUT_CSR = 1
 PFS_TILE_EDGES = 256
-ABI_VERSION = 8
+ABI_VERSION = 9
 
 _P = ct.c_void_p
 
@@ -129,7 +129,9 @@ class LossArgs(ct.Structure):
         [(n, ct.c_float) for n in "total_time wutils wvar pclass pfiber sharpness noiselevel".split()] + \
         [(n, _P) for n in "galaxies time2 fibre_time n_prime class_mean class_coef scalars g_loss g_time workspace".split()] + \
         [("workspace_bytes", ct.c_size_t), ("stream", _P), ("sharpness_dev", _P)] + \
-        [("G", ct.c_int32), ("class_tables", ct.c_int32)]          # ABI 8: graph dimension
+        [("G", ct.c_int32), ("class_tables", ct.c_int32)] + \
+        [("S_total", ct.c_int32), ("world", ct.c_int32), ("shard_record", _P), ("shard_records", _P)]
+# ABI 8 appended the graph dimension (G, class_tables), ABI 9 the fibre-sharded graph (S_total ... shard_records)
 
 
 class WideSegments(ct.Structure):
@@ -193,6 +195,8 @@ SYMBOLS = {
     "pfs_loss_workspace_bytes": (ct.c_size_t, [_I32, _I32]),
     "pfs_loss_fwd": (ct.c_int, [ct.POINTER(LossArgs)]),
     "pfs_loss_bwd": (ct.c_int, [ct.POINTER(LossArgs)]),
+    "pfs_loss_shard_fwd": (ct.c_int, [ct.POINTER(LossArgs)]),
+    "pfs_loss_shard_merge": (ct.c_int, [ct.POINTER(LossArgs)]),
     "pfs_wide_transpose": (ct.c_int, [_P, _I32, _I32, _I64, _P, _P]),
 }
 _SIZEOF_CHECKS = {

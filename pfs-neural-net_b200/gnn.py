@@ -16,7 +16,9 @@ step) and parameter gradients are summed over the graphs.
 import torch
 import torch.nn.functional as Fn
 
+from . import _abi
 from . import functional as pf
+from . import shard as _shard
 from . import wide as pw
 from .topology import get_topology
 
@@ -132,6 +134,37 @@ def _wide_args(x_s, x_t, edge_attr, u):
     return x_s, x_t, edge_attr, u.reshape(1, -1)
 
 
+def _refuse_sharded_narrow(what):
+    """The fp32 kernels reduce over the fibres of the call only: inside a fibre-sharding scope they would return per-shard
+    BatchNorm statistics and class sums."""
+    if _shard.active():
+        raise _abi.PfsError("%s: a fibre-sharded graph runs on the bf16 wide path (Fdim >= 32, bf16 tensors); the fp32 "
+                            "kernels are not sharded" % what)
+
+
+class _SumGradsOverShards(torch.autograd.Function):
+    """Identity on a module's parameters whose backward sums their gradients over the fibre shards in ONE all-reduce:
+    the parameters of a fibre-local module (encoder_s, decoder_s) see only the rank's own fibres."""
+
+    @staticmethod
+    def forward(ctx, *params):
+        return tuple(p.view_as(p) for p in params)
+
+    @staticmethod
+    def backward(ctx, *grads):
+        return tuple(_shard.allreduce_packed(list(grads)))
+
+
+def _fibre_local(module, x):
+    """module(x) for a module applied to the rank's own fibres; inside an active fibre-sharding scope its parameter
+    gradients are summed over the shards, so every rank's .grad is the global gradient."""
+    if not _shard.active():
+        return module(x)
+    names, params = zip(*module.named_parameters())
+    routed = _SumGradsOverShards.apply(*params)
+    return torch.func.functional_call(module, dict(zip(names, routed)), (x,))
+
+
 def _norm_tensors(mod):
     norm = mod.norm if isinstance(mod.norm, torch.nn.Module) else None
     if norm is None:
@@ -157,6 +190,7 @@ class EdgeModel(MLP):
             normed, gamma, beta, rm, rv, nbt = _norm_tensors(self)
             return pw.WideEdgeFunction.apply(topo, self.training, normed, *wide, self[0].weight, self[0].bias,
                                              self[2].weight, self[2].bias, gamma, beta, rm, rv, nbt)
+        _refuse_sharded_narrow("EdgeModel (fp32)")
         single, x_s, x_t, edge_attr, u = _batched(x_s, x_t, edge_attr, u)
         topo = get_topology(edge_index, x_s.shape[1], x_t.shape[1])
         normed, gamma, beta, rm, rv, nbt = _norm_tensors(self)
@@ -184,6 +218,7 @@ class SModel(torch.nn.Module):
             m1, m2 = self.node_mlp_1, self.node_mlp_2
             return pw.WideSourceFunction.apply(topo, self.training, normed, *wide, m1[0].weight, m1[0].bias, m1[2].weight,
                                m1[2].bias, m2[0].weight, m2[0].bias, m2[2].weight, m2[2].bias, gamma, beta, rm, rv, nbt)
+        _refuse_sharded_narrow("SModel (fp32)")
         single, x_s, x_t, edge_attr, u = _batched(x_s, x_t, edge_attr, u)
         topo = get_topology(edge_index, x_s.shape[1], x_t.shape[1])
         normed, gamma, beta, rm, rv, nbt = _norm_tensors(self)
@@ -214,6 +249,7 @@ class TModel(torch.nn.Module):
             m1, m2 = self.node_mlp_1, self.node_mlp_2
             return pw.WideTargetFunction.apply(topo, self.training, normed, *wide, m1[0].weight, m1[0].bias, m1[2].weight,
                                m1[2].bias, m2[0].weight, m2[0].bias, m2[2].weight, m2[2].bias, gamma, beta, rm, rv, nbt)
+        _refuse_sharded_narrow("TModel (fp32)")
         single, x_s, x_t, edge_attr, u = _batched(x_s, x_t, edge_attr, u)
         topo = get_topology(edge_index, x_s.shape[1], x_t.shape[1])
         normed, gamma, beta, rm, rv, nbt = _norm_tensors(self)
@@ -242,6 +278,7 @@ class GlobalModel(MLP):
             return pw.WideGlobalFunction.apply(normed, x_s, x_t, u, self[0].weight, self[0].bias, self[2].weight,
                                                self[2].bias, self.norm.weight if normed else None,
                                                float(torch.finfo(u.dtype).eps))
+        _refuse_sharded_narrow("GlobalModel (fp32)")
         single = x_s.dim() == 2
         if single:
             x_s, x_t = x_s.unsqueeze(0), x_t.unsqueeze(0)
@@ -331,8 +368,9 @@ class GNN(torch.nn.Module):
     def forward(self, graph):
         x_s, x_t = graph.x_s, graph.x_t
         edge_index, x_e, x_u = graph.edge_index, graph.x_e, graph.x_u
-        # per-node encoders stay in PyTorch (SURVEY.md section 2 row 2)
-        x_s = self.encoder_s(x_s)
+        # per-node encoders stay in PyTorch (SURVEY.md section 2 row 2).  Fibre-sharded, encoder_s sees the local fibres
+        # and its gradients are summed over the shards; encoder_t's already are global (replicated classes, global g_x_t)
+        x_s = _fibre_local(self.encoder_s, x_s)
         x_t = self.encoder_t(x_t)
         _, x_s, x_t, x_e, x_u = self.mpb((edge_index, x_s, x_t, x_e, x_u))
         self._last_edge_index = edge_index
@@ -365,6 +403,7 @@ class GNN(torch.nn.Module):
             if x_e.dim() != 2:
                 raise RuntimeError("the bf16 wide path takes one graph per call (2-D tensors)")
             return pw.WideTimeHeadFunction.apply(scale, x_e, d[0].weight, d[0].bias, d[2].weight, d[2].bias).unsqueeze(-1)
+        _refuse_sharded_narrow("the time head (fp32)")
         single = x_e.dim() == 2
         xe3 = x_e.unsqueeze(0) if single else x_e
         topo = _FlatTopology(xe3.shape[1], x_e.device)
@@ -389,7 +428,7 @@ class GNN(torch.nn.Module):
         return tuple(o[0] for o in out) if single else out
 
     def node_prediction(self, x_s, scale=1):
-        pred = self.decoder_s(x_s)
+        pred = _fibre_local(self.decoder_s, x_s)
         time = torch.softmax(pred, dim=-1) * scale
         return self.round(time)
 
@@ -407,7 +446,6 @@ class _FlatTopology:
         self._ws = None
 
     def struct(self, G, F):
-        from . import _abi
         t = _abi.TopologyStruct()
         t.layout, t.G, t.F, t.S, t.T, t.E = _abi.PFS_LAYOUT_DENSE, int(G), int(F), self.S, 1, self.E
         return t

@@ -13,12 +13,19 @@ Both functions also take a batch of G graphs that share one `edge_index` (the le
 `Loader.collate`): edge times [G, E], one class table [T, 2] for all graphs or one per graph [G, T, 2].  Each
 graph gets its own loss, computed exactly as a call on that graph alone would compute it (bitwise), in the same
 five kernel launches whatever G is.
+
+Inside `shard.fibre_sharded()` (one graph whose fibres are split over the ranks, DESIGN.md section 7) both functions
+compute the loss of the WHOLE graph on every rank from the rank's own fibres: each rank reduces its fibres to a record
+of 2 + 3T doubles, one all-reduce makes every record visible to every rank, and a merge in rank order gives every rank
+bitwise the same class statistics, scalars and loss.  The gradient w.r.t. the local edge times is that of the global
+loss, so the Blocks' gradient all-reduces sum the parts of one function.
 """
 import ctypes as ct
 
 import torch
 
 from . import _abi
+from . import shard as _shard
 
 NOISELEVEL = 0.3          # softfloor default (reference src/train.py:21)
 
@@ -27,10 +34,12 @@ class LossFunction(torch.autograd.Function):
     """loss(time): forward = pfs_loss_fwd, backward = pfs_loss_bwd (gradient w.r.t. the edge times only).
 
     G = 0: one graph (time [S*T], hours / counts [T]; the loss is a scalar).  G >= 1: a batch (time [G, S*T], hours /
-    counts [T] shared or [G, T]; the loss is [G] and every other output gains the leading G)."""
+    counts [T] shared or [G, T]; the loss is [G] and every other output gains the leading G).
+    S_total > 0: this rank's S fibres of a graph of S_total fibres sharded over the active group (G = 0): the forward is
+    pfs_loss_shard_fwd, the record exchange (shard.exchange_rows) and pfs_loss_shard_merge."""
 
     @staticmethod
-    def forward(ctx, time, noise, hours, counts, G, S, T, consts):
+    def forward(ctx, time, noise, hours, counts, G, S, T, consts, S_total):
         for t, n in ((time, "time"), (noise, "noise"), (hours, "hours"), (counts, "counts")):
             if not t.is_cuda:
                 raise _abi.PfsError("pfs_b200 loss needs CUDA tensors, %s is on %s (no CPU fallback)" % (n, t.device))
@@ -62,8 +71,16 @@ class LossFunction(torch.autograd.Function):
         a.workspace, a.workspace_bytes = ws.data_ptr(), ws.numel()
         with torch.cuda.device(dev):
             a.stream = torch.cuda.current_stream(dev).cuda_stream
-            _abi.check(lib.pfs_loss_fwd(ct.byref(a)), "pfs_loss_fwd")
-        ctx.G, ctx.S, ctx.T, ctx.consts = G, S, T, dict(consts)
+            if S_total:
+                record = torch.empty(2 + 3 * T, dtype=torch.float64, device=dev)
+                a.S_total, a.world, a.shard_record = S_total, _shard.world_size(), record.data_ptr()
+                _abi.check(lib.pfs_loss_shard_fwd(ct.byref(a)), "pfs_loss_shard_fwd")
+                records = _shard.exchange_rows(record)                  # [world, 2 + 3T], rank order, on every rank
+                a.shard_records = records.data_ptr()
+                _abi.check(lib.pfs_loss_shard_merge(ct.byref(a)), "pfs_loss_shard_merge")
+            else:
+                _abi.check(lib.pfs_loss_fwd(ct.byref(a)), "pfs_loss_fwd")
+        ctx.G, ctx.S, ctx.T, ctx.S_total, ctx.consts = G, S, T, S_total, dict(consts)
         ctx.save_for_backward(time, noise, hours, counts, out["time2"], out["fibre_time"], out["class_mean"], out["class_coef"])
         sc = out["scalars"]
         ctx.mark_non_differentiable(sc, out["n_prime"], out["fibre_time"], out["time2"])
@@ -76,7 +93,7 @@ class LossFunction(torch.autograd.Function):
         g_time = torch.empty_like(time)
         gl = g_loss.detach().to(torch.float32).reshape(-1).contiguous()
         a = _abi.LossArgs()
-        a.S, a.T, a.G, a.class_tables = ctx.S, ctx.T, ctx.G, int(hours.dim() == 2)
+        a.S, a.T, a.G, a.class_tables, a.S_total = ctx.S, ctx.T, ctx.G, int(hours.dim() == 2), ctx.S_total
         for k, v in dict(time=time, noise=noise, hours=hours, counts=counts, time2=time2, fibre_time=fibre_time,
                          class_mean=class_mean, class_coef=class_coef, g_loss=gl, g_time=g_time).items():
             setattr(a, k, v.data_ptr())
@@ -87,7 +104,7 @@ class LossFunction(torch.autograd.Function):
         with torch.cuda.device(dev):
             a.stream = torch.cuda.current_stream(dev).cuda_stream
             _abi.check(_abi.load_library().pfs_loss_bwd(ct.byref(a)), "pfs_loss_bwd")
-        return g_time, None, None, None, None, None, None, None
+        return g_time, None, None, None, None, None, None, None, None
 
 
 def _graph_rows(x, E):
@@ -120,7 +137,7 @@ def _batched_loss(time, class_info, S, T, nfields, consts, noise):
         noise = n
     hours = class_info[..., 0].to(torch.float32)
     counts = (class_info[..., 1] / nfields).to(torch.float32)
-    return LossFunction.apply(t, noise.to(torch.float32), hours, counts, G, S, T, consts)
+    return LossFunction.apply(t, noise.to(torch.float32), hours, counts, G, S, T, consts, 0)
 
 
 def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=42, wutils=2000.0, wvar=1.0, pclass=0.1,
@@ -133,23 +150,39 @@ def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=
     are bitwise those of a single-graph call on time[g] with the same noise.  `noise` has the shape of `time`; when
     it is omitted it is drawn by ONE torch.rand_like over the whole batch, which is not the random stream of G
     separate single-graph calls (those draw E values each, interleaved with whatever else uses the generator):
-    pass `noise` to reproduce them."""
+    pass `noise` to reproduce them.
+
+    Inside `shard.fibre_sharded()`: `time` holds this rank's `nfibers` fibres (a contiguous fibre range, canonical order)
+    of one graph; the loss, scalars and n_prime are those of the whole graph (bitwise the same on every rank),
+    fibre_time and time2 the local rows.  Without `noise` the whole graph's S_total * T draws are made by one
+    torch.rand and this rank takes its slice [f0 * T, f1 * T), so a run seeded alike on every rank draws bitwise the
+    noise of the single-GPU run and no two shards share draws.  A batch of graphs is refused."""
     consts = dict(total_time=total_time, wutils=wutils, wvar=wvar, pclass=pclass, pfiber=pfiber, noiselevel=NOISELEVEL)
     if torch.is_tensor(sharpness):                # device scalar: the value is read by the kernels (CUDA-graph replays)
         consts.update(sharpness=0.0, sharpness_dev=sharpness.to(torch.float32).reshape(1))
     else:
         consts.update(sharpness=sharpness)
     nfibers, nclasses = int(nfibers), int(nclasses)
+    sharded = _shard.active()
     if time.dim() == 3 or (time.dim() == 2 and time.shape[1] == nfibers * nclasses):
+        if sharded:
+            raise _abi.PfsError("loss: a fibre-sharded graph is one graph per call, not a batch of %d" % time.shape[0])
         return _batched_loss(time, class_info, nfibers, nclasses, nfields, consts, noise)
     time = time.reshape(-1)
     if time.dtype != torch.float32:
         time = time.float()                       # bf16 head output: dtype plumbing, the loss itself is fp32
+    S_total = _shard.total_count(nfibers) if sharded else 0      # cached: no host synchronisation per step
     if noise is None:
-        noise = torch.rand_like(time)             # the draw of softfloor, reference src/train.py:22
+        if sharded:                               # the whole graph's draw, this rank's slice
+            f0 = sum(_shard.shard_counts(nfibers)[:_shard.rank()])       # cached like S_total
+            noise = torch.rand(S_total * nclasses, dtype=torch.float32, device=time.device)
+            noise = noise[f0 * nclasses:(f0 + nfibers) * nclasses]
+        else:
+            noise = torch.rand_like(time)         # the draw of softfloor, reference src/train.py:22
     hours = class_info[:, 0].to(torch.float32)
     counts = (class_info[:, 1] / nfields).to(torch.float32)
-    return LossFunction.apply(time, noise.reshape(-1).to(torch.float32), hours, counts, 0, nfibers, nclasses, consts)
+    return LossFunction.apply(time, noise.reshape(-1).to(torch.float32), hours, counts, 0, nfibers, nclasses, consts,
+                              S_total)
 
 
 def loss_function(gnn, graph, class_info, pclass=0.1, pfiber=1.0, sharpness=0.5, finaloutput=False, *, nfibers=None,

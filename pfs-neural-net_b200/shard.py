@@ -55,6 +55,10 @@ def world_size():
     return dist.get_world_size(_state["group"]) if _state["active"] else 1
 
 
+def rank():
+    return dist.get_rank(_state["group"]) if _state["active"] else 0
+
+
 def allreduce_sum(t):
     """Sum of a (small, fp32) tensor over the shards; identity when not sharded."""
     if not active():
@@ -85,10 +89,29 @@ def allreduce_packed(tensors):
     return out
 
 
+def exchange_rows(row):
+    """Every shard's `row` (a 1-D tensor of n values), stacked in rank order as a [world, n] tensor of its dtype that is
+    bitwise the same on every rank: each rank fills its own row of a zero buffer and ONE all-reduce (sum) completes it --
+    adding zeros is exact, and all-reduce is the one collective every backend offers for CUDA tensors.  Not sharded:
+    the row as a [1, n] tensor."""
+    row = row.reshape(-1)
+    if not active():
+        return row.reshape(1, -1)
+    world = dist.get_world_size(_state["group"])
+    buf = torch.zeros(world, row.numel(), dtype=row.dtype, device=row.device)
+    buf[dist.get_rank(_state["group"])] = row
+    dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=_state["group"])
+    _state["bytes"] += buf.numel() * buf.element_size()
+    _state["calls"] += 1
+    return buf
+
+
 def shard_counts(n_local):
     """Per-shard values of a host-known integer (rows or edges of this shard), as a tuple indexed by rank.  The
     exchange (the only host synchronisation of the sharded path) runs ONCE per distinct local value inside a
-    fibre_sharded() scope family: shard sizes are properties of the partition, not of the step."""
+    fibre_sharded() scope family: shard sizes are properties of the partition, not of the step.  The cache is keyed by
+    (group, local value), and a miss is a collective, so all ranks must miss together: run a partition with other shard
+    sizes (another graph) in a group of its own when some rank's local value could repeat an earlier one."""
     if not active():
         return (int(n_local),)
     key = (id(_state["group"]), int(n_local))
@@ -120,16 +143,8 @@ def allreduce_moments(n, mean, m2):
     if not active():
         return n, mean, m2
     counts = shard_counts(int(n))
-    world = len(counts)
-    # gathered as an all-reduce of a [world, 2F] buffer in which every rank fills its own row (adding zeros is
-    # exact): all-reduce is the one collective every backend offers for CUDA tensors
     F = mean.numel()
-    allp = torch.zeros(world, 2 * F, dtype=torch.float32, device=mean.device)
-    allp[dist.get_rank(_state["group"])] = torch.cat([mean.reshape(-1), m2.reshape(-1)]).float()
-    dist.all_reduce(allp, op=dist.ReduceOp.SUM, group=_state["group"])
-    _state["bytes"] += allp.numel() * 4
-    _state["calls"] += 1
-    allp = allp.double()                                       # [world, 2F]
+    allp = exchange_rows(torch.cat([mean.reshape(-1), m2.reshape(-1)]).float()).double()       # [world, 2F]
     cnt = torch.tensor(counts, dtype=torch.float64, device=mean.device)[:, None]
     n_tot = float(sum(counts))
     # sum of n, n*mean, and m2 + n*mean^2 would cancel; merge the moments exactly:

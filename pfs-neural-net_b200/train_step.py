@@ -18,10 +18,14 @@ class table [T, 2] for all of them or [G, T, 2]: the step then trains on the sum
 parameter gradients of the G graphs stepped one after the other, summed) and returns the G utilities.  `load()`
 copies the next batch of the same shapes and topology into the step's input tensors, so an epoch over
 `Loader.batches(G)` replays the one captured graph.
+
+Inside `shard.fibre_sharded()` (one graph split over the ranks by fibre ranges) the step runs eager only
+(`use_graph=False`): its all-reduces are not captured into a CUDA graph.
 """
 import torch
 
 from . import loss as _loss
+from . import shard as _shard
 
 
 class TrainStep:
@@ -39,6 +43,9 @@ class TrainStep:
         self.loss = self.utility = None
         self._graph = None
         if use_graph:
+            if _shard.active():
+                raise ValueError("TrainStep: a fibre-sharded step all-reduces between ranks and runs eager "
+                                 "(use_graph=False); collectives are not captured into a CUDA graph")
             for g in optimizer.param_groups:
                 if not g.get("capturable", False):
                     raise ValueError("CUDA-graph capture needs torch.optim.Adam(..., capturable=True)")
