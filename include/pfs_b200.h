@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define PFS_ABI_VERSION 9
+#define PFS_ABI_VERSION 10
 
 enum {
     PFS_OK = 0,
@@ -395,7 +395,8 @@ int pfs_wide_transpose(const void* in_bf16, int32_t R, int32_t C, int64_t ld, vo
 /* -------------------------------------------------------------------------------------------
  * Training loss that consumes the edge times (reference src/train.py:21-80: softfloor + loss_function
  * from `time = gnn.edge_prediction(...)` on; SURVEY.md section 8f row N1).  fp32, dense canonical edge
- * order e = k*T + i (the reference reshapes the times to [NFIBERS, NCLASSES], src/train.py:67).  `noise`
+ * order e = k*T + i (the reference reshapes the times to [NFIBERS, NCLASSES], src/train.py:67), or any edge
+ * list (E > 0, ABI 10, below).  `noise`
  * is the uniform [0,1) draw of softfloor (torch.rand_like, src/train.py:22), supplied by the caller so the
  * result is reproducible.
  *   forward : galaxies = max(0, softfloor(time / T_i)), time2 = galaxies T_i, n'_i, fibre times, and
@@ -417,6 +418,14 @@ int pfs_wide_transpose(const void* in_bf16, int32_t R, int32_t C, int64_t ld, vo
  *      of pfs_loss_fwd.
  * pfs_loss_bwd with S_total set takes the variance over S_total fibres; time, noise, time2, fibre_time and g_time are
  * the local rows, class_mean and class_coef the merged ones.
+ * Any edge list (ABI 10): E > 0 edges per graph in any order (duplicates, fibres and classes without edges allowed),
+ * edge e = (fibre csr_src, class csr_tgt) as listed by the CSR / CSC arrays of pfs_build_topology, shared by the G graphs.
+ * Every per-edge array is then [G, E] in edge-list order (E replaces S*T above).  The variance runs over the fibre x class
+ * matrix of cells c_ki = sum of time2 over the edges (k, i), 0 where fibre k has no edge to class i; a fibre without edges
+ * has fibre time 0, a class without edges n'_i = 0.  The forward is 4 launches and also writes cell_time [G, E] (the cell
+ * value of every edge), which the backward (1 launch) reads.  Workspace: G * pfs_loss_list_workspace_bytes(T).  Graph g's
+ * results are bitwise those of a one-graph call.  E > 0 with S_total set, or with a NULL edge array or cell_time, and
+ * E = 0 with an edge array set, are refused (PFS_ERR_ARG).
  * ---------------------------------------------------------------------------------------- */
 typedef struct pfs_loss_args {
     int32_t S, T;                                /* fibres, classes (per graph) */
@@ -447,9 +456,20 @@ typedef struct pfs_loss_args {
     int32_t world;                               /* ABI 9: ranks of the sharded graph (pfs_loss_shard_merge) */
     double* shard_record;                        /* ABI 9: pfs_loss_shard_fwd output, [2 + 3T] */
     const double* shard_records;                 /* ABI 9: pfs_loss_shard_merge input, [world][2 + 3T] in rank order */
+    int32_t E;                                   /* ABI 10: edges per graph of an edge list; 0 = the dense canonical order
+                                                    e = k*T + i (the ABI 9 behaviour, every array below NULL) */
+    const int32_t* csr_rowptr;                   /* ABI 10: [S+1]  pfs_build_topology's CSR range of each fibre */
+    const int32_t* csr_eid;                      /* ABI 10: [E]    edge id at CSR position q */
+    const int32_t* csr_src;                      /* ABI 10: [E]    fibre at CSR position q */
+    const int32_t* csr_tgt;                      /* ABI 10: [E]    class at CSR position q */
+    const int32_t* csc_colptr;                   /* ABI 10: [T+1]  CSC range of each class */
+    const int32_t* csc_q;                        /* ABI 10: [E]    CSR position of the j-th class-sorted edge */
+    float* cell_time;                            /* ABI 10: [G, E] forward output, backward input: the cell value c_ki of
+                                                    every edge */
 } pfs_loss_args;
 size_t pfs_sizeof_loss_args(void);
 size_t pfs_loss_workspace_bytes(int32_t S, int32_t T);
+size_t pfs_loss_list_workspace_bytes(int32_t T);      /* per graph, E > 0 */
 int pfs_loss_fwd(const pfs_loss_args* a);
 int pfs_loss_bwd(const pfs_loss_args* a);
 int pfs_loss_shard_fwd(const pfs_loss_args* a);

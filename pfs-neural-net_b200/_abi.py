@@ -18,7 +18,7 @@ HEADER = os.path.join(os.path.dirname(_HERE), "include", "pfs_b200.h")
 PFS_LAYOUT_DENSE = 0
 PFS_LAYOUT_CSR = 1
 PFS_TILE_EDGES = 256
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 _P = ct.c_void_p
 
@@ -130,8 +130,10 @@ class LossArgs(ct.Structure):
         [(n, _P) for n in "galaxies time2 fibre_time n_prime class_mean class_coef scalars g_loss g_time workspace".split()] + \
         [("workspace_bytes", ct.c_size_t), ("stream", _P), ("sharpness_dev", _P)] + \
         [("G", ct.c_int32), ("class_tables", ct.c_int32)] + \
-        [("S_total", ct.c_int32), ("world", ct.c_int32), ("shard_record", _P), ("shard_records", _P)]
-# ABI 8 appended the graph dimension (G, class_tables), ABI 9 the fibre-sharded graph (S_total ... shard_records)
+        [("S_total", ct.c_int32), ("world", ct.c_int32), ("shard_record", _P), ("shard_records", _P)] + \
+        [("E", ct.c_int32)] + [(n, _P) for n in "csr_rowptr csr_eid csr_src csr_tgt csc_colptr csc_q cell_time".split()]
+# ABI 8 appended the graph dimension (G, class_tables), ABI 9 the fibre-sharded graph (S_total ... shard_records),
+# ABI 10 the edge list (E ... cell_time)
 
 
 class WideSegments(ct.Structure):
@@ -193,6 +195,7 @@ SYMBOLS = {
     # training loss (reference src/train.py:21-80)
     "pfs_sizeof_loss_args": (ct.c_size_t, []),
     "pfs_loss_workspace_bytes": (ct.c_size_t, [_I32, _I32]),
+    "pfs_loss_list_workspace_bytes": (ct.c_size_t, [_I32]),
     "pfs_loss_fwd": (ct.c_int, [ct.POINTER(LossArgs)]),
     "pfs_loss_bwd": (ct.c_int, [ct.POINTER(LossArgs)]),
     "pfs_loss_shard_fwd": (ct.c_int, [ct.POINTER(LossArgs)]),

@@ -14,6 +14,13 @@
 // penalty, per class sum of galaxies, mean and M2 of time2).  The caller exchanges the records, and k_loss_shard_merge
 // combines them in rank order and runs the same tail as k_loss_scalars on the global totals.  The backward is the one-graph
 // kernel with the variance taken over S_total fibres.
+//
+// Any edge list (ABI 10, DESIGN.md section 8b): E edges per graph in any order, with duplicates, empty fibres and empty
+// classes, visited through the CSR / CSC arrays of pfs_build_topology.  The variance runs over the fibre x class matrix of
+// cells c_ki = sum of time2 over the edges (k, i), 0 where fibre k has no edge to class i.  Four forward kernels (edge
+// pass in CSR order, fibre sums, one CTA per class over its CSC list, the loss tail) and one backward kernel; a class
+// segment is cut into chunks by its length alone and the chunks are combined in a fixed tree, so the results do not
+// depend on G or on a graph's position in the batch.
 #include <cstdarg>
 #include <cstdio>
 #include <math_constants.h>
@@ -367,14 +374,203 @@ __global__ void __launch_bounds__(256) k_loss_edge_bwd(LossConst c, int S_var, c
     }
 }
 
+// ---- edge-list loss --------------------------------------------------------------------------------------------------
+// the CSR / CSC arrays of pfs_build_topology, shared by the G graphs; graph g's edges start at g*E
+struct ListTopo {
+    long long E;                                 // edges per graph
+    const int* __restrict__ rowptr;              // [S+1] CSR range of each fibre
+    const int* __restrict__ eid;                 // [E]   edge id at CSR position p
+    const int* __restrict__ src;                 // [E]   fibre at CSR position p
+    const int* __restrict__ tgt;                 // [E]   class at CSR position p
+    const int* __restrict__ colptr;              // [T+1] CSC range of each class
+    const int* __restrict__ cscq;                // [E]   CSR position of the j-th class-sorted edge (fibre-ascending per class)
+};
+
+// per edge, visited in CSR order: galaxies and time2 at the edge id, with the arithmetic of k_loss_edge_fwd
+__global__ void __launch_bounds__(256) k_loss_list_edge_fwd(LossConst c, const ListTopo t, const float* __restrict__ time,
+                                                            const float* __restrict__ noise, const float* __restrict__ hours,
+                                                            float* __restrict__ galaxies, float* __restrict__ time2) {
+    resolve_sharpness(c);
+    const long long n = (long long)c.G * t.E;
+    for (long long x = (long long)blockIdx.x * blockDim.x + threadIdx.x; x < n; x += (long long)gridDim.x * blockDim.x) {
+        const int g = c.G > 1 ? (int)(x / t.E) : 0;
+        const long long p = x - (long long)g * t.E;
+        const size_t e = (size_t)g * t.E + t.eid[p];
+        const float h = hours[(size_t)g * c.class_stride + t.tgt[p]];
+        float sf, dsf;
+        softfloor_eval(time[e] / h, noise[e], c, sf, dsf);
+        const float gal = fmaxf(sf, 0.f);
+        galaxies[e] = gal;
+        time2[e] = gal * h;
+    }
+}
+
+// fibre sums of time2 over each fibre's CSR range: one warp per fibre, GS = G*S fibres over all graphs (a fibre without
+// edges gets 0).  On the canonical graph the lanes sum the edges of k_loss_fibre_sums in its order.
+__global__ void __launch_bounds__(256) k_loss_list_fibre_sums(int S, const ListTopo t, long long GS,
+                                                              const float* __restrict__ time2, float* __restrict__ fibre_time) {
+    const long long w = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (w >= GS) return;
+    const int g = (int)(w / S), k = (int)(w - (long long)g * S);
+    const float* t2 = time2 + (size_t)g * t.E;
+    float s = 0.f;
+    for (int p = t.rowptr[k] + lane; p < t.rowptr[k + 1]; p += 32) s += t2[t.eid[p]];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) fibre_time[w] = s;
+}
+
+// Class pass: one CTA of 256 threads per (graph, class), block = g*T + i.  The class's CSC segment is cut into 256 chunks of
+// ceil(len / 256) edges.  Within a class the edges are fibre-ascending, so the edges of one cell are a run; a run belongs
+// to the chunk where it starts (that thread reads on past its chunk's end, the next chunk skips it).  Each thread writes
+// the cell value to cell_time at every edge of its runs and reduces its cells to (count, mean, M2) and its galaxies to a
+// sum, all in fp64; the 256 partial results are combined by a fixed tree (the pairwise update, Chan et al.), then the
+// S - count zero cells are folded in.  stats [G][3][T] = {sum galaxies, mean and M2 of the cells over all S fibres}.
+__global__ void __launch_bounds__(256) k_loss_list_class(int S, int T, const ListTopo t, const float* __restrict__ galaxies,
+                                                         const float* __restrict__ time2, float* __restrict__ cell_time,
+                                                         double* __restrict__ stats) {
+    __shared__ double s_n[256], s_mean[256], s_m2[256], s_gal[256];
+    const int g = blockIdx.x / T, i = blockIdx.x - g * T;
+    const size_t off = (size_t)g * t.E;
+    galaxies += off;
+    time2 += off;
+    cell_time += off;
+    const int j0 = t.colptr[i], j1 = t.colptr[i + 1];
+    const int len = (j1 - j0 + 255) / 256;
+    const long long c0 = j0 + (long long)threadIdx.x * len;
+    int j = (int)min(c0, (long long)j1);
+    const int jend = (int)min(c0 + len, (long long)j1);
+    if (j > j0 && j < jend) {                   // the run that crosses into this chunk belongs to the previous one
+        const int kp = t.src[t.cscq[j - 1]];
+        while (j < jend && t.src[t.cscq[j]] == kp) ++j;
+    }
+    double n = 0.0, mean = 0.0, m2 = 0.0, gal = 0.0;
+    while (j < jend) {
+        const int k = t.src[t.cscq[j]];
+        float cell = 0.f;
+        int r = j;
+        do {
+            const int e = t.eid[t.cscq[r]];
+            cell += time2[e];
+            gal += (double)galaxies[e];
+            ++r;
+        } while (r < j1 && t.src[t.cscq[r]] == k);
+        for (int w = j; w < r; ++w) cell_time[t.eid[t.cscq[w]]] = cell;
+        n += 1.0;
+        const double d = (double)cell - mean;
+        mean += d / n;
+        m2 += d * ((double)cell - mean);
+        j = r;
+    }
+    s_n[threadIdx.x] = n; s_mean[threadIdx.x] = mean; s_m2[threadIdx.x] = m2; s_gal[threadIdx.x] = gal;
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {          // chunk a = thread, chunk b = thread + o (b follows a in the segment)
+        if (threadIdx.x < o) {
+            const int b = threadIdx.x + o;
+            const double na = s_n[threadIdx.x], nb = s_n[b];
+            if (nb > 0.0) {
+                const double nab = na + nb, d = s_mean[b] - s_mean[threadIdx.x];
+                s_mean[threadIdx.x] += d * nb / nab;
+                s_m2[threadIdx.x] += s_m2[b] + d * d * na * nb / nab;
+                s_n[threadIdx.x] = nab;
+            }
+            s_gal[threadIdx.x] += s_gal[b];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        const double cnt = s_n[0], mc = s_mean[0], Sd = (double)S;
+        double* o = stats + (size_t)g * 3 * T;
+        o[i] = s_gal[0];
+        o[T + i] = mc * cnt / Sd;                                    // = sum of the cells / S
+        o[2 * T + i] = s_m2[0] + cnt * (Sd - cnt) / Sd * mc * mc;    // + the S - cnt zero cells, pairwise
+    }
+}
+
+// one CTA per graph: the loss tail on the class pass's totals
+__global__ void __launch_bounds__(1024) k_loss_list_scalars(const LossConst c, const double* __restrict__ stats,
+                                                            const float* __restrict__ counts, const float* __restrict__ fibre_time,
+                                                            float* __restrict__ n_prime, float* __restrict__ class_mean,
+                                                            float* __restrict__ class_coef, float* __restrict__ scalars) {
+    __shared__ double red[1024];
+    __shared__ float s_min;
+    const int S = c.S, T = c.T;
+    const size_t g = blockIdx.x;
+    const double* st = stats + g * 3 * T;
+    counts += g * c.class_stride;
+    fibre_time += g * S;
+    n_prime += g * T;
+    class_mean += g * T;
+    class_coef += g * T;
+    scalars += g * 8;
+    loss_tail(c, (double)S,
+              [&](int i, double& s0, double& mean, double& m2) {
+                  s0 = st[i];
+                  mean = st[T + i];
+                  m2 = st[2 * T + i];
+              },
+              [&] { return fibre_penalty_sum(c, fibre_time, red); },
+              counts, n_prime, class_mean, class_coef, scalars, red, &s_min);
+}
+
+// g_time of k_loss_edge_bwd per edge in CSR order, with the edge's cell value in place of its time2
+__global__ void __launch_bounds__(256) k_loss_list_edge_bwd(LossConst c, const ListTopo t, const float* __restrict__ time,
+                                                            const float* __restrict__ noise, const float* __restrict__ hours,
+                                                            const float* __restrict__ cell_time,
+                                                            const float* __restrict__ fibre_time,
+                                                            const float* __restrict__ class_mean,
+                                                            const float* __restrict__ class_coef,
+                                                            const float* __restrict__ g_loss, float* __restrict__ g_time) {
+    resolve_sharpness(c);
+    const long long n = (long long)c.G * t.E;
+    const float vscale = 2.f * c.wvar / (float)(c.S - 1);
+    for (long long x = (long long)blockIdx.x * blockDim.x + threadIdx.x; x < n; x += (long long)gridDim.x * blockDim.x) {
+        const int g = c.G > 1 ? (int)(x / t.E) : 0;
+        const long long p = x - (long long)g * t.E;
+        const size_t e = (size_t)g * t.E + t.eid[p];
+        const int i = t.tgt[p];
+        const size_t ci = (size_t)g * c.T + i;
+        const float h = hours[(size_t)g * c.class_stride + i];
+        float sf, dsf;
+        softfloor_eval(time[e] / h, noise[e], c, sf, dsf);
+        float gt = 0.f;
+        if (sf > 0.f) {
+            const float gl = g_loss ? g_loss[g] : 1.f;
+            const float ot = fibre_time[(size_t)g * c.S + t.src[p]] - c.total_time;
+            const float dft = 2.f * c.pfiber * (ot > 0.f ? ot : 0.01f * ot);
+            const float d_t2 = dft - vscale * (cell_time[e] - class_mean[ci]);
+            gt = gl * (class_coef[ci] + h * d_t2) * dsf / h;
+        }
+        g_time[e] = gt;
+    }
+}
+
+// the edge arrays of an edge-list call (E > 0): every array set, no sharding
+int list_topo(const pfs_loss_args& a, ListTopo& t) {
+    L_REQUIRE(a.csr_rowptr && a.csr_eid && a.csr_src && a.csr_tgt && a.csc_colptr && a.csc_q && a.cell_time,
+              "loss: an edge list (E > 0) needs csr_rowptr, csr_eid, csr_src, csr_tgt, csc_colptr, csc_q and cell_time");
+    t.E = a.E;
+    t.rowptr = a.csr_rowptr; t.eid = a.csr_eid; t.src = a.csr_src; t.tgt = a.csr_tgt;
+    t.colptr = a.csc_colptr; t.cscq = a.csc_q;
+    return PFS_OK;
+}
+
 int make_const(const pfs_loss_args& a, LossConst& c) {
-    if (a.S_total) {         // one shard of a graph: the graph needs 2 fibres, the shard 1
+    L_REQUIRE(a.E >= 0, "loss: negative edge count E");
+    if (a.E > 0) {           // an edge list: nothing of size S*T is stored
+        L_REQUIRE(a.S_total == 0, "loss: an edge list (E > 0) cannot be fibre-sharded; S_total must be 0");
+        L_REQUIRE(a.S >= 2 && a.T >= 1, "loss: bad edge-list sizes (at least 2 fibres and 1 class)");
+    } else if (a.S_total) {         // one shard of a graph: the graph needs 2 fibres, the shard 1
         L_REQUIRE(a.S >= 1 && a.S_total >= 2 && a.S <= a.S_total && a.T >= 1 && (long long)a.S * a.T < (1ll << 31),
                   "loss: bad shard sizes (at least 1 local fibre, 2 over all shards)");
         L_REQUIRE(a.G == 0 || a.G == 1, "loss: a sharded graph is one graph per call (G 0 or 1)");
     } else {
         L_REQUIRE(a.S >= 2 && a.T >= 1 && (long long)a.S * a.T < (1ll << 31), "loss: bad graph sizes (at least 2 fibres)");
     }
+    if (a.E == 0)
+        L_REQUIRE(!a.csr_rowptr && !a.csr_eid && !a.csr_src && !a.csr_tgt && !a.csc_colptr && !a.csc_q && !a.cell_time,
+                  "loss: edge arrays are set but E (edges per graph) is 0");
     L_REQUIRE(a.G >= 0, "loss: negative graph count");
     L_REQUIRE(a.class_tables == 0 || a.class_tables == 1, "loss: class_tables is 0 (one [T] table) or 1 ([G, T])");
     c.S = a.S; c.T = a.T;
@@ -415,12 +611,35 @@ int loss_edges_and_partials(const pfs_loss_args* a, const LossConst& c, cudaStre
     return PFS_OK;
 }
 
+// the edge-list forward (E > 0): edge pass, fibre sums, class pass, tail (4 launches)
+int loss_list_fwd(const pfs_loss_args* a, const LossConst& c, cudaStream_t st) {
+    ListTopo t;
+    if (int rc = list_topo(*a, t)) return rc;
+    L_REQUIRE((long long)c.G * c.T < (1ll << 31), "loss: too many graphs x classes for one launch (G*T < 2^31)");
+    if (a->workspace_bytes < (size_t)c.G * 3 * c.T * sizeof(double) + 256)
+        return lfail(PFS_ERR_WORKSPACE, "loss: workspace too small (%zu bytes for %d graph(s) of an edge list)",
+                     a->workspace_bytes, c.G);
+    double* stats = (double*)(((uintptr_t)a->workspace + 255) & ~(uintptr_t)255);
+    const long long GS = (long long)c.G * c.S;
+    k_loss_list_edge_fwd<<<edge_grid(c.G * t.E), 256, 0, st>>>(c, t, a->time, a->noise, a->hours, a->galaxies, a->time2);
+    L_LAUNCH_CHECK("k_loss_list_edge_fwd");
+    k_loss_list_fibre_sums<<<(unsigned)((GS * 32 + 255) / 256), 256, 0, st>>>(c.S, t, GS, a->time2, a->fibre_time);
+    L_LAUNCH_CHECK("k_loss_list_fibre_sums");
+    k_loss_list_class<<<c.G * c.T, 256, 0, st>>>(c.S, c.T, t, a->galaxies, a->time2, a->cell_time, stats);
+    L_LAUNCH_CHECK("k_loss_list_class");
+    k_loss_list_scalars<<<c.G, 1024, 0, st>>>(c, stats, a->counts, a->fibre_time, a->n_prime, a->class_mean, a->class_coef,
+                                              a->scalars);
+    L_LAUNCH_CHECK("k_loss_list_scalars");
+    return PFS_OK;
+}
+
 }  // namespace
 
 extern "C" {
 
 size_t pfs_sizeof_loss_args(void) { return sizeof(pfs_loss_args); }
 size_t pfs_loss_workspace_bytes(int32_t S, int32_t T) { return (size_t)class_row_blocks(S) * 3 * T * sizeof(float) + 256; }
+size_t pfs_loss_list_workspace_bytes(int32_t T) { return (size_t)3 * T * sizeof(double) + 256; }
 
 
 int pfs_loss_fwd(const pfs_loss_args* a) {
@@ -431,6 +650,7 @@ int pfs_loss_fwd(const pfs_loss_args* a) {
     if (int rc = make_const(*a, c)) return rc;
     cudaStream_t st = (cudaStream_t)a->stream;
     pfs_host::mark_launch(nullptr, st);
+    if (a->E > 0) return loss_list_fwd(a, c, st);
     const int nrb = class_row_blocks(c.S);
     float* partial;
     if (int rc = loss_edges_and_partials(a, c, st, nrb, &partial)) return rc;
@@ -477,6 +697,15 @@ int pfs_loss_bwd(const pfs_loss_args* a) {
     if (int rc = make_const(*a, c)) return rc;
     cudaStream_t st = (cudaStream_t)a->stream;
     pfs_host::mark_launch(nullptr, st);
+    if (a->E > 0) {
+        ListTopo t;
+        if (int rc = list_topo(*a, t)) return rc;
+        k_loss_list_edge_bwd<<<edge_grid(c.G * t.E), 256, 0, st>>>(c, t, a->time, a->noise, a->hours, a->cell_time,
+                                                                   a->fibre_time, a->class_mean, a->class_coef, a->g_loss,
+                                                                   a->g_time);
+        L_LAUNCH_CHECK("k_loss_list_edge_bwd");
+        return PFS_OK;
+    }
     const int S_var = a->S_total ? a->S_total : c.S;
     k_loss_edge_bwd<<<edge_grid((long long)c.G * c.S * c.T), 256, 0, st>>>(c, S_var, a->time, a->noise, a->hours, a->time2,
                                                                     a->fibre_time, a->class_mean, a->class_coef, a->g_loss,

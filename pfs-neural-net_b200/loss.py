@@ -7,7 +7,14 @@ message-passing path, consuming `GNN.edge_prediction`'s times.
 reads (`gnn`, NFIBERS, NCLASSES, NFIELDS, TOTAL_TIME, wutils, wvar; src/config.py:16-28) are explicit
 arguments with the reference's values as defaults.  The uniform noise of `softfloor` is drawn with
 `torch.rand_like` exactly where the reference draws it (so a seeded run consumes the generator the
-same way) or can be passed in.  fp32, dense canonical edge order; no CPU fallback.
+same way) or can be passed in.  fp32; no CPU fallback.
+
+The edge order is the canonical dense one (e = k*T + i, which the reference reshapes to [NFIBERS, NCLASSES]) or any
+edge list: `loss_from_times(..., edge_index=...)`, and `loss_function` on a graph whose `edge_index` is not canonical
+(a class-permuted file such as the reference's graphs/graph-0.pt, or a sparse visibility graph).  On an edge list the
+variance runs over the fibre x class matrix of cells c_ki = sum of time2 over the edges (k, i), 0 where fibre k has no
+edge to class i (DESIGN.md section 8b): on any permutation of the complete graph that is the reference loss of the
+un-permuted graph.
 
 Both functions also take a batch of G graphs that share one `edge_index` (the leading graph dimension of
 `Loader.collate`): edge times [G, E], one class table [T, 2] for all graphs or one per graph [G, T, 2].  Each
@@ -36,17 +43,19 @@ class LossFunction(torch.autograd.Function):
     G = 0: one graph (time [S*T], hours / counts [T]; the loss is a scalar).  G >= 1: a batch (time [G, S*T], hours /
     counts [T] shared or [G, T]; the loss is [G] and every other output gains the leading G).
     S_total > 0: this rank's S fibres of a graph of S_total fibres sharded over the active group (G = 0): the forward is
-    pfs_loss_shard_fwd, the record exchange (shard.exchange_rows) and pfs_loss_shard_merge."""
+    pfs_loss_shard_fwd, the record exchange (shard.exchange_rows) and pfs_loss_shard_merge.
+    edges: None (canonical order, E = S*T) or an edge list {"E": edges per graph, and the int32 CSR / CSC arrays of
+    Topology.csr()}; the forward saves the per-edge cell values for the backward."""
 
     @staticmethod
-    def forward(ctx, time, noise, hours, counts, G, S, T, consts, S_total):
+    def forward(ctx, time, noise, hours, counts, G, S, T, consts, S_total, edges=None):
         for t, n in ((time, "time"), (noise, "noise"), (hours, "hours"), (counts, "counts")):
             if not t.is_cuda:
                 raise _abi.PfsError("pfs_b200 loss needs CUDA tensors, %s is on %s (no CPU fallback)" % (n, t.device))
             if t.dtype != torch.float32:
                 raise _abi.PfsError("pfs_b200 loss is fp32, %s is %s" % (n, t.dtype))
         time, noise, hours, counts = (t.contiguous() for t in (time, noise, hours, counts))
-        E = S * T
+        E = S * T if edges is None else edges["E"]
         nt = max(G, 1) * T if hours.dim() == 2 else T
         if time.numel() != max(G, 1) * E or noise.numel() != time.numel() or hours.numel() != nt or counts.numel() != nt:
             raise _abi.PfsError("loss: expected %d edge times / noise values and %d class rows" % (max(G, 1) * E, nt))
@@ -60,7 +69,12 @@ class LossFunction(torch.autograd.Function):
                    fibre_time=torch.empty(lead + (S,), **f32), n_prime=torch.empty(lead + (T,), **f32),
                    class_mean=torch.empty(lead + (T,), **f32), class_coef=torch.empty(lead + (T,), **f32),
                    scalars=torch.zeros(lead + (8,), **f32))
-        ws = torch.empty(max(G, 1) * lib.pfs_loss_workspace_bytes(S, T), dtype=torch.uint8, device=dev)
+        if edges is None:
+            ws = torch.empty(max(G, 1) * lib.pfs_loss_workspace_bytes(S, T), dtype=torch.uint8, device=dev)
+        else:
+            out["cell_time"] = torch.empty(lead + (E,), **f32)
+            ws = torch.empty(max(G, 1) * lib.pfs_loss_list_workspace_bytes(T), dtype=torch.uint8, device=dev)
+            _set_edges(a, edges)
         for k, v in dict(time=time, noise=noise, hours=hours, counts=counts, **out).items():
             setattr(a, k, v.data_ptr())
         sharp_dev = consts.get("sharpness_dev")
@@ -80,15 +94,16 @@ class LossFunction(torch.autograd.Function):
                 _abi.check(lib.pfs_loss_shard_merge(ct.byref(a)), "pfs_loss_shard_merge")
             else:
                 _abi.check(lib.pfs_loss_fwd(ct.byref(a)), "pfs_loss_fwd")
-        ctx.G, ctx.S, ctx.T, ctx.S_total, ctx.consts = G, S, T, S_total, dict(consts)
-        ctx.save_for_backward(time, noise, hours, counts, out["time2"], out["fibre_time"], out["class_mean"], out["class_coef"])
+        ctx.G, ctx.S, ctx.T, ctx.S_total, ctx.consts, ctx.edges = G, S, T, S_total, dict(consts), edges
+        ctx.save_for_backward(time, noise, hours, counts, out["time2"], out["fibre_time"], out["class_mean"], out["class_coef"],
+                              out.get("cell_time"))
         sc = out["scalars"]
         ctx.mark_non_differentiable(sc, out["n_prime"], out["fibre_time"], out["time2"])
         return sc[..., 0].clone(), sc, out["n_prime"], out["fibre_time"], out["time2"]
 
     @staticmethod
     def backward(ctx, g_loss, *_):
-        time, noise, hours, counts, time2, fibre_time, class_mean, class_coef = ctx.saved_tensors
+        time, noise, hours, counts, time2, fibre_time, class_mean, class_coef, cell_time = ctx.saved_tensors
         dev = time.device
         g_time = torch.empty_like(time)
         gl = g_loss.detach().to(torch.float32).reshape(-1).contiguous()
@@ -97,6 +112,9 @@ class LossFunction(torch.autograd.Function):
         for k, v in dict(time=time, noise=noise, hours=hours, counts=counts, time2=time2, fibre_time=fibre_time,
                          class_mean=class_mean, class_coef=class_coef, g_loss=gl, g_time=g_time).items():
             setattr(a, k, v.data_ptr())
+        if ctx.edges is not None:
+            _set_edges(a, ctx.edges)
+            a.cell_time = cell_time.data_ptr()
         for k, v in ctx.consts.items():
             if k != "sharpness_dev":
                 setattr(a, k, float(v))
@@ -104,7 +122,25 @@ class LossFunction(torch.autograd.Function):
         with torch.cuda.device(dev):
             a.stream = torch.cuda.current_stream(dev).cuda_stream
             _abi.check(_abi.load_library().pfs_loss_bwd(ct.byref(a)), "pfs_loss_bwd")
-        return g_time, None, None, None, None, None, None, None, None
+        return g_time, None, None, None, None, None, None, None, None, None
+
+
+_EDGE_ARRAYS = ("csr_rowptr", "csr_eid", "csr_src", "csr_tgt", "csc_colptr", "csc_q")
+
+
+def _set_edges(a, edges):
+    a.E = edges["E"]
+    for k in _EDGE_ARRAYS:
+        setattr(a, k, edges[k].data_ptr())
+
+
+def _edge_list(edge_index, S, T):
+    """the LossFunction `edges` of an edge_index [2, E]: the cached CSR / CSC arrays of its Topology (built once per
+    edge_index, in the first call; a captured step finds them cached)"""
+    from .topology import get_topology
+    topo = get_topology(edge_index, S, T)
+    arrays = topo.csr()
+    return dict(E=topo.E, **{k: arrays[k] for k in _EDGE_ARRAYS})
 
 
 def _graph_rows(x, E):
@@ -114,8 +150,8 @@ def _graph_rows(x, E):
     return x if x.dim() == 2 and x.shape[1] == E else None
 
 
-def _batched_loss(time, class_info, S, T, nfields, consts, noise):
-    E = S * T
+def _batched_loss(time, class_info, S, T, nfields, consts, noise, edges=None):
+    E = S * T if edges is None else edges["E"]
     t = _graph_rows(time, E)
     if t is None:
         raise _abi.PfsError("loss: a batch of edge times is [G, %d] or [G, %d, 1], got %s" % (E, E, tuple(time.shape)))
@@ -137,11 +173,11 @@ def _batched_loss(time, class_info, S, T, nfields, consts, noise):
         noise = n
     hours = class_info[..., 0].to(torch.float32)
     counts = (class_info[..., 1] / nfields).to(torch.float32)
-    return LossFunction.apply(t, noise.to(torch.float32), hours, counts, G, S, T, consts, 0)
+    return LossFunction.apply(t, noise.to(torch.float32), hours, counts, G, S, T, consts, 0, edges)
 
 
 def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=42, wutils=2000.0, wvar=1.0, pclass=0.1,
-                    pfiber=1.0, sharpness=0.5, noise=None):
+                    pfiber=1.0, sharpness=0.5, noise=None, edge_index=None):
     """Loss terms from the edge times [E] (or [E,1]); returns (loss, scalars, n_prime, fibre_time, time2) where
     scalars = [loss, totutils, class_penalty, fibre_penalty, variance, #minima, 0, 0].
 
@@ -156,7 +192,12 @@ def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=
     of one graph; the loss, scalars and n_prime are those of the whole graph (bitwise the same on every rank),
     fibre_time and time2 the local rows.  Without `noise` the whole graph's S_total * T draws are made by one
     torch.rand and this rank takes its slice [f0 * T, f1 * T), so a run seeded alike on every rank draws bitwise the
-    noise of the single-GPU run and no two shards share draws.  A batch of graphs is refused."""
+    noise of the single-GPU run and no two shards share draws.  A batch of graphs is refused.
+
+    `edge_index` [2, E] (int64, on the device): the edges in any order, edge e = (fibre edge_index[0, e], class
+    edge_index[1, e]); `time` is [E], [E, 1], [G, E] or [G, E, 1] in that order, and so are `noise` and time2.  None:
+    the canonical dense order e = k*T + i.  An edge list is not fibre-sharded: inside `shard.fibre_sharded()` it is
+    refused."""
     consts = dict(total_time=total_time, wutils=wutils, wvar=wvar, pclass=pclass, pfiber=pfiber, noiselevel=NOISELEVEL)
     if torch.is_tensor(sharpness):                # device scalar: the value is read by the kernels (CUDA-graph replays)
         consts.update(sharpness=0.0, sharpness_dev=sharpness.to(torch.float32).reshape(1))
@@ -164,10 +205,17 @@ def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=
         consts.update(sharpness=sharpness)
     nfibers, nclasses = int(nfibers), int(nclasses)
     sharded = _shard.active()
-    if time.dim() == 3 or (time.dim() == 2 and time.shape[1] == nfibers * nclasses):
+    edges = None
+    if edge_index is not None:
+        if sharded:
+            raise _abi.PfsError("loss: an edge list cannot be fibre-sharded: the sharded loss splits the canonical order "
+                                "e = k*T + i into contiguous fibre ranges")
+        edges = _edge_list(edge_index, nfibers, nclasses)
+    E = nfibers * nclasses if edges is None else edges["E"]
+    if time.dim() == 3 or (time.dim() == 2 and time.shape[1] == E):
         if sharded:
             raise _abi.PfsError("loss: a fibre-sharded graph is one graph per call, not a batch of %d" % time.shape[0])
-        return _batched_loss(time, class_info, nfibers, nclasses, nfields, consts, noise)
+        return _batched_loss(time, class_info, nfibers, nclasses, nfields, consts, noise, edges)
     time = time.reshape(-1)
     if time.dtype != torch.float32:
         time = time.float()                       # bf16 head output: dtype plumbing, the loss itself is fp32
@@ -182,7 +230,7 @@ def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=
     hours = class_info[:, 0].to(torch.float32)
     counts = (class_info[:, 1] / nfields).to(torch.float32)
     return LossFunction.apply(time, noise.reshape(-1).to(torch.float32), hours, counts, 0, nfibers, nclasses, consts,
-                              S_total)
+                              S_total, edges)
 
 
 def loss_function(gnn, graph, class_info, pclass=0.1, pfiber=1.0, sharpness=0.5, finaloutput=False, *, nfibers=None,
@@ -201,12 +249,16 @@ def loss_function(gnn, graph, class_info, pclass=0.1, pfiber=1.0, sharpness=0.5,
     nclasses = int(nclasses if nclasses is not None else graph.x_t.shape[-2])
     nfibers = int(nfibers if nfibers is not None else graph.x_s.shape[-2])
     topo = get_topology(graph.edge_index, nfibers, nclasses)
+    edge_index = None
     if not topo.canonical:
-        raise _abi.PfsError("the loss needs the canonical dense edge order e = k*T + i (reference src/train.py:67 "
-                            "reshapes the times to [NFIBERS, NCLASSES])")
+        if _shard.active():
+            raise _abi.PfsError("loss: a fibre-sharded graph needs the canonical dense edge order e = k*T + i, because the "
+                                "sharded loss splits that order into contiguous fibre ranges; this graph's edge_index is "
+                                "not canonical")
+        edge_index = graph.edge_index           # any edge list: the cell-matrix loss of DESIGN.md section 8b
     time = gnn.edge_prediction(graph.x_e, scale=total_time / nclasses).squeeze(-1)
     loss, sc, n_prime, fibre_time, time2 = loss_from_times(time, class_info, nfibers, nclasses, nfields, total_time, wutils,
-                                                            wvar, pclass, pfiber, sharpness, noise)
+                                                            wvar, pclass, pfiber, sharpness, noise, edge_index)
     if batched:
         loss = loss.sum() if reduction == "sum" else loss.mean()
     if not finaloutput:
