@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define PFS_ABI_VERSION 10
+#define PFS_ABI_VERSION 11
 
 enum {
     PFS_OK = 0,
@@ -426,6 +426,16 @@ int pfs_wide_transpose(const void* in_bf16, int32_t R, int32_t C, int64_t ld, vo
  * value of every edge), which the backward (1 launch) reads.  Workspace: G * pfs_loss_list_workspace_bytes(T).  Graph g's
  * results are bitwise those of a one-graph call.  E > 0 with S_total set, or with a NULL edge array or cell_time, and
  * E = 0 with an edge array set, are refused (PFS_ERR_ARG).
+ * Edge list sharded over fibre ranges (ABI 11): each rank holds the edges of its contiguous fibre range (S local fibres,
+ * fibres renumbered from 0, S_total over all ranks, E > 0 local edges and their CSR / CSC arrays, one graph per call).
+ *   1. pfs_loss_list_shard_fwd: the per-edge and per-fibre outputs of the local edges (cell_time included) and this
+ *      rank's record shard_record [2 + 3T] = {S, local fibre-penalty sum, per class: sum galaxies, mean and M2 of the
+ *      cells over the S local fibres, zero cells included} (4 launches, workspace pfs_loss_list_workspace_bytes(T));
+ *   2. the records exchanged as for ABI 9;
+ *   3. pfs_loss_shard_merge with E = 0 and every edge array NULL (the records mean what ABI 9's mean).
+ *   With world = 1 the results are bitwise those of pfs_loss_fwd on the same edge list.
+ * pfs_loss_list_shard_bwd: the edge-list backward with the variance over S_total fibres (1 launch).  Both refuse
+ * (PFS_ERR_ARG, before any CUDA call) a NULL array, E <= 0, S_total unset, S > S_total and G > 1.
  * ---------------------------------------------------------------------------------------- */
 typedef struct pfs_loss_args {
     int32_t S, T;                                /* fibres, classes (per graph) */
@@ -474,6 +484,8 @@ int pfs_loss_fwd(const pfs_loss_args* a);
 int pfs_loss_bwd(const pfs_loss_args* a);
 int pfs_loss_shard_fwd(const pfs_loss_args* a);
 int pfs_loss_shard_merge(const pfs_loss_args* a);
+int pfs_loss_list_shard_fwd(const pfs_loss_args* a);     /* ABI 11 */
+int pfs_loss_list_shard_bwd(const pfs_loss_args* a);     /* ABI 11 */
 
 #ifdef __cplusplus
 }

@@ -18,7 +18,7 @@ HEADER = os.path.join(os.path.dirname(_HERE), "include", "pfs_b200.h")
 PFS_LAYOUT_DENSE = 0
 PFS_LAYOUT_CSR = 1
 PFS_TILE_EDGES = 256
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 _P = ct.c_void_p
 
@@ -133,7 +133,7 @@ class LossArgs(ct.Structure):
         [("S_total", ct.c_int32), ("world", ct.c_int32), ("shard_record", _P), ("shard_records", _P)] + \
         [("E", ct.c_int32)] + [(n, _P) for n in "csr_rowptr csr_eid csr_src csr_tgt csc_colptr csc_q cell_time".split()]
 # ABI 8 appended the graph dimension (G, class_tables), ABI 9 the fibre-sharded graph (S_total ... shard_records),
-# ABI 10 the edge list (E ... cell_time)
+# ABI 10 the edge list (E ... cell_time); ABI 11 adds functions only
 
 
 class WideSegments(ct.Structure):
@@ -200,6 +200,8 @@ SYMBOLS = {
     "pfs_loss_bwd": (ct.c_int, [ct.POINTER(LossArgs)]),
     "pfs_loss_shard_fwd": (ct.c_int, [ct.POINTER(LossArgs)]),
     "pfs_loss_shard_merge": (ct.c_int, [ct.POINTER(LossArgs)]),
+    "pfs_loss_list_shard_fwd": (ct.c_int, [ct.POINTER(LossArgs)]),      # ABI 11: an edge list sharded over fibre ranges
+    "pfs_loss_list_shard_bwd": (ct.c_int, [ct.POINTER(LossArgs)]),
     "pfs_wide_transpose": (ct.c_int, [_P, _I32, _I32, _I64, _P, _P]),
 }
 _SIZEOF_CHECKS = {

@@ -21,6 +21,11 @@
 // pass in CSR order, fibre sums, one CTA per class over its CSC list, the loss tail) and one backward kernel; a class
 // segment is cut into chunks by its length alone and the chunks are combined in a fixed tree, so the results do not
 // depend on G or on a graph's position in the batch.
+//
+// An edge list sharded over fibre ranges (ABI 11): a cell c_ki belongs to fibre k alone, so each shard runs the edge pass,
+// fibre sums and class pass on its own edges with its own S, and k_loss_list_shard_record writes the record of
+// k_loss_shard_record from the class pass's totals (zero cells over the local fibres included); k_loss_shard_merge combines
+// the records unchanged.  The backward is k_loss_list_edge_bwd with the variance taken over S_total fibres.
 #include <cstdarg>
 #include <cstdio>
 #include <math_constants.h>
@@ -514,8 +519,26 @@ __global__ void __launch_bounds__(1024) k_loss_list_scalars(const LossConst c, c
               counts, n_prime, class_mean, class_coef, scalars, red, &s_min);
 }
 
-// g_time of k_loss_edge_bwd per edge in CSR order, with the edge's cell value in place of its time2
-__global__ void __launch_bounds__(256) k_loss_list_edge_bwd(LossConst c, const ListTopo t, const float* __restrict__ time,
+// Sharded edge list, phase 1 (one graph, one CTA): this shard's record [2 + 3T] doubles from the class pass's totals over
+// its S local fibres (zero cells included) = {S, local fibre-penalty sum in the order of k_loss_list_scalars, the stats
+// rows}.  The record means what k_loss_shard_record's does, so k_loss_shard_merge combines it unchanged.
+__global__ void __launch_bounds__(1024) k_loss_list_shard_record(const LossConst c, const double* __restrict__ stats,
+                                                                 const float* __restrict__ fibre_time,
+                                                                 double* __restrict__ record) {
+    __shared__ double red[1024];
+    const int T = c.T;
+    for (int i = threadIdx.x; i < 3 * T; i += blockDim.x) record[2 + i] = stats[i];
+    const double fpen = fibre_penalty_sum(c, fibre_time, red);
+    if (threadIdx.x == 0) {
+        record[0] = (double)c.S;
+        record[1] = fpen;
+    }
+}
+
+// g_time of k_loss_edge_bwd per edge in CSR order, with the edge's cell value in place of its time2; S_var: the fibres the
+// variance runs over (S, or S_total of a sharded edge list)
+__global__ void __launch_bounds__(256) k_loss_list_edge_bwd(LossConst c, int S_var, const ListTopo t,
+                                                            const float* __restrict__ time,
                                                             const float* __restrict__ noise, const float* __restrict__ hours,
                                                             const float* __restrict__ cell_time,
                                                             const float* __restrict__ fibre_time,
@@ -524,7 +547,7 @@ __global__ void __launch_bounds__(256) k_loss_list_edge_bwd(LossConst c, const L
                                                             const float* __restrict__ g_loss, float* __restrict__ g_time) {
     resolve_sharpness(c);
     const long long n = (long long)c.G * t.E;
-    const float vscale = 2.f * c.wvar / (float)(c.S - 1);
+    const float vscale = 2.f * c.wvar / (float)(S_var - 1);
     for (long long x = (long long)blockIdx.x * blockDim.x + threadIdx.x; x < n; x += (long long)gridDim.x * blockDim.x) {
         const int g = c.G > 1 ? (int)(x / t.E) : 0;
         const long long p = x - (long long)g * t.E;
@@ -556,9 +579,14 @@ int list_topo(const pfs_loss_args& a, ListTopo& t) {
     return PFS_OK;
 }
 
-int make_const(const pfs_loss_args& a, LossConst& c) {
+// list_shard: the caller is pfs_loss_list_shard_fwd / _bwd (one shard of an edge list, E > 0 and S_total checked there)
+int make_const(const pfs_loss_args& a, LossConst& c, bool list_shard = false) {
     L_REQUIRE(a.E >= 0, "loss: negative edge count E");
-    if (a.E > 0) {           // an edge list: nothing of size S*T is stored
+    if (list_shard) {        // one shard of an edge list: the graph needs 2 fibres, the shard 1
+        L_REQUIRE(a.S >= 1 && a.S_total >= 2 && a.S <= a.S_total && a.T >= 1,
+                  "loss: bad edge-list shard sizes (at least 1 local fibre, 2 over all shards, S <= S_total)");
+        L_REQUIRE(a.G == 0 || a.G == 1, "loss: a sharded graph is one graph per call (G 0 or 1)");
+    } else if (a.E > 0) {    // an edge list: nothing of size S*T is stored
         L_REQUIRE(a.S_total == 0, "loss: an edge list (E > 0) cannot be fibre-sharded; S_total must be 0");
         L_REQUIRE(a.S >= 2 && a.T >= 1, "loss: bad edge-list sizes (at least 2 fibres and 1 class)");
     } else if (a.S_total) {         // one shard of a graph: the graph needs 2 fibres, the shard 1
@@ -611,26 +639,54 @@ int loss_edges_and_partials(const pfs_loss_args* a, const LossConst& c, cudaStre
     return PFS_OK;
 }
 
-// the edge-list forward (E > 0): edge pass, fibre sums, class pass, tail (4 launches)
-int loss_list_fwd(const pfs_loss_args* a, const LossConst& c, cudaStream_t st) {
+// the edge pass, the fibre sums and the class pass of an edge list (pfs_loss_fwd with E > 0, pfs_loss_list_shard_fwd);
+// the class pass's totals [G][3][T] go to *stats
+int loss_list_edges_and_classes(const pfs_loss_args* a, const LossConst& c, cudaStream_t st, double** stats) {
     ListTopo t;
     if (int rc = list_topo(*a, t)) return rc;
     L_REQUIRE((long long)c.G * c.T < (1ll << 31), "loss: too many graphs x classes for one launch (G*T < 2^31)");
     if (a->workspace_bytes < (size_t)c.G * 3 * c.T * sizeof(double) + 256)
         return lfail(PFS_ERR_WORKSPACE, "loss: workspace too small (%zu bytes for %d graph(s) of an edge list)",
                      a->workspace_bytes, c.G);
-    double* stats = (double*)(((uintptr_t)a->workspace + 255) & ~(uintptr_t)255);
+    *stats = (double*)(((uintptr_t)a->workspace + 255) & ~(uintptr_t)255);
     const long long GS = (long long)c.G * c.S;
     k_loss_list_edge_fwd<<<edge_grid(c.G * t.E), 256, 0, st>>>(c, t, a->time, a->noise, a->hours, a->galaxies, a->time2);
     L_LAUNCH_CHECK("k_loss_list_edge_fwd");
     k_loss_list_fibre_sums<<<(unsigned)((GS * 32 + 255) / 256), 256, 0, st>>>(c.S, t, GS, a->time2, a->fibre_time);
     L_LAUNCH_CHECK("k_loss_list_fibre_sums");
-    k_loss_list_class<<<c.G * c.T, 256, 0, st>>>(c.S, c.T, t, a->galaxies, a->time2, a->cell_time, stats);
+    k_loss_list_class<<<c.G * c.T, 256, 0, st>>>(c.S, c.T, t, a->galaxies, a->time2, a->cell_time, *stats);
     L_LAUNCH_CHECK("k_loss_list_class");
+    return PFS_OK;
+}
+
+// the edge-list forward (E > 0): edge pass, fibre sums, class pass, tail (4 launches)
+int loss_list_fwd(const pfs_loss_args* a, const LossConst& c, cudaStream_t st) {
+    double* stats;
+    if (int rc = loss_list_edges_and_classes(a, c, st, &stats)) return rc;
     k_loss_list_scalars<<<c.G, 1024, 0, st>>>(c, stats, a->counts, a->fibre_time, a->n_prime, a->class_mean, a->class_coef,
                                               a->scalars);
     L_LAUNCH_CHECK("k_loss_list_scalars");
     return PFS_OK;
+}
+
+// the per-edge backward of an edge list (1 launch), the variance over S_var fibres
+int loss_list_bwd(const pfs_loss_args* a, const LossConst& c, int S_var, cudaStream_t st) {
+    ListTopo t;
+    if (int rc = list_topo(*a, t)) return rc;
+    k_loss_list_edge_bwd<<<edge_grid(c.G * t.E), 256, 0, st>>>(c, S_var, t, a->time, a->noise, a->hours, a->cell_time,
+                                                               a->fibre_time, a->class_mean, a->class_coef, a->g_loss,
+                                                               a->g_time);
+    L_LAUNCH_CHECK("k_loss_list_edge_bwd");
+    return PFS_OK;
+}
+
+// the arguments of pfs_loss_list_shard_fwd / _bwd, all checked before any CUDA call
+int list_shard_args(const pfs_loss_args* a, const char* who, LossConst& c) {
+    if (a->E <= 0) return lfail(PFS_ERR_ARG, "%s: E (edges of this shard) must be > 0", who);
+    if (a->S_total <= 0) return lfail(PFS_ERR_ARG, "%s: S_total (fibres over all shards) is not set", who);
+    ListTopo t;
+    if (int rc = list_topo(*a, t)) return rc;
+    return make_const(*a, c, true);
 }
 
 }  // namespace
@@ -697,21 +753,37 @@ int pfs_loss_bwd(const pfs_loss_args* a) {
     if (int rc = make_const(*a, c)) return rc;
     cudaStream_t st = (cudaStream_t)a->stream;
     pfs_host::mark_launch(nullptr, st);
-    if (a->E > 0) {
-        ListTopo t;
-        if (int rc = list_topo(*a, t)) return rc;
-        k_loss_list_edge_bwd<<<edge_grid(c.G * t.E), 256, 0, st>>>(c, t, a->time, a->noise, a->hours, a->cell_time,
-                                                                   a->fibre_time, a->class_mean, a->class_coef, a->g_loss,
-                                                                   a->g_time);
-        L_LAUNCH_CHECK("k_loss_list_edge_bwd");
-        return PFS_OK;
-    }
+    if (a->E > 0) return loss_list_bwd(a, c, c.S, st);
     const int S_var = a->S_total ? a->S_total : c.S;
     k_loss_edge_bwd<<<edge_grid((long long)c.G * c.S * c.T), 256, 0, st>>>(c, S_var, a->time, a->noise, a->hours, a->time2,
                                                                     a->fibre_time, a->class_mean, a->class_coef, a->g_loss,
                                                                     a->g_time);
     L_LAUNCH_CHECK("k_loss_edge_bwd");
     return PFS_OK;
+}
+
+int pfs_loss_list_shard_fwd(const pfs_loss_args* a) {
+    L_REQUIRE(a && a->time && a->noise && a->hours && a->galaxies && a->time2 && a->fibre_time && a->shard_record &&
+                  a->workspace, "null pointer");
+    LossConst c;
+    if (int rc = list_shard_args(a, "pfs_loss_list_shard_fwd", c)) return rc;
+    cudaStream_t st = (cudaStream_t)a->stream;
+    pfs_host::mark_launch(nullptr, st);
+    double* stats;
+    if (int rc = loss_list_edges_and_classes(a, c, st, &stats)) return rc;
+    k_loss_list_shard_record<<<1, 1024, 0, st>>>(c, stats, a->fibre_time, a->shard_record);
+    L_LAUNCH_CHECK("k_loss_list_shard_record");
+    return PFS_OK;
+}
+
+int pfs_loss_list_shard_bwd(const pfs_loss_args* a) {
+    L_REQUIRE(a && a->time && a->noise && a->hours && a->fibre_time && a->class_mean && a->class_coef && a->g_time,
+              "null pointer");
+    LossConst c;
+    if (int rc = list_shard_args(a, "pfs_loss_list_shard_bwd", c)) return rc;
+    cudaStream_t st = (cudaStream_t)a->stream;
+    pfs_host::mark_launch(nullptr, st);
+    return loss_list_bwd(a, c, a->S_total, st);
 }
 
 }  // extern "C"

@@ -25,8 +25,11 @@ Inside `shard.fibre_sharded()` (one graph whose fibres are split over the ranks,
 compute the loss of the WHOLE graph on every rank from the rank's own fibres: each rank reduces its fibres to a record
 of 2 + 3T doubles, one all-reduce makes every record visible to every rank, and a merge in rank order gives every rank
 bitwise the same class statistics, scalars and loss.  The gradient w.r.t. the local edge times is that of the global
-loss, so the Blocks' gradient all-reduces sum the parts of one function.
+loss, so the Blocks' gradient all-reduces sum the parts of one function.  The graph is a slab of the canonical order, or
+an edge list split by `shard.partition_fibres` whose `edge_ids` (the global positions of the rank's edges) are passed in:
+every cell c_ki lies on the rank that owns fibre k, so the records need no other exchange.
 """
+import collections
 import ctypes as ct
 
 import torch
@@ -45,7 +48,9 @@ class LossFunction(torch.autograd.Function):
     S_total > 0: this rank's S fibres of a graph of S_total fibres sharded over the active group (G = 0): the forward is
     pfs_loss_shard_fwd, the record exchange (shard.exchange_rows) and pfs_loss_shard_merge.
     edges: None (canonical order, E = S*T) or an edge list {"E": edges per graph, and the int32 CSR / CSC arrays of
-    Topology.csr()}; the forward saves the per-edge cell values for the backward."""
+    Topology.csr()}; the forward saves the per-edge cell values for the backward.  An edge list with S_total > 0 is this
+    rank's edges of a sharded edge list: pfs_loss_list_shard_fwd, the exchange and pfs_loss_shard_merge, and the backward
+    pfs_loss_list_shard_bwd."""
 
     @staticmethod
     def forward(ctx, time, noise, hours, counts, G, S, T, consts, S_total, edges=None):
@@ -88,9 +93,14 @@ class LossFunction(torch.autograd.Function):
             if S_total:
                 record = torch.empty(2 + 3 * T, dtype=torch.float64, device=dev)
                 a.S_total, a.world, a.shard_record = S_total, _shard.world_size(), record.data_ptr()
-                _abi.check(lib.pfs_loss_shard_fwd(ct.byref(a)), "pfs_loss_shard_fwd")
+                fwd = "pfs_loss_shard_fwd" if edges is None else "pfs_loss_list_shard_fwd"
+                _abi.check(getattr(lib, fwd)(ct.byref(a)), fwd)
                 records = _shard.exchange_rows(record)                  # [world, 2 + 3T], rank order, on every rank
                 a.shard_records = records.data_ptr()
+                if edges is not None:                 # the merge reads the records alone: E = 0, no edge arrays
+                    a.E = 0
+                    for k in _EDGE_ARRAYS + ("cell_time",):
+                        setattr(a, k, None)
                 _abi.check(lib.pfs_loss_shard_merge(ct.byref(a)), "pfs_loss_shard_merge")
             else:
                 _abi.check(lib.pfs_loss_fwd(ct.byref(a)), "pfs_loss_fwd")
@@ -121,7 +131,8 @@ class LossFunction(torch.autograd.Function):
         a.sharpness_dev = _abi.ptr(ctx.consts.get("sharpness_dev"))
         with torch.cuda.device(dev):
             a.stream = torch.cuda.current_stream(dev).cuda_stream
-            _abi.check(_abi.load_library().pfs_loss_bwd(ct.byref(a)), "pfs_loss_bwd")
+            bwd = "pfs_loss_list_shard_bwd" if ctx.edges is not None and ctx.S_total else "pfs_loss_bwd"
+            _abi.check(getattr(_abi.load_library(), bwd)(ct.byref(a)), bwd)
         return g_time, None, None, None, None, None, None, None, None, None
 
 
@@ -141,6 +152,31 @@ def _edge_list(edge_index, S, T):
     topo = get_topology(edge_index, S, T)
     arrays = topo.csr()
     return dict(E=topo.E, **{k: arrays[k] for k in _EDGE_ARRAYS})
+
+
+_EDGE_IDS_CHECKED = collections.OrderedDict()
+
+
+def _check_edge_ids(edge_ids, E, E_total, device):
+    """`edge_ids` of a sharded edge list: 1-D int64 on `device`, one per local edge, every value in [0, E_total).  The
+    range is read once per tensor (one host synchronisation) and remembered, like a Topology: an index out of range would
+    fault the device in the noise gather."""
+    if not torch.is_tensor(edge_ids) or edge_ids.dtype != torch.int64 or edge_ids.dim() != 1 or edge_ids.device != device:
+        raise _abi.PfsError("loss: edge_ids are the global positions of this rank's edges, a 1-D int64 tensor on %s; got %s"
+                            % (device, (edge_ids.dtype, tuple(edge_ids.shape), str(edge_ids.device))
+                               if torch.is_tensor(edge_ids) else type(edge_ids).__name__))
+    if edge_ids.numel() != E:
+        raise _abi.PfsError("loss: edge_ids has %d entries for %d local edges" % (edge_ids.numel(), E))
+    key = (edge_ids.data_ptr(), edge_ids._version, E, E_total, str(device))
+    if key in _EDGE_IDS_CHECKED:
+        _EDGE_IDS_CHECKED.move_to_end(key)
+        return
+    lo, hi = torch.stack([edge_ids.min(), edge_ids.max()]).tolist()
+    if lo < 0 or hi >= E_total:
+        raise _abi.PfsError("loss: edge_ids out of range [%d, %d] for %d edges over all shards" % (lo, hi, E_total))
+    _EDGE_IDS_CHECKED[key] = edge_ids             # keeps the tensor alive, so its address cannot be recycled under the key
+    while len(_EDGE_IDS_CHECKED) > 16:
+        _EDGE_IDS_CHECKED.popitem(last=False)
 
 
 def _graph_rows(x, E):
@@ -177,7 +213,7 @@ def _batched_loss(time, class_info, S, T, nfields, consts, noise, edges=None):
 
 
 def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=42, wutils=2000.0, wvar=1.0, pclass=0.1,
-                    pfiber=1.0, sharpness=0.5, noise=None, edge_index=None):
+                    pfiber=1.0, sharpness=0.5, noise=None, edge_index=None, edge_ids=None):
     """Loss terms from the edge times [E] (or [E,1]); returns (loss, scalars, n_prime, fibre_time, time2) where
     scalars = [loss, totutils, class_penalty, fibre_penalty, variance, #minima, 0, 0].
 
@@ -196,8 +232,16 @@ def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=
 
     `edge_index` [2, E] (int64, on the device): the edges in any order, edge e = (fibre edge_index[0, e], class
     edge_index[1, e]); `time` is [E], [E, 1], [G, E] or [G, E, 1] in that order, and so are `noise` and time2.  None:
-    the canonical dense order e = k*T + i.  An edge list is not fibre-sharded: inside `shard.fibre_sharded()` it is
-    refused."""
+    the canonical dense order e = k*T + i.
+
+    `edge_ids` [E] (int64, on the device; only inside `shard.fibre_sharded()`): this rank's edges of an edge list sharded
+    over fibre ranges are `edge_index` (local fibres numbered from 0, `nfibers` of them) and their positions in the whole
+    graph's edge list are `edge_ids` -- the second and third values of `shard.partition_fibres`.  As for the canonical
+    sharded graph, the loss, scalars and n_prime are those of the whole graph (bitwise the same on every rank), fibre_time
+    the local rows and time2 the local edges in local order.  Without `noise` the whole edge list's draws are made by one
+    torch.rand and this rank takes [edge_ids], so a run seeded alike on every rank draws bitwise the noise of the
+    single-GPU run.  Every rank of the group must pass `edge_ids` (or none may): the path decides which collectives run.
+    Inside the scope an edge list without `edge_ids` is refused; outside it, `edge_ids` is."""
     consts = dict(total_time=total_time, wutils=wutils, wvar=wvar, pclass=pclass, pfiber=pfiber, noiselevel=NOISELEVEL)
     if torch.is_tensor(sharpness):                # device scalar: the value is read by the kernels (CUDA-graph replays)
         consts.update(sharpness=0.0, sharpness_dev=sharpness.to(torch.float32).reshape(1))
@@ -206,10 +250,17 @@ def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=
     nfibers, nclasses = int(nfibers), int(nclasses)
     sharded = _shard.active()
     edges = None
+    if edge_ids is not None:
+        if not sharded:
+            raise _abi.PfsError("loss: edge_ids (the global positions of a shard's edges) are only taken inside "
+                                "shard.fibre_sharded(); outside it there is no shard")
+        if edge_index is None:
+            raise _abi.PfsError("loss: edge_ids are the global positions of the edges of edge_index, which is missing")
     if edge_index is not None:
-        if sharded:
-            raise _abi.PfsError("loss: an edge list cannot be fibre-sharded: the sharded loss splits the canonical order "
-                                "e = k*T + i into contiguous fibre ranges")
+        if sharded and edge_ids is None:
+            raise _abi.PfsError("loss: an edge list cannot be fibre-sharded without the global positions of its edges: the "
+                                "canonical sharded loss splits the order e = k*T + i into contiguous fibre ranges; pass "
+                                "edge_ids from shard.partition_fibres")
         edges = _edge_list(edge_index, nfibers, nclasses)
     E = nfibers * nclasses if edges is None else edges["E"]
     if time.dim() == 3 or (time.dim() == 2 and time.shape[1] == E):
@@ -220,8 +271,13 @@ def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=
     if time.dtype != torch.float32:
         time = time.float()                       # bf16 head output: dtype plumbing, the loss itself is fp32
     S_total = _shard.total_count(nfibers) if sharded else 0      # cached: no host synchronisation per step
+    if edge_ids is not None:
+        E_total = _shard.total_count(E, kind="edges")                # cached apart from the fibre counts
+        _check_edge_ids(edge_ids, E, E_total, time.device)
     if noise is None:
-        if sharded:                               # the whole graph's draw, this rank's slice
+        if edge_ids is not None:                  # the whole edge list's draw, this rank's edges
+            noise = torch.rand(E_total, dtype=torch.float32, device=time.device)[edge_ids]
+        elif sharded:                             # the whole graph's draw, this rank's slice
             f0 = sum(_shard.shard_counts(nfibers)[:_shard.rank()])       # cached like S_total
             noise = torch.rand(S_total * nclasses, dtype=torch.float32, device=time.device)
             noise = noise[f0 * nclasses:(f0 + nfibers) * nclasses]
@@ -234,14 +290,20 @@ def loss_from_times(time, class_info, nfibers, nclasses, nfields=10, total_time=
 
 
 def loss_function(gnn, graph, class_info, pclass=0.1, pfiber=1.0, sharpness=0.5, finaloutput=False, *, nfibers=None,
-                  nclasses=None, nfields=10, total_time=42, wutils=2000.0, wvar=1.0, noise=None, reduction="sum"):
+                  nclasses=None, nfields=10, total_time=42, wutils=2000.0, wvar=1.0, noise=None, reduction="sum",
+                  edge_ids=None):
     """reference src/train.py:29-80 with its globals as arguments (`gnn` first; NFIBERS / NCLASSES default to the
     graph's node counts).
 
     On a collated batch (`Loader.collate`: x_e [G, E, F]) `class_info` is [T, 2] or [G, T, 2] and `noise` [G, E];
     returns (loss, utilities [G]) where loss is the sum of the G per-graph losses (`reduction="sum"`: the parameter
     gradients are those of the G single-graph losses backpropagated one after the other, as the Block sums them over
-    graphs) or their mean (`"mean"`).  With `finaloutput=True` every per-graph diagnostic carries the leading G."""
+    graphs) or their mean (`"mean"`).  With `finaloutput=True` every per-graph diagnostic carries the leading G.
+
+    Inside `shard.fibre_sharded()`, `edge_ids` (the third value of `shard.partition_fibres`) makes the graph this rank's
+    part of an edge list sharded over fibre ranges: the loss takes the edge-list path of `loss_from_times` even where the
+    rank's local edge_index happens to be canonical (a complete slab of a sparse graph), so every rank of the group runs
+    the same collectives."""
     from .topology import get_topology
     if reduction not in ("sum", "mean"):
         raise ValueError("loss_function: reduction is 'sum' or 'mean', got %r" % (reduction,))
@@ -250,15 +312,17 @@ def loss_function(gnn, graph, class_info, pclass=0.1, pfiber=1.0, sharpness=0.5,
     nfibers = int(nfibers if nfibers is not None else graph.x_s.shape[-2])
     topo = get_topology(graph.edge_index, nfibers, nclasses)
     edge_index = None
-    if not topo.canonical:
+    if edge_ids is not None:
+        edge_index = graph.edge_index           # one shard of an edge list, canonical or not (loss_from_times checks)
+    elif not topo.canonical:
         if _shard.active():
             raise _abi.PfsError("loss: a fibre-sharded graph needs the canonical dense edge order e = k*T + i, because the "
                                 "sharded loss splits that order into contiguous fibre ranges; this graph's edge_index is "
-                                "not canonical")
+                                "not canonical (pass edge_ids from shard.partition_fibres to train an edge list)")
         edge_index = graph.edge_index           # any edge list: the cell-matrix loss of DESIGN.md section 8b
     time = gnn.edge_prediction(graph.x_e, scale=total_time / nclasses).squeeze(-1)
     loss, sc, n_prime, fibre_time, time2 = loss_from_times(time, class_info, nfibers, nclasses, nfields, total_time, wutils,
-                                                            wvar, pclass, pfiber, sharpness, noise, edge_index)
+                                                            wvar, pclass, pfiber, sharpness, noise, edge_index, edge_ids)
     if batched:
         loss = loss.sum() if reduction == "sum" else loss.mean()
     if not finaloutput:

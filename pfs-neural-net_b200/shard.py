@@ -106,15 +106,17 @@ def exchange_rows(row):
     return buf
 
 
-def shard_counts(n_local):
+def shard_counts(n_local, kind=None):
     """Per-shard values of a host-known integer (rows or edges of this shard), as a tuple indexed by rank.  The
     exchange (the only host synchronisation of the sharded path) runs ONCE per distinct local value inside a
     fibre_sharded() scope family: shard sizes are properties of the partition, not of the step.  The cache is keyed by
     (group, local value), and a miss is a collective, so all ranks must miss together: run a partition with other shard
-    sizes (another graph) in a group of its own when some rank's local value could repeat an earlier one."""
+    sizes (another graph) in a group of its own when some rank's local value could repeat an earlier one.
+    `kind` (e.g. "edges") counts under a cache key of its own, so a rank whose edge count equals its fibre count (or
+    any count of another kind cached earlier) still misses together with the other ranks."""
     if not active():
         return (int(n_local),)
-    key = (id(_state["group"]), int(n_local))
+    key = (id(_state["group"]), int(n_local)) if kind is None else (id(_state["group"]), kind, int(n_local))
     hit = _state["counts"].get(key)
     if hit is None:
         world, rank = dist.get_world_size(_state["group"]), dist.get_rank(_state["group"])
@@ -130,9 +132,9 @@ def shard_counts(n_local):
     return hit
 
 
-def total_count(n_local):
-    """Sum of a per-shard integer over the shards (host int, cached like shard_counts)."""
-    return sum(shard_counts(n_local))
+def total_count(n_local, kind=None):
+    """Sum of a per-shard integer over the shards (host int, cached like shard_counts, under `kind`)."""
+    return sum(shard_counts(n_local, kind))
 
 
 def allreduce_moments(n, mean, m2):
@@ -159,7 +161,8 @@ def partition_fibres(edge_index, S, world, rank):
     canonical order and needs no index work).  Rank r owns the fibres [S*r/world, S*(r+1)/world) and every edge
     whose source lies in that range, in the order the edge list has them.
     Returns (local edge_index [2, E_r] with fibres renumbered from 0, fibre slice, positions of the kept edges in
-    the global edge list -- use them to slice x_e / to scatter results back)."""
+    the global edge list -- use them to slice x_e / to scatter results back, and pass them as the `edge_ids` of
+    loss.loss_function / TrainStep to train the sharded edge list)."""
     f0, f1 = (S * rank) // world, (S * (rank + 1)) // world
     src = edge_index[0]
     keep = torch.nonzero((src >= f0) & (src < f1)).flatten()

@@ -20,7 +20,8 @@ copies the next batch of the same shapes and topology into the step's input tens
 `Loader.batches(G)` replays the one captured graph.
 
 Inside `shard.fibre_sharded()` (one graph split over the ranks by fibre ranges) the step runs eager only
-(`use_graph=False`): its all-reduces are not captured into a CUDA graph.
+(`use_graph=False`): its all-reduces are not captured into a CUDA graph.  `edge_ids` (from `shard.partition_fibres`)
+makes the step's graph one rank's part of a sharded edge list (loss.loss_function).
 """
 import torch
 
@@ -30,16 +31,17 @@ from . import shard as _shard
 
 class TrainStep:
     def __init__(self, model, graph, class_info, optimizer, *, pclass=0.1, pfiber=1.0, nfields=10, total_time=42,
-                 wutils=2000.0, wvar=1.0, use_graph=True, warmup=3, noise=None):
+                 wutils=2000.0, wvar=1.0, use_graph=True, warmup=3, noise=None, edge_ids=None):
         """`noise`: optional static device tensor [E] (a batch: [G, E]) of softfloor draws in [0, 1) (reference
         src/train.py:22); the caller refills it (copy_) before a step to control the draw.  None: torch.rand_like per
         step, as the reference.  The tensors of `graph` and `class_info` are the step's static inputs: `load()`
-        overwrites them in place."""
+        overwrites them in place.  `edge_ids`: inside `shard.fibre_sharded()`, the global positions of the graph's
+        edges in a sharded edge list (see loss.loss_function)."""
         self.model, self.graph, self.class_info, self.opt = model, graph, class_info, optimizer
         self.kw = dict(pclass=pclass, pfiber=pfiber, nfields=nfields, total_time=total_time, wutils=wutils, wvar=wvar)
         dev = class_info.device
         self.sharp = torch.zeros(1, dtype=torch.float32, device=dev)
-        self.noise = noise
+        self.noise, self.edge_ids = noise, edge_ids
         self.loss = self.utility = None
         self._graph = None
         if use_graph:
@@ -88,7 +90,7 @@ class TrainStep:
         self.opt.zero_grad(set_to_none=True)
         out = self.model(self.graph)
         self.loss, self.utility = _loss.loss_function(self.model, out, self.class_info, sharpness=self.sharp,
-                                                      noise=self.noise, **self.kw)
+                                                      noise=self.noise, edge_ids=self.edge_ids, **self.kw)
         self.loss.backward()
         self.opt.step()
 
