@@ -454,6 +454,21 @@ int bn_forward_tail(int F, int G, long long rows, const float* partial, int ntil
     }
     return PFS_OK;
 }
+// BatchNorm-backward sums over the rows of each graph: out[g] = (sum g, sum g xhat) [G][2F]; partial: G * 64 * 2F floats
+int bn_bwd_stats(const float* gout, const float* y, const float* save, int rows, int F, int G, float eps, float* partial,
+                 float* out, cudaStream_t st) {
+    int nchunk = (rows + 4095) / 4096;           // one CTA per 4096 rows of a graph (1 for the C3 graphs)
+    if (nchunk > 64) nchunk = 64;
+    constexpr int kStatThreads = 1024;           // ~100 row lanes per CTA: few rows, many loads in flight per lane
+    k_bn_bwd_stats_rows<<<dim3(nchunk, G), kStatThreads, sizeof(float) * 2 * kStatThreads, st>>>(
+        gout, y, save, rows, F, eps, nchunk, nchunk > 1 ? partial : out);
+    PFS_LAUNCH_CHECK("k_bn_bwd_stats_rows");
+    if (nchunk > 1) {
+        k_bn_bwd_stats_final<<<(G * 2 * F + 127) / 128, 128, 0, st>>>(partial, nchunk, 2 * F, G, out);
+        PFS_LAUNCH_CHECK("k_bn_bwd_stats_final");
+    }
+    return PFS_OK;
+}
 int affine_rows(const float* in, const float* save, int F, long long rows, int G, float* out, cudaStream_t st) {
     const long long per_graph = rows * F / 2;
     if (per_graph == 0) return PFS_OK;
@@ -533,17 +548,23 @@ int edge_bwd_impl(const pfs_edge_args& a, const Topo& tp) {
     // k_edge_bwd2 (two CTAs per SM: x_e staged only, hidden layer in two halves, shared accumulator registers) where
     // its tiles fit 113 KB, else the double-buffered one-CTA-per-SM k_edge_bwd (Fdim 16).
     // Measured at C3: 1.21 ms against 1.60 ms.
-    constexpr bool lean = SM::lean_fits;
+    // Where the staged tiles of k_edge_bwd do not fit either (Fdim 16 with up to 256 short fibres per tile: an edge
+    // list of 72 fibres or more), k_edge_bwd2 runs at one CTA per SM.
     const bool split = tp.nsplit > 0;
-    auto kern = lean ? (split ? k_edge_bwd2<F, true> : k_edge_bwd2<F>) : (split ? k_edge_bwd<F, true> : k_edge_bwd<F>);
     const int max_fib = max_fibres_per_tile(tp);
     const bool sc = stage_class_table(tp, H);
     size_t smem_bwd = SM::bytes_lean;
     int nbuf = 1;
+    bool lean = SM::lean_fits;
     if (!lean) {
         nbuf = pick_nbuf([&](int nb) { return SM::bytes(max_fib, tp.T, sc, nb); }, smem_bwd);
-        if (!nbuf) return fail(PFS_ERR_UNSUPPORTED, "edge_bwd: tile staging does not fit shared memory");
+        if (!nbuf) {
+            lean = true;
+            nbuf = 1;
+            smem_bwd = SM::bytes_lean;
+        }
     }
+    auto kern = lean ? (split ? k_edge_bwd2<F, true> : k_edge_bwd2<F>) : (split ? k_edge_bwd<F, true> : k_edge_bwd<F>);
     PFS_TRY(allow_smem(kern, smem_bwd));
     const int grid = persistent_grid(kern, smem_bwd, total);
     constexpr int pstride = 2 * H * F + F;
@@ -757,16 +778,7 @@ int source_bwd_impl(const pfs_source_args& a, const Topo& tp) {
         PFS_TRY((run_prep<F, M>(tp.G, jobs, 1, a.w1, M, a.u, pl, nfloats, wstage, st)));
     }
     if (mode != 0) {
-        int nchunk = (tp.S + 4095) / 4096;           // one CTA per 4096 fibres of a graph (1 for the C3 graphs)
-        if (nchunk > 64) nchunk = 64;
-        constexpr int kStatThreads = 1024;           // ~100 row lanes per CTA: few rows, many loads in flight per lane
-        k_bn_bwd_stats_rows<<<dim3(nchunk, tp.G), kStatThreads, sizeof(float) * 2 * kStatThreads, st>>>(
-            a.g_out, a.y_pre, a.bn_save, tp.S, F, a.eps, nchunk, nchunk > 1 ? bnpart : bnstat);
-        PFS_LAUNCH_CHECK("k_bn_bwd_stats_rows");
-        if (nchunk > 1) {
-            k_bn_bwd_stats_final<<<(tp.G * 2 * F + 127) / 128, 128, 0, st>>>(bnpart, nchunk, 2 * F, tp.G, bnstat);
-            PFS_LAUNCH_CHECK("k_bn_bwd_stats_final");
-        }
+        PFS_TRY(bn_bwd_stats(a.g_out, a.y_pre, a.bn_save, tp.S, F, tp.G, a.eps, bnpart, bnstat, st));
         PFS_TRY(colsum_pair(bnstat, tp.G, 2 * F, F, a.g_gamma, 0, a.g_beta, F, st));
     }
     {
@@ -837,6 +849,9 @@ int target_fwd_impl(const pfs_target_args& a, const Topo& tp) {
     float* stage = ws.f(class_stage_floats(tp, M));
     float* cscs = ws.f(csc_scratch_floats(tp, M) + 1);
     float* wstage = ws.f(kConstFloats);
+    const bool tiled = tail_tiled(tp.T, F);
+    const int nt = tail_tiles(tp.T);
+    float* bnp = tiled ? ws.f((size_t)tp.G * nt * bn_partial_stride(F)) : nullptr;
     if (!ws.ok) return fail(PFS_ERR_WORKSPACE, "target_fwd: workspace too small (%zu B)", a.workspace_bytes);
     if (a.normed) PFS_REQUIRE(a.gamma && a.beta && a.bn_save, "normed target model needs gamma, beta, bn_save");
     if (a.normed && a.training && tp.T <= 1)
@@ -857,10 +872,25 @@ int target_fwd_impl(const pfs_target_args& a, const Topo& tp) {
         PFS_LAUNCH_CHECK("k_target_edge_fwd");
     }
     PFS_TRY(class_sums(tp, stage, M, a.act_sum, cscs, st));
+    if (tiled) {
+        // rows kernel, then the BatchNorm over the T rows from its per-tile records (the running buffers are updated
+        // there, once per graph in graph order) and the affine
+        TargetTailParams p = make_tail(a, tp);
+        p.bn_partial = bnp;
+        const size_t smem = tail_rows_smem(F);
+        PFS_TRY(allow_smem(k_target_tail_rows_fwd, smem));
+        k_target_tail_rows_fwd<<<dim3(nt, tp.G), kThreads, smem, st>>>(p);
+        PFS_LAUNCH_CHECK("k_target_tail_rows_fwd");
+        if (a.normed) {
+            PFS_TRY(bn_forward_tail(F, tp.G, tp.T, bnp, nt, 0, a.training, a.gamma, a.beta, a.running_mean, a.running_var,
+                                    (long long*)a.num_batches_tracked, a.eps, a.momentum, a.bn_save, st));
+            PFS_TRY(affine_rows(a.y_pre, a.bn_save, F, tp.T, tp.G, a.x_t_out, st));
+        }
+        return PFS_OK;
+    }
     {
         TargetTailParams p = make_tail(a, tp);
         const size_t smem = sizeof(float) * ((size_t)tp.T * 8 * F + 4 * F);
-        if (smem > 200 * 1024) return fail(PFS_ERR_UNSUPPORTED, "target tail: T*F too large for one CTA (%zu B)", smem);
         PFS_TRY(allow_smem(k_target_tail_fwd, smem));
         k_target_tail_fwd<<<tp.G, kThreads, smem, st>>>(p);
         PFS_LAUNCH_CHECK("k_target_tail_fwd");
@@ -886,37 +916,53 @@ int target_bwd_impl(const pfs_target_args& a, const Topo& tp) {
     const int gride = persistent_grid(ke, SM::bytes, total);
     constexpr int pstride_e = M * F;
     constexpr int ptail = tail_partial_floats(F);
+    const bool tiled = tail_tiled(tp.T, F);
+    const int nt = tiled ? tail_tiles(tp.T) : 1;           // parameter-gradient partials per graph
     Bump ws(a.workspace, a.workspace_bytes);
     const bool cached = a.table_s != nullptr;              // R_s kept by the forward: not recomputed
     float* Rs = cached ? a.table_s : ws.f((size_t)tp.G * tp.S * M);
     float* dasum = ws.f((size_t)tp.G * tp.T * M);
-    float* gpart = ws.f((size_t)tp.G * ptail);
+    float* gpart = ws.f((size_t)tp.G * nt * ptail);
+    float* bnstat = tiled ? ws.f((size_t)tp.G * 2 * F) : nullptr;
+    float* bnpart = tiled ? ws.f((size_t)tp.G * 64 * 2 * F) : nullptr;
     float* dRs = ws.f((size_t)tp.G * tp.S * M);
     float* wpe = ws.f((size_t)gride * pstride_e);
     float* opart = ws.f((size_t)kMaxCtas * (M * F + M));
     float* wstage = ws.f(kConstFloats);
     float* dRs_split = split ? ws.f((size_t)tp.G * tp.nslots * M) : nullptr;
     if (!ws.ok) return fail(PFS_ERR_WORKSPACE, "target_bwd: workspace too small (%zu B)", a.workspace_bytes);
-    {
-        TargetTailParams p = make_tail(a, tp);
-        p.dasum = dasum;
-        p.gpartial = gpart;
+    TargetTailParams p = make_tail(a, tp);
+    p.dasum = dasum;
+    p.gpartial = gpart;
+    if (tiled) {
+        if (p.mode != 0) PFS_TRY(bn_bwd_stats(a.g_out, a.y_pre, a.bn_save, tp.T, F, tp.G, a.eps, bnpart, bnstat, st));
+        p.bn_stat = bnstat;
+        const size_t smem = tail_rows_smem(F);
+        PFS_TRY(allow_smem(k_target_tail_rows_bwd, smem));
+        k_target_tail_rows_bwd<<<dim3(nt, tp.G), kThreads, smem, st>>>(p);
+        PFS_LAUNCH_CHECK("k_target_tail_rows_bwd");
+        k_target_tail_gu<<<(tp.G * F + 127) / 128, 128, 0, st>>>(gpart, nt, tp.G, F, a.w3, a.g_u);
+        PFS_LAUNCH_CHECK("k_target_tail_gu");
+    } else {
         const size_t smem = sizeof(float) * ((size_t)tp.T * 8 * F + 6 * F);
-        if (smem > 200 * 1024) return fail(PFS_ERR_UNSUPPORTED, "target tail: T*F too large for one CTA (%zu B)", smem);
         PFS_TRY(allow_smem(k_target_tail_bwd, smem));
         k_target_tail_bwd<<<tp.G, kThreads, smem, st>>>(p);
         PFS_LAUNCH_CHECK("k_target_tail_bwd");
     }
     Reducer rd;                       // all the final sums of this call go out in one launch at its end
     {
-        rd.source(gpart, tp.G, ptail);
+        rd.source(gpart, tp.G * nt, ptail);
         rd.add(tail_off_w2(F), M * M, M, a.g_w2, M, 0);
         rd.add(tail_off_b2(F), M, M, a.g_b2, M, 0);
         rd.add(tail_off_w3(F), H * H, H, a.g_w3, H, 0);
         rd.add(tail_off_b3(F), H, H, a.g_b3, H, 0);
         rd.add(tail_off_w4(F), F * H, H, a.g_w4, H, 0);
         rd.add(tail_off_b4(F), F, F, a.g_b4, F, 0);
-        if (a.normed) {
+        if (a.normed && tiled) {
+            rd.source(bnstat, tp.G, 2 * F);
+            rd.add(F, F, F, a.g_gamma, F, 0);
+            rd.add(0, F, F, a.g_beta, F, 0);
+        } else if (a.normed) {
             rd.add(tail_off_gamma(F), F, F, a.g_gamma, F, 0);
             rd.add(tail_off_beta(F), F, F, a.g_beta, F, 0);
         }
@@ -1156,6 +1202,8 @@ size_t pfs_workspace_bytes(const pfs_topology* t) {
     fl += G * (36 * F * F + 128 * F);
     fl += G * 64 * 2 * F + 64;                                   // chunk partials of the node BatchNorm backward sums
     if (t->nsplit > 0) fl += G * (size_t)t->nslots * (10 * F + 1) + 64;   // split tiles: chunk records / partial fibre sums
+    if (tail_tiled(t->T, t->F))                                   // class-tiled TModel tail: per-tile partials, BatchNorm-backward sums
+        fl += G * tail_tiles(t->T) * (tail_partial_floats(t->F) + bn_partial_stride(t->F)) + G * 65 * 2 * F;
     fl += 4096;
     return fl * sizeof(float) + 64 * 256;
 }

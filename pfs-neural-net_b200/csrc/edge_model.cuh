@@ -358,7 +358,8 @@ __global__ void __launch_bounds__(kThreads) k_edge_bwd(const EdgeBwdParams p) {
 }
 
 // ------------------------------------------------------------------------------------------
-// k_edge_bwd2: the same backward shaped for TWO CTAs per SM (<= 128 registers, 113 KB of shared memory):
+// k_edge_bwd2: the same backward shaped for TWO CTAs per SM (<= 128 registers, 113 KB of shared memory; at Fdim 16,
+// where its 170 KB allow one CTA per SM, it runs where k_edge_bwd's staged tiles do not fit and has all registers):
 //   * only x_e is staged (single buffer: it has to be in shared memory for dW1_e); the other per-edge rows and
 //     the node tables come straight from global / L1, the second resident CTA hides their latency;
 //   * the hidden layer is processed in two halves of 2F units (h, dh: 2F live registers each instead of 4F);
@@ -390,7 +391,7 @@ __device__ __forceinline__ void edge_bwd_half(const EdgeBwdParams& p, const floa
 }
 
 template <int F, bool SPLIT = false>
-__global__ void __launch_bounds__(kThreads, 2) k_edge_bwd2(const EdgeBwdParams p) {
+__global__ void __launch_bounds__(kThreads, EdgeBwdSmem<F>::lean_fits ? 2 : 1) k_edge_bwd2(const EdgeBwdParams p) {
     constexpr int H = 4 * F;
     using SM = EdgeBwdSmem<F>;
     using Stage = typename SM::StageLean;

@@ -80,7 +80,10 @@ struct TargetTailParams {
     float* g_x_t;                // [G,T,F] direct part
     float* g_u;                  // [G,F]
     float* dasum;                // [G,T,2F] gradient table gathered by the edge pass
-    float* gpartial;             // [G][tail_partial_floats(F)]
+    float* gpartial;             // [G][tail_partial_floats(F)], class-tiled: [G][tail_tiles(T)][tail_partial_floats(F)]
+    // class-tiled tail only
+    float* bn_partial;           // forward: [G][tail_tiles(T)][bn_partial_stride(F)] per-tile (mean, M2, count)
+    const float* bn_stat;        // backward: [G][2F] sum g, sum g xhat over the T rows
 };
 
 // layout of one graph's parameter-gradient partial (floats)
@@ -98,17 +101,19 @@ __device__ __forceinline__ float class_count(const TargetTailParams& p, int i) {
     return p.colptr ? (float)(p.colptr[i + 1] - p.colptr[i]) : (float)p.dense_count;
 }
 
-// shared by forward and backward: hcat = [x_t | agg], b3e = b3 + W3[:, 3F:] . u, a3 = lrelu(h3)
-__device__ __forceinline__ void tail_forward_core(const TargetTailParams& p, int g, float* HC, float* A3, float* b3e) {
+// shared by forward and backward: hcat = [x_t | agg], b3e = b3 + W3[:, 3F:] . u, a3 = lrelu(h3) for the n classes
+// r0 .. r0 + n - 1 of graph g (shared-memory row r holds class r0 + r)
+__device__ __forceinline__ void tail_forward_core(const TargetTailParams& p, int g, int r0, int n, float* HC, float* A3,
+                                                  float* b3e) {
     const int F = p.F, T = p.T, M = 2 * F, H = 4 * F, K3 = 3 * F;
-    for (int i = threadIdx.x; i < T * F; i += blockDim.x) {
+    for (int i = threadIdx.x; i < n * F; i += blockDim.x) {
         const int r = i / F, k = i - r * F;
-        HC[r * K3 + k] = p.x_t[((size_t)g * T + r) * F + k];
+        HC[r * K3 + k] = p.x_t[((size_t)g * T + r0 + r) * F + k];
     }
-    for (int i = threadIdx.x; i < T * M; i += blockDim.x) {
+    for (int i = threadIdx.x; i < n * M; i += blockDim.x) {
         const int r = i / M, j = i - r * M;
-        const float* a = p.act_sum + ((size_t)g * T + r) * M;
-        float s = class_count(p, r) * p.b2[j];
+        const float* a = p.act_sum + ((size_t)g * T + r0 + r) * M;
+        float s = class_count(p, r0 + r) * p.b2[j];
         for (int k = 0; k < M; ++k) s = fmaf(a[k], p.w2[j * M + k], s);
         HC[r * K3 + F + j] = s;
     }
@@ -118,7 +123,7 @@ __device__ __forceinline__ void tail_forward_core(const TargetTailParams& p, int
         b3e[j] = s;
     }
     __syncthreads();
-    for (int i = threadIdx.x; i < T * H; i += blockDim.x) {
+    for (int i = threadIdx.x; i < n * H; i += blockDim.x) {
         const int r = i / H, j = i - r * H;
         float s = b3e[j];
         for (int k = 0; k < K3; ++k) s = fmaf(HC[r * K3 + k], p.w3[j * H + k], s);
@@ -135,7 +140,7 @@ __global__ void __launch_bounds__(kThreads) k_target_tail_fwd(const TargetTailPa
     float* A3 = HC + T * K3;      // [T][4F]
     float* Y = A3 + T * H;        // [T][F]
     float* b3e = Y + T * F;       // [4F]
-    tail_forward_core(p, g, HC, A3, b3e);
+    tail_forward_core(p, g, 0, T, HC, A3, b3e);
     for (int i = threadIdx.x; i < T * F; i += blockDim.x) {
         const int r = i / F, f = i - r * F;
         float s = p.b4[f];
@@ -191,7 +196,7 @@ __global__ void __launch_bounds__(kThreads) k_target_tail_bwd(const TargetTailPa
     float* DY = A3 + T * H;       // [T][F]
     float* b3e = DY + T * F;      // [4F]
     float* st = b3e + H;          // [2F] sum g, sum g xhat
-    tail_forward_core(p, g, HC, A3, b3e);
+    tail_forward_core(p, g, 0, T, HC, A3, b3e);
     float* gp = p.gpartial + (size_t)g * tail_partial_floats(F);
     const float* sv = p.bn_save + (size_t)g * 4 * F;
     const float* go = p.gout + (size_t)g * T * F;
@@ -319,6 +324,178 @@ __global__ void __launch_bounds__(kThreads) k_target_tail_bwd(const TargetTailPa
         for (int j = 0; j < M; ++j) s = fmaf(DHC[r * K3 + F + j], p.w2[j * M + k], s);
         p.dasum[(size_t)g * T * M + i] = s;
     }
+}
+
+// ------------------------------------------------------------------------------------------
+// class-tiled tail, for graphs whose T classes do not fit the one-CTA tail's shared memory.  CTA (tile, g) owns the
+// classes [tile * kTailRows, tile * kTailRows + kTailRows) of graph g.  The BatchNorm statistics and the parameter
+// gradients leave as one partial per (graph, tile), which k_bn_finalize_all and k_reduce_multi combine in tile order;
+// the tile count depends on T alone, so a graph's results do not depend on the batch it is in.
+// Dynamic shared memory: kTailRows * (3F + 4F + F) + 4F floats (32.25 KB at Fdim 16).
+// ------------------------------------------------------------------------------------------
+constexpr int kTailRows = 64;
+constexpr size_t kTailOneCtaSmem = 200 * 1024;
+__host__ __device__ constexpr int tail_tiles(int T) { return (T + kTailRows - 1) / kTailRows; }
+// the one-CTA backward holds T * 8F + 6F floats (its forward 2F fewer): above the budget the tail runs class-tiled
+inline bool tail_tiled(int T, int F) { return sizeof(float) * ((size_t)T * 8 * F + 6 * F) > kTailOneCtaSmem; }
+inline size_t tail_rows_smem(int F) { return sizeof(float) * ((size_t)kTailRows * 8 * F + 4 * F); }
+
+// y_pre for the tile's rows (the output too when not normed) and, in training, the tile's BatchNorm record
+__global__ void __launch_bounds__(kThreads) k_target_tail_rows_fwd(const TargetTailParams p) {
+    extern __shared__ __align__(16) float sm[];
+    const int F = p.F, T = p.T, H = 4 * F, K3 = 3 * F;
+    const int g = blockIdx.y, r0 = blockIdx.x * kTailRows, n = min(kTailRows, T - r0);
+    float* HC = sm;                       // [kTailRows][3F]
+    float* A3 = HC + kTailRows * K3;      // [kTailRows][4F]
+    float* Y = A3 + kTailRows * H;        // [kTailRows][F]
+    float* b3e = Y + kTailRows * F;       // [4F]
+    tail_forward_core(p, g, r0, n, HC, A3, b3e);
+    const size_t row0 = ((size_t)g * T + r0) * F;
+    for (int i = threadIdx.x; i < n * F; i += blockDim.x) {
+        const int r = i / F, f = i - r * F;
+        float s = p.b4[f];
+        for (int j = 0; j < H; ++j) s = fmaf(A3[r * H + j], p.w4[f * H + j], s);
+        Y[i] = s;
+        p.y_pre[row0 + i] = s;
+        if (p.mode == 0) p.x_t_out[row0 + i] = s;
+    }
+    if (p.mode != 1) return;
+    __syncthreads();
+    if (threadIdx.x < F) {              // two-pass mean and M2 of the tile's rows
+        const int f = threadIdx.x;
+        float s = 0.f;
+        for (int r = 0; r < n; ++r) s += Y[r * F + f];
+        const float mean = s / (float)n;
+        float m2 = 0.f;
+        for (int r = 0; r < n; ++r) {
+            const float d = Y[r * F + f] - mean;
+            m2 += d * d;
+        }
+        float* rec = p.bn_partial + ((size_t)g * gridDim.x + blockIdx.x) * bn_partial_stride(F);
+        rec[f] = mean;
+        rec[F + f] = m2;
+        if (f == 0) rec[2 * F] = (float)n;
+    }
+}
+
+// the tile's rows of the backward tail: g_x_t (direct part), dasum and one parameter-gradient partial.  dgamma and
+// dbeta are the BatchNorm sums in p.bn_stat (reduced by the caller); the gamma / beta slots of the partial are unused.
+__global__ void __launch_bounds__(kThreads) k_target_tail_rows_bwd(const TargetTailParams p) {
+    extern __shared__ __align__(16) float sm[];
+    const int F = p.F, T = p.T, M = 2 * F, H = 4 * F, K3 = 3 * F;
+    const int g = blockIdx.y, r0 = blockIdx.x * kTailRows, n = min(kTailRows, T - r0);
+    float* HC = sm;                       // [kTailRows][3F]  hcat, later dhcat
+    float* A3 = HC + kTailRows * K3;      // [kTailRows][4F]  hidden activations, overwritten in place by dh3
+    float* DH = A3;
+    float* DY = A3 + kTailRows * H;       // [kTailRows][F]
+    float* b3e = DY + kTailRows * F;      // [4F]
+    tail_forward_core(p, g, r0, n, HC, A3, b3e);
+    float* gp = p.gpartial + ((size_t)g * gridDim.x + blockIdx.x) * tail_partial_floats(F);
+    const float* sv = p.bn_save + (size_t)g * 4 * F;
+    const size_t row0 = ((size_t)g * T + r0) * F;
+    const float* go = p.gout + row0;
+    const float* yp = p.y_pre + row0;
+    for (int i = threadIdx.x; i < n * F; i += blockDim.x) {
+        const int f = i % F;
+        const float gv = go[i];
+        float dy;
+        if (p.mode == 1) {
+            const float* st = p.bn_stat + (size_t)g * 2 * F;
+            const float xh = (yp[i] - sv[f]) * rsqrtf(sv[F + f] + p.eps);
+            dy = sv[2 * F + f] * (gv - st[f] / (float)T - xh * st[F + f] / (float)T);
+        } else if (p.mode == 2) {
+            dy = gv * sv[2 * F + f];
+        } else {
+            dy = gv;
+        }
+        DY[i] = dy;
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < F * H; i += blockDim.x) {     // dW4
+        const int f = i / H, j = i - f * H;
+        float s = 0.f;
+        for (int r = 0; r < n; ++r) s = fmaf(DY[r * F + f], A3[r * H + j], s);
+        gp[tail_off_w4(F) + i] = s;
+    }
+    if (threadIdx.x < F) {                                       // db4
+        float s = 0.f;
+        for (int r = 0; r < n; ++r) s += DY[r * F + threadIdx.x];
+        gp[tail_off_b4(F) + threadIdx.x] = s;
+    }
+    __syncthreads();              // dW4 has read every activation: dh3 may overwrite them
+    for (int i = threadIdx.x; i < n * H; i += blockDim.x) {
+        const int r = i / H, j = i - r * H;
+        float s = 0.f;
+        for (int f = 0; f < F; ++f) s = fmaf(DY[r * F + f], p.w4[f * H + j], s);
+        DH[i] = s * (A3[i] > 0.f ? 1.f : kSlope);
+    }
+    __syncthreads();
+    // dW3 (hcat columns, then the u columns), db3 = the tile's column sums of dh3 (k_target_tail_gu reads them back)
+    for (int i = threadIdx.x; i < H * H; i += blockDim.x) {
+        const int j = i / H, k = i - j * H;
+        float s = 0.f;
+        if (k < K3) {
+            for (int r = 0; r < n; ++r) s = fmaf(DH[r * H + j], HC[r * K3 + k], s);
+        } else {
+            float tot = 0.f;
+            for (int r = 0; r < n; ++r) tot += DH[r * H + j];
+            s = tot * p.u[(size_t)g * F + (k - K3)];
+        }
+        gp[tail_off_w3(F) + i] = s;
+    }
+    for (int j = threadIdx.x; j < H; j += blockDim.x) {
+        float tot = 0.f;
+        for (int r = 0; r < n; ++r) tot += DH[r * H + j];
+        gp[tail_off_b3(F) + j] = tot;
+    }
+    __syncthreads();
+    float* DHC = HC;   // hcat is dead after dW3: dhcat = dh3 . W3[:, :3F]
+    for (int i = threadIdx.x; i < n * K3; i += blockDim.x) {
+        const int r = i / K3, k = i - r * K3;
+        float s = 0.f;
+        for (int j = 0; j < H; ++j) s = fmaf(DH[r * H + j], p.w3[j * H + k], s);
+        DHC[i] = s;
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < n * F; i += blockDim.x) {
+        const int r = i / F, k = i - r * F;
+        p.g_x_t[row0 + i] = DHC[r * K3 + k];
+    }
+    const float* as = p.act_sum + ((size_t)g * T + r0) * M;
+    for (int i = threadIdx.x; i < M * M; i += blockDim.x) {      // dW2 = dagg^T . act_sum
+        const int j = i / M, k = i - j * M;
+        float s = 0.f;
+        for (int r = 0; r < n; ++r) s = fmaf(DHC[r * K3 + F + j], as[(size_t)r * M + k], s);
+        gp[tail_off_w2(F) + i] = s;
+    }
+    for (int j = threadIdx.x; j < M; j += blockDim.x) {          // db2 = sum_i count_i dagg[i]
+        float s = 0.f;
+        for (int r = 0; r < n; ++r) s = fmaf(class_count(p, r0 + r), DHC[r * K3 + F + j], s);
+        gp[tail_off_b2(F) + j] = s;
+    }
+    float* da = p.dasum + ((size_t)g * T + r0) * M;
+    for (int i = threadIdx.x; i < n * M; i += blockDim.x) {      // dasum = dagg . W2
+        const int r = i / M, k = i - r * M;
+        float s = 0.f;
+        for (int j = 0; j < M; ++j) s = fmaf(DHC[r * K3 + F + j], p.w2[j * M + k], s);
+        da[i] = s;
+    }
+}
+
+// g_u[g] = W3[:, 3F:]^T . (sum over the tiles, in tile order, of the tiles' dh3 column sums)
+__global__ void k_target_tail_gu(const float* __restrict__ gpartial, int ntiles, int G, int F,
+                                 const float* __restrict__ w3, float* __restrict__ g_u) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= G * F) return;
+    const int g = i / F, f = i - g * F, H = 4 * F;
+    const float* gp = gpartial + (size_t)g * ntiles * tail_partial_floats(F) + tail_off_b3(F);
+    float s = 0.f;
+    for (int j = 0; j < H; ++j) {
+        float tot = 0.f;
+        for (int t = 0; t < ntiles; ++t) tot += gp[(size_t)t * tail_partial_floats(F) + j];
+        s = fmaf(tot, w3[j * H + 3 * F + f], s);
+    }
+    g_u[i] = s;
 }
 
 // ------------------------------------------------------------------------------------------
